@@ -495,6 +495,24 @@ def subpath_probe(tp, scenes, device, hbm_peak, solver, gm, rp, with_cpu):
     return out
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, res, first, n):
+    """--dump-outputs: what MomaTrajOpt.download() hands a caller for candidates first .. first + n - 1 (the last
+    plan of the timed solve), one float64 DIR/<name>.npy per result array, candidates along the first axis. Above
+    64 MB in all, a fixed seeded sample of the candidates is written. candidate_index.npy lists the candidates
+    written (index inside the plan)."""
+    rows = {k: v[first:first + n] for k, v in res.items() if isinstance(v, np.ndarray)}
+    per_cand = 8 * (1 + sum(v[0].size for v in rows.values()))
+    m = min(n, (DUMP_BYTES - 4096 * (len(rows) + 1)) // per_cand)
+    idx = np.arange(n) if m == n else np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "candidate_index.npy"), idx.astype(np.float64))
+    for k, v in rows.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v[idx].astype(np.float64))
+
+
 def run_reference(args):
     """--impl reference: the reference's CPU algorithm for the path on the host cores — the oracle port (bit-identical
     to the reference's optimizer and map compiled unmodified, tests/test_ref_pin.py); rank 0
@@ -554,7 +572,13 @@ def main():
     ap.add_argument("--slots", type=int, default=2048,
                     help="candidates in flight on the device (continuous batching: a finished candidate's slot is "
                          "refilled from the queue of waiting plans on the device)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the results of the last timed plan to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the device solve's results; it does not apply to --impl reference")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -569,7 +593,7 @@ def main():
     pts, _ = scenes.cuboids_scene(42)
     gm = tp.GridMap(desc, device=local)
     gm.regenerateMap(pts)
-    K, W = max(args.steps, 1), max(args.warmup, 0)
+    K, W = args.steps, max(args.warmup, 0)
     # One step = one plan of 256 candidates. Every rank owns DISTINCT plans (seeded by rank and step): candidates
     # and plans are independent, so they shard with no data-path collective (weak scaling: K plans per GPU). The
     # K plans of a rank are queued on its device and stream through a fixed pool of candidate slots.
@@ -602,6 +626,8 @@ def main():
     res = solver.download()
     n_ok = int(res["status"].sum())
     evals_total = int(res["evals"].sum())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, (K - 1) * n_cand, n_cand)
 
     # ---- end-to-end arm: host buffers in, host results out, through the public API — the worker flow of
     # planner.cpp:847-1010 (pre-processing, H2D of the problems, the solve, the success gate, the per-plan selection
