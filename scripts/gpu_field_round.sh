@@ -1,12 +1,8 @@
 #!/bin/bash
-# Dev: field parity tests + 800x800x80 rebuild timing for the EDT kernel variants.
+# Dev: field parity tests + 800x800x80 rebuild timing of the default EDT kernels and of the divide and conquer.
 mkdir -p gpurun_out
 export PYTHONPATH=.
 python -m pytest tests/test_gpu_parity.py tests/test_gpu_rog.py tests/test_gpu_headline.py -m gpu -x -q -k "field or rog or baseline or raster" > gpurun_out/field_tests.log 2>&1
 tail -2 gpurun_out/field_tests.log
-for ns in 4 2; do
-echo "NS=$ns"; TOPAY_EDT_NS=$ns KEEP_SQ=0 python scripts/field_probe.py 2>&1 | tail -2
-TOPAY_EDT_NS=$ns KEEP_SQ=0 timeout 300 ncu --metrics gpu__time_duration.sum,smsp__inst_executed.sum --clock-control none --csv --log-file gpurun_out/r02_launches_field_ns$ns.csv python scripts/field_probe.py > /dev/null 2>&1
-grep "k_edt_scan\|k_edt_contig_thread" gpurun_out/r02_launches_field_ns$ns.csv | tail -6 | awk -F'","' '{print substr($5,1,40), $(NF-2), $(NF)}'
-done
+echo "default"; KEEP_SQ=0 python scripts/field_probe.py 2>&1 | tail -2
 echo "D&C"; TOPAY_EDT_SCAN=0 KEEP_SQ=0 python scripts/field_probe.py 2>&1 | tail -2

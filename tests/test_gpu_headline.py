@@ -122,6 +122,7 @@ def test_two_lanes_give_the_single_lane_results(gpu_scene, monkeypatch):
         res[lanes, ns] = s.optimizeTrajBatch(paths, bv, ba)
         st = s.stats()
         assert res[lanes, ns]["evals"].sum() <= st["slot_ticks"]
+        assert st["eval_launches"] == lanes * st["ticks"]
         win[lanes, ns] = s.planWinners(plans, use_gate=True)
         s.close()
     for key in ((2, 9), (2, 2)):

@@ -1,7 +1,10 @@
-// Host-side helpers shared by field.cu and solver.cu.
+// Host-side helpers shared by field.cu, edt.cu, rogfield.cu and solver.cu.
 #pragma once
 #include <cuda_runtime.h>
 
+#include <algorithm>
+#include <map>
+#include <mutex>
 #include <string>
 
 #include "hd.cuh"
@@ -38,7 +41,7 @@ struct TpRogSink {
     double* neg;                 // res * sqrt(negative transform)  (tmp_buffer1_ / neg_buffer)
 };
 
-// Scratch of the separable exact EDT (field.cu), shared by the dense and the ROG-ring field.
+// Scratch of the separable exact EDT (edt.cu), shared by the dense and the ROG-ring field.
 struct TpEdtScratch {
     cudaStream_t stream;
     int16_t* packed16;            // pass-1 output (sign-packed 1-D distances), A*B*C
@@ -59,6 +62,31 @@ inline void tp_pool_keep(int device) {
         unsigned long long keep = ~0ull;
         cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep);
     }
+}
+
+// cudaMalloc of `count` elements (at least one). On failure *p is null, the error text is set and the result is
+// TOPAY_ERR_ALLOC.
+template <typename T>
+int tp_dev_malloc(T** p, size_t count) {
+    cudaError_t e = cudaMalloc((void**)p, std::max<size_t>(count, 1) * sizeof(T));
+    if (e != cudaSuccess) {
+        tp_set_error(std::string("cudaMalloc failed: ") + cudaGetErrorString(e));
+        *p = nullptr;
+        return TOPAY_ERR_ALLOC;
+    }
+    return TOPAY_OK;
+}
+
+// Raises `kernel`'s max dynamic shared memory to at least `bytes`. The attribute belongs to the kernel, not to one
+// solver or field, and objects of different sizes coexist in a process (bench: 64-piece plans next to 16-piece latency
+// plans), so it only ever grows: every call sets the largest size asked for that kernel so far.
+inline cudaError_t tp_grow_dyn_smem(const void* kernel, size_t bytes) {
+    static std::mutex mu;
+    static std::map<const void*, size_t> high;
+    std::lock_guard<std::mutex> lock(mu);
+    size_t& h = high[kernel];
+    h = std::max(h, bytes);
+    return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h);
 }
 
 #define TP_CUDA_OK(call, cleanup)                                                              \

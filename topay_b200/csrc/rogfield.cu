@@ -9,7 +9,7 @@
 //
 // The local update box is gathered out of the ring into a dense [bx][by][bz] occupancy array
 // (one coalesced pass), transformed by the same exact integer EDT kernels as the dense field
-// (field.cu: z, y, x, both signs), and scattered back through the per-axis wrap rule. What the
+// (edt.cu: z, y, x, both signs), and scattered back through the per-axis wrap rule. What the
 // reference leaves behind in its persistent buffers is reproduced cell for cell, including the
 // cells its combine step reads without the wrap (box coordinates used as memory coordinates,
 // esdf_map.cpp:305-315, 391-398), which is why the negative distances live in their own ring
@@ -183,17 +183,6 @@ __global__ void k_rog_line(TpRog r, const double* __restrict__ s, const double* 
     out[i] = tp_rog_line_free2d(r, a, b, threshold, cap > (1L << 30) ? (1 << 30) : (int)cap) ? 1 : 0;
 }
 
-template <typename T>
-int rmalloc(T** p, size_t count) {
-    cudaError_t e = cudaMalloc((void**)p, std::max<size_t>(count, 1) * sizeof(T));
-    if (e != cudaSuccess) {
-        tp_set_error(std::string("cudaMalloc failed: ") + cudaGetErrorString(e));
-        *p = nullptr;
-        return TOPAY_ERR_ALLOC;
-    }
-    return TOPAY_OK;
-}
-
 int ifloor(double v) { return (int)std::floor(v); }
 
 // globalIndexToLocalIndex (sliding_map.cpp:205-218)
@@ -293,10 +282,10 @@ extern "C" int topay_rogfield_create(const topay_rog_desc* d, int device, topay_
     f->n2 = (size_t)f->size[0] * f->size[1];
     f->n3 = f->n2 * f->size[2];
     TP_CUDA_OK(cudaStreamCreateWithFlags(&f->stream, cudaStreamNonBlocking), { delete f; });
-#define RA(p, n)                                  \
-    if ((rc = rmalloc(&(p), (n))) != TOPAY_OK) {  \
-        topay_rogfield_destroy(f);                \
-        return rc;                                \
+#define RA(p, n)                                        \
+    if ((rc = tp_dev_malloc(&(p), (n))) != TOPAY_OK) {  \
+        topay_rogfield_destroy(f);                      \
+        return rc;                                      \
     }
     RA(f->occ_cnt, f->n3 + 1);   // +1: the 16-bit atomics work on aligned 32-bit words
     RA(f->unk_cnt, f->n3 + 1);

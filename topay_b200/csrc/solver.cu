@@ -26,6 +26,34 @@ struct TpRunningGuard {
 
 #define TP_EV 7   // CUDA events per tick in timed mode: start, after integrate / penalty / chain / adjoint / L-BFGS / generate
 
+// Live slots up to which a tick runs k_cand as one fused launch: one wave of candidate blocks (3 blocks x 148 SMs).
+constexpr int TP_FUSE_MAX_SLOTS = 444;
+
+// One lane of a run: the live lists and counts its kernels read and write, the stream it is enqueued on, and its
+// live-slot count, which returns from the device through a pinned word after every batch.
+struct TpLane {
+    int32_t* list;          // [TP_TICKS + 1][n_slots] live lists
+    int32_t* count;         // [TP_TICKS + 1] live counts
+    cudaStream_t stream;
+    int32_t* h_live;        // pinned
+    int live;
+};
+
+// Launches of an enqueue, counted where they are enqueued.
+struct TpLaunches {
+    int64_t kernels = 0, evals = 0;
+    void add_to(topay_solver_stats& st) const {
+        st.kernel_launches += kernels;
+        st.eval_launches += evals;
+    }
+};
+
+// A captured batch of ticks and the launches one replay of it makes.
+struct TpBatchGraph {
+    cudaGraphExec_t exec;
+    TpLaunches launches;
+};
+
 struct topay_solver {
     TpSolverDev dev;
     TpParams params;
@@ -41,20 +69,16 @@ struct topay_solver {
     TpCandState* h_state;
     double *p_head, *p_tail, *p_sxy, *p_exy, *p_ixy;
     std::vector<void*> allocs;
-    int32_t* h_active;   // pinned: [0] live slots after the batch, [1..3] queue state
+    int32_t* h_active;   // pinned: [0] lane A's live slots after the batch, [1..3] queue state, [4] lane B's live slots
     unsigned long long* h_nodes;  // pinned
-    int slots;           // ticks per batch (TP_TICKS)
     int n_slots_used;    // slots seeded by the last run (min(n_slots, n_cand))
     std::vector<cudaEvent_t> ev;  // event pool for the penalty kernel timing
     cudaEvent_t ev_begin, ev_end;
-    bool spin_sync;         // TOPAY_SPIN_SYNC=1: always spin on the stream (lowest latency, one busy core per plan);
-                            // default: spin while at most two solves run in this process, sleep beyond that
     cudaEvent_t ev_batch;   // blocking-sync event: the host thread sleeps while a batch of ticks runs
                             // (P plans in flight x N ranks would otherwise spin on as many cores)
     topay_solver_stats stats;
     size_t smem_cand;    // dynamic shared memory of the adjoint / generate launches (banded system)
     size_t smem_lbfgs;   // ... of the L-BFGS launch (TMA ring + tables)
-    int fuse_max;        // live slots up to which a tick runs k_cand as one fused launch (TOPAY_FUSE_MAX)
     // initial state kept on the host for repeated runs
     double* h_x0;
     size_t h_x0_count;
@@ -62,17 +86,16 @@ struct topay_solver {
     // launch geometry or a captured pointer changes
     bool timed;                 // per-launch CUDA events around k_penalty (plain launches, no graph)
     // one CUDA graph per launch-grid bucket (live slots rounded up), rebuilt when max_N or a captured pointer changes
-    std::map<int, cudaGraphExec_t> graphs;
+    std::map<int, TpBatchGraph> graphs;
     int graph_max_N;
     // Two LANES (large pools only): the slots are split into two halves with their own live lists, and a batch runs
-    // the halves' tick chains as two parallel branches of one CUDA graph (second branch on stream2). The kernels of
-    // a tick are bound by different things (k_penalty: FP64 issue; the two-loop: HBM; the banded LU: one warp's
-    // latency chain), so one half's k_penalty overlaps the other half's k_cand. Store, queue and results are shared:
-    // which lane solves a candidate does not change its result.
+    // the halves' tick chains as two parallel branches of one CUDA graph (lane B's branch on its own stream). The
+    // kernels of a tick are bound by different things (k_penalty: FP64 issue; the two-loop: HBM; the banded LU: one
+    // warp's latency chain), so one half's k_penalty overlaps the other half's k_cand. Store, queue and results are
+    // shared: which lane solves a candidate does not change its result.
+    TpLane lane[2];             // lane A: dev.list / dev.count on `stream`; lane B: its own lists on a second stream
     int lanes;                  // lanes of the run in progress (1 or 2)
     int lane_min_slots;         // two lanes from this many seeded slots on (TOPAY_LANE_MIN_SLOTS; 0 = never)
-    int32_t *list_b, *count_b;  // lane B's live lists / counts (lane A uses dev.list / dev.count)
-    cudaStream_t stream2;
     cudaEvent_t ev_fork, ev_join;
     // scenario sweeps: candidates of one upload may belong to different fields (topay_solver_assign_fields)
     std::vector<topay_field*> fields;
@@ -102,16 +125,10 @@ bool solver_field_ready(const topay_solver* s) {
 
 template <typename T>
 int dev_alloc(topay_solver* s, T** p, size_t count) {
-    void* q = nullptr;
-    if (count == 0) count = 1;
-    cudaError_t e = cudaMalloc(&q, count * sizeof(T));
-    if (e != cudaSuccess) {
-        tp_set_error(std::string("cudaMalloc failed: ") + cudaGetErrorString(e));
-        return TOPAY_ERR_ALLOC;
-    }
-    cudaMemsetAsync(q, 0, count * sizeof(T), s->stream);
-    s->allocs.push_back(q);
-    *p = (T*)q;
+    const int rc = tp_dev_malloc(p, count);
+    if (rc != TOPAY_OK) return rc;
+    cudaMemsetAsync(*p, 0, std::max<size_t>(count, 1) * sizeof(T), s->stream);
+    s->allocs.push_back(*p);
     return TOPAY_OK;
 }
 
@@ -135,8 +152,43 @@ int grid_bucket(int n) {
     }
 }
 
-void launch_eval(topay_solver* s, bool timed, int tick, int ny) {
-    const TpSolverDev& D = s->dev;
+// k_penalty<Kpad, MULTI>, [log2(Kpad) - 2][MULTI]
+using PenaltyKernel = decltype(&k_penalty<4>);
+const PenaltyKernel k_penalty_of[4][2] = {{k_penalty<4>, k_penalty<4, true>},
+                                          {k_penalty<8>, k_penalty<8, true>},
+                                          {k_penalty<16>, k_penalty<16, true>},
+                                          {k_penalty<32>, k_penalty<32, true>}};
+int kpad_index(int kpad) { return kpad == 4 ? 0 : kpad == 8 ? 1 : kpad == 16 ? 2 : 3; }
+
+// k_cand<MODE> of a launch mode, and its dynamic shared memory: the banded system (adjoint, generate), the L-BFGS
+// ring (advance), or the larger of the two (all three halves fused)
+constexpr int TP_MODE_ALL = TP_MODE_ADJ | TP_MODE_ADVANCE | TP_MODE_GEN;
+constexpr int TP_CAND_MODES[4] = {TP_MODE_ADJ, TP_MODE_ADVANCE, TP_MODE_GEN, TP_MODE_ALL};
+using CandKernel = decltype(&k_cand<TP_MODE_ALL>);
+CandKernel cand_kernel(int mode) {
+    switch (mode) {
+        case TP_MODE_ADJ: return k_cand<TP_MODE_ADJ>;
+        case TP_MODE_ADVANCE: return k_cand<TP_MODE_ADVANCE>;
+        case TP_MODE_GEN: return k_cand<TP_MODE_GEN>;
+        default: return k_cand<TP_MODE_ALL>;
+    }
+}
+size_t cand_smem(const topay_solver* s, int mode) {
+    if (mode == TP_MODE_ADVANCE) return s->smem_lbfgs;
+    if (mode == TP_MODE_ALL) return std::max(s->smem_cand, s->smem_lbfgs);
+    return s->smem_cand;
+}
+
+// What a kernel of lane L reads: the solver's device view with the lane's live lists.
+TpSolverDev lane_dev(const topay_solver* s, const TpLane& L) {
+    TpSolverDev D = s->dev;
+    D.list = L.list;
+    D.count = L.count;
+    return D;
+}
+
+void launch_eval(topay_solver* s, const TpLane& L, bool timed, int tick, int ny, TpLaunches& n) {
+    const TpSolverDev D = lane_dev(s, L);
     const int groups = (s->max_N + D.ppw - 1) / D.ppw;
     const int end_warps = D.end_tasks ? (s->max_N + 31) / 32 : 0;
     dim3 blk(TP_WARPS_PER_BLOCK * 32);
@@ -147,68 +199,30 @@ void launch_eval(topay_solver* s, bool timed, int tick, int ny) {
     const size_t sm_pen = penalty_smem(D.Kpad);
     TpGrid G;
     solver_grid(s, &G);
+    cudaStream_t q = L.stream;
     const int te = tick % TP_TICKS;
-    if (timed) cudaEventRecord(s->ev[TP_EV * te], s->stream);
-    k_integrate<<<g1, blk, sm_int, s->stream>>>(D, tick);
-    if (timed) cudaEventRecord(s->ev[TP_EV * te + 1], s->stream);
-    if (D.n_fields > 1) {
-        switch (D.Kpad) {
-            case 4: k_penalty<4, true><<<g2, blk2, sm_pen, s->stream>>>(D, s->params, G, groups, tick); break;
-            case 8: k_penalty<8, true><<<g2, blk2, sm_pen, s->stream>>>(D, s->params, G, groups, tick); break;
-            case 16: k_penalty<16, true><<<g2, blk2, sm_pen, s->stream>>>(D, s->params, G, groups, tick); break;
-            default: k_penalty<32, true><<<g2, blk2, sm_pen, s->stream>>>(D, s->params, G, groups, tick); break;
-        }
-    } else {
-        switch (D.Kpad) {
-            case 4: k_penalty<4><<<g2, blk2, sm_pen, s->stream>>>(D, s->params, G, groups, tick); break;
-            case 8: k_penalty<8><<<g2, blk2, sm_pen, s->stream>>>(D, s->params, G, groups, tick); break;
-            case 16: k_penalty<16><<<g2, blk2, sm_pen, s->stream>>>(D, s->params, G, groups, tick); break;
-            default: k_penalty<32><<<g2, blk2, sm_pen, s->stream>>>(D, s->params, G, groups, tick); break;
-        }
-    }
-    if (timed) cudaEventRecord(s->ev[TP_EV * te + 2], s->stream);
-    k_chain<<<g1, blk, 0, s->stream>>>(D, s->params, tick);
-    if (timed) cudaEventRecord(s->ev[TP_EV * te + 3], s->stream);
-    s->stats.kernel_launches += 3;
-    s->stats.eval_launches += 1;
+    if (timed) cudaEventRecord(s->ev[TP_EV * te], q);
+    k_integrate<<<g1, blk, sm_int, q>>>(D, tick);
+    if (timed) cudaEventRecord(s->ev[TP_EV * te + 1], q);
+    k_penalty_of[kpad_index(D.Kpad)][D.n_fields > 1]<<<g2, blk2, sm_pen, q>>>(D, s->params, G, groups, tick);
+    if (timed) cudaEventRecord(s->ev[TP_EV * te + 2], q);
+    k_chain<<<g1, blk, 0, q>>>(D, s->params, tick);
+    if (timed) cudaEventRecord(s->ev[TP_EV * te + 3], q);
+    n.kernels += 3;
+    n.evals += 1;
 }
 
-void launch_cand(topay_solver* s, int mode, int tick_in, int tick_out, int nx) {
-    const int sd = (int)(s->smem_cand / sizeof(double)), sl = (int)(s->smem_lbfgs / sizeof(double));
-    constexpr int ALL = TP_MODE_ADJ | TP_MODE_ADVANCE | TP_MODE_GEN;
-    if (mode == ALL) {
-        const size_t sm = std::max(s->smem_cand, s->smem_lbfgs);
-        k_cand<ALL><<<nx, TP_CAND_THREADS, sm, s->stream>>>(s->dev, s->params, (int)(sm / sizeof(double)), tick_in, tick_out);
-    } else if (mode == TP_MODE_GEN)
-        k_cand<TP_MODE_GEN><<<nx, TP_CAND_THREADS, s->smem_cand, s->stream>>>(s->dev, s->params, sd, tick_in, tick_out);
-    else if (mode == TP_MODE_ADJ)
-        k_cand<TP_MODE_ADJ><<<nx, TP_CAND_THREADS, s->smem_cand, s->stream>>>(s->dev, s->params, sd, tick_in, tick_out);
-    else
-        k_cand<TP_MODE_ADVANCE><<<nx, TP_CAND_THREADS, s->smem_lbfgs, s->stream>>>(s->dev, s->params, sl, tick_in, tick_out);
-    s->stats.kernel_launches += 1;
+void launch_cand(topay_solver* s, const TpLane& L, int mode, int tick_in, int tick_out, int nx, TpLaunches& n) {
+    const size_t sm = cand_smem(s, mode);
+    cand_kernel(mode)<<<nx, TP_CAND_THREADS, sm, L.stream>>>(lane_dev(s, L), s->params, (int)(sm / sizeof(double)),
+                                                            tick_in, tick_out);
+    n.kernels += 1;
 }
 
 void drop_graphs(topay_solver* s) {
-    for (auto& kv : s->graphs) cudaGraphExecDestroy(kv.second);
+    for (auto& kv : s->graphs) cudaGraphExecDestroy(kv.second.exec);
     s->graphs.clear();
 }
-
-// While alive, the launch helpers address lane B: its lists, its stream.
-struct TpLaneB {
-    topay_solver* s;
-    int32_t *list, *count;
-    cudaStream_t stream;
-    explicit TpLaneB(topay_solver* s_) : s(s_), list(s_->dev.list), count(s_->dev.count), stream(s_->stream) {
-        s->dev.list = s->list_b;
-        s->dev.count = s->count_b;
-        s->stream = s->stream2;
-    }
-    ~TpLaneB() {
-        s->dev.list = list;
-        s->dev.count = count;
-        s->stream = stream;
-    }
-};
 
 }  // namespace
 
@@ -262,13 +276,10 @@ static int solver_create(const topay_opt_params* opt, const topay_robot_params* 
     s->device = dev;
     s->n_cand = 0;
     s->max_N = 0;
-    s->slots = TP_TICKS;
     s->n_slots_used = 0;
     s->timed = false;
     s->graph_max_N = -1;
     s->checker = nullptr;
-    s->spin_sync = getenv("TOPAY_SPIN_SYNC") && atoi(getenv("TOPAY_SPIN_SYNC")) != 0;
-    s->fuse_max = getenv("TOPAY_FUSE_MAX") ? atoi(getenv("TOPAY_FUSE_MAX")) : 444;   // 3 blocks x 148 SMs
     s->d_pn = nullptr;
     s->d_start = nullptr;
     memset(&s->stats, 0, sizeof(s->stats));
@@ -312,8 +323,8 @@ static int solver_create(const topay_opt_params* opt, const topay_robot_params* 
     ALLOC(D.slot_gid, C);
     ALLOC(D.list, (size_t)(TP_TICKS + 1) * C);
     ALLOC(D.count, (size_t)TP_TICKS + 1);
-    ALLOC(s->list_b, (size_t)(TP_TICKS + 1) * C);
-    ALLOC(s->count_b, (size_t)TP_TICKS + 1);
+    ALLOC(s->lane[1].list, (size_t)(TP_TICKS + 1) * C);
+    ALLOC(s->lane[1].count, (size_t)TP_TICKS + 1);
     ALLOC(D.queue, 4);
     // slots
     ALLOC(D.st, C);
@@ -359,12 +370,17 @@ static int solver_create(const topay_opt_params* opt, const topay_robot_params* 
     }
     TP_CUDA_OK(cudaMallocHost(&s->h_active, 8 * sizeof(int32_t)), { topay_solver_destroy(s); });
     TP_CUDA_OK(cudaMallocHost(&s->h_nodes, 2 * sizeof(unsigned long long)), { topay_solver_destroy(s); });
-    s->ev.resize(TP_EV * s->slots);
+    s->ev.resize(TP_EV * TP_TICKS);
     for (auto& e : s->ev) cudaEventCreate(&e);
     cudaEventCreate(&s->ev_begin);
     cudaEventCreate(&s->ev_end);
     cudaEventCreateWithFlags(&s->ev_batch, cudaEventBlockingSync | cudaEventDisableTiming);
-    cudaStreamCreateWithFlags(&s->stream2, cudaStreamNonBlocking);
+    s->lane[0].list = D.list;
+    s->lane[0].count = D.count;
+    s->lane[0].stream = s->stream;
+    s->lane[0].h_live = s->h_active;
+    cudaStreamCreateWithFlags(&s->lane[1].stream, cudaStreamNonBlocking);
+    s->lane[1].h_live = s->h_active + 4;
     cudaEventCreateWithFlags(&s->ev_fork, cudaEventDisableTiming);
     cudaEventCreateWithFlags(&s->ev_join, cudaEventDisableTiming);
     s->lanes = 1;
@@ -389,43 +405,13 @@ static int solver_create(const topay_opt_params* opt, const topay_robot_params* 
         topay_solver_destroy(s);
         return TOPAY_ERR_TOO_LARGE;
     }
-    // the attribute belongs to the kernel, not to this solver: solvers of different capacities coexist
-    // (bench: 64-piece plans and 16-piece latency plans), so it only ever grows
-    {
-        static std::atomic<size_t> attr_set{0}, attr_lb{0};
-        size_t cur = attr_set.load();
-        while (cur < s->smem_cand && !attr_set.compare_exchange_weak(cur, s->smem_cand)) {}
-        cur = attr_lb.load();
-        while (cur < s->smem_lbfgs && !attr_lb.compare_exchange_weak(cur, s->smem_lbfgs)) {}
-        TP_CUDA_OK(cudaFuncSetAttribute(k_cand<TP_MODE_ADJ>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)attr_set.load()),
-                   { topay_solver_destroy(s); });
-        TP_CUDA_OK(cudaFuncSetAttribute(k_cand<TP_MODE_GEN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)attr_set.load()),
-                   { topay_solver_destroy(s); });
-        TP_CUDA_OK(cudaFuncSetAttribute(k_cand<TP_MODE_ADVANCE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)attr_lb.load()),
-                   { topay_solver_destroy(s); });
-        TP_CUDA_OK(cudaFuncSetAttribute(k_cand<TP_MODE_ADJ | TP_MODE_ADVANCE | TP_MODE_GEN>,
-                                        cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                        (int)std::max(attr_set.load(), attr_lb.load())),
-                   { topay_solver_destroy(s); });
-    }
+    for (int mode : TP_CAND_MODES)
+        TP_CUDA_OK(tp_grow_dyn_smem((const void*)cand_kernel(mode), cand_smem(s, mode)), { topay_solver_destroy(s); });
     const size_t sm_int = (size_t)TP_WARPS_PER_BLOCK * D.ppw * 3 * (2 * D.K + 1) * sizeof(double);
-    {
-        static std::atomic<size_t> attr_int{0};
-        size_t cur = attr_int.load();
-        while (cur < sm_int && !attr_int.compare_exchange_weak(cur, sm_int)) {}
-        TP_CUDA_OK(cudaFuncSetAttribute(k_integrate, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)attr_int.load()),
-                   { topay_solver_destroy(s); });
-    }
-    {
-        TP_CUDA_OK(cudaFuncSetAttribute(k_penalty<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)penalty_smem(4)), { topay_solver_destroy(s); });
-        TP_CUDA_OK(cudaFuncSetAttribute(k_penalty<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)penalty_smem(8)), { topay_solver_destroy(s); });
-        TP_CUDA_OK(cudaFuncSetAttribute(k_penalty<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)penalty_smem(16)), { topay_solver_destroy(s); });
-        TP_CUDA_OK(cudaFuncSetAttribute(k_penalty<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)penalty_smem(32)), { topay_solver_destroy(s); });
-        cudaFuncSetAttribute(k_penalty<4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)penalty_smem(4));
-        cudaFuncSetAttribute(k_penalty<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)penalty_smem(8));
-        cudaFuncSetAttribute(k_penalty<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)penalty_smem(16));
-        cudaFuncSetAttribute(k_penalty<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)penalty_smem(32));
-    }
+    TP_CUDA_OK(tp_grow_dyn_smem((const void*)k_integrate, sm_int), { topay_solver_destroy(s); });
+    for (int k = 0; k < 4; k++)
+        for (PenaltyKernel kern : k_penalty_of[k])
+            TP_CUDA_OK(tp_grow_dyn_smem((const void*)kern, penalty_smem(4 << k)), { topay_solver_destroy(s); });
     TP_CUDA_OK(cudaStreamSynchronize(s->stream), { topay_solver_destroy(s); });
     *out = s;
     return TOPAY_OK;
@@ -450,7 +436,7 @@ extern "C" void topay_solver_destroy(topay_solver* s) {
     if (s->ev_batch) cudaEventDestroy(s->ev_batch);
     if (s->ev_fork) cudaEventDestroy(s->ev_fork);
     if (s->ev_join) cudaEventDestroy(s->ev_join);
-    if (s->stream2) cudaStreamDestroy(s->stream2);
+    if (s->lane[1].stream) cudaStreamDestroy(s->lane[1].stream);
     if (s->stream) cudaStreamDestroy(s->stream);
     delete s;
 }
@@ -551,9 +537,11 @@ extern "C" int topay_solver_eval(topay_solver* s, int stage, const topay_problem
     const TpSolverDev& D = s->dev;
     const int n = prob->n_cand;
     seed_slots(s);   // slot i <- candidate i
-    launch_cand(s, TP_MODE_GEN, TP_TICKS, -1, n);
-    launch_eval(s, false, TP_TICKS, n);
-    launch_cand(s, TP_MODE_ADJ, TP_TICKS, -1, n);
+    TpLaunches launches;
+    launch_cand(s, s->lane[0], TP_MODE_GEN, TP_TICKS, -1, n, launches);
+    launch_eval(s, s->lane[0], false, TP_TICKS, n, launches);
+    launch_cand(s, s->lane[0], TP_MODE_ADJ, TP_TICKS, -1, n, launches);
+    launches.add_to(s->stats);
     TP_CUDA_OK(cudaStreamSynchronize(s->stream), {});
     TP_CUDA_OK(cudaGetLastError(), {});
     s->n_cand = 0;   // the uploaded problem carried the evaluation's phase / multipliers: not a solvable upload
@@ -644,48 +632,47 @@ extern "C" int topay_solver_upload(topay_solver* s, int n_cand, const int32_t* p
                           x.data(), xstride, past.data(), 1, nullptr, nullptr);
 }
 
-// One batch of TP_TICKS ticks over at most `ny` live slots: roll the list, then per tick the three evaluation
-// kernels and k_cand; the live count after the batch and the queue state return through pinned memory.
-static void enqueue_lane(topay_solver* s, int ny, bool timed, int32_t* h_live) {
-    const TpSolverDev& D = s->dev;
-    cudaStream_t q = s->stream;
-    k_list_roll<<<1, 1024, 0, q>>>(D);
+// One batch of TP_TICKS ticks of lane L over at most `ny` live slots: roll the list, then per tick the three
+// evaluation kernels and k_cand; the lane's live count after the batch returns through its pinned word.
+static void enqueue_lane(topay_solver* s, const TpLane& L, int ny, bool timed, TpLaunches& n) {
+    cudaStream_t q = L.stream;
+    k_list_roll<<<1, 1024, 0, q>>>(lane_dev(s, L));
+    n.kernels += 1;
     // Up to one wave of candidate blocks the three halves of k_cand run as ONE launch (the banded system stays in
     // shared memory from the adjoint solve to the next factorisation, two launch boundaries less on the dependent
     // chain of a small plan); above that they are separate launches, each at its own occupancy.
-    const bool fused = !timed && ny <= s->fuse_max;
+    const bool fused = !timed && ny <= TP_FUSE_MAX_SLOTS;
     for (int t = 0; t < TP_TICKS; t++) {
-        launch_eval(s, timed, t, ny);
+        launch_eval(s, L, timed, t, ny, n);
         if (fused) {
-            launch_cand(s, TP_MODE_ADJ | TP_MODE_ADVANCE | TP_MODE_GEN, t, t + 1, ny);
+            launch_cand(s, L, TP_MODE_ALL, t, t + 1, ny, n);
             continue;
         }
-        launch_cand(s, TP_MODE_ADJ, t, -1, ny);
+        launch_cand(s, L, TP_MODE_ADJ, t, -1, ny, n);
         if (timed) cudaEventRecord(s->ev[TP_EV * t + 4], q);
-        launch_cand(s, TP_MODE_ADVANCE, t, -1, ny);
+        launch_cand(s, L, TP_MODE_ADVANCE, t, -1, ny, n);
         if (timed) cudaEventRecord(s->ev[TP_EV * t + 5], q);
-        launch_cand(s, TP_MODE_GEN, t, t + 1, ny);
+        launch_cand(s, L, TP_MODE_GEN, t, t + 1, ny, n);
         if (timed) cudaEventRecord(s->ev[TP_EV * t + 6], q);
     }
-    cudaMemcpyAsync(h_live, D.count + TP_TICKS, sizeof(int32_t), cudaMemcpyDeviceToHost, q);
-    s->stats.kernel_launches += 1;
+    cudaMemcpyAsync(L.h_live, L.count + TP_TICKS, sizeof(int32_t), cudaMemcpyDeviceToHost, q);
 }
 
-static void enqueue_batch(topay_solver* s, int ny, int ny_b, bool timed) {
+// One batch of both lanes (ny, ny_b: their launch grids); returns the launches it enqueued.
+static TpLaunches enqueue_batch(topay_solver* s, int ny, int ny_b, bool timed) {
+    TpLaunches n;
     cudaStream_t q = s->stream;
     if (s->lanes == 2) {
         // fork: lane B's chain is a second branch of the captured graph
         cudaEventRecord(s->ev_fork, q);
-        cudaStreamWaitEvent(s->stream2, s->ev_fork, 0);
-        {
-            TpLaneB lane_b(s);
-            enqueue_lane(s, ny_b, timed, s->h_active + 4);
-        }
-        cudaEventRecord(s->ev_join, s->stream2);
+        cudaStreamWaitEvent(s->lane[1].stream, s->ev_fork, 0);
+        enqueue_lane(s, s->lane[1], ny_b, timed, n);
+        cudaEventRecord(s->ev_join, s->lane[1].stream);
     }
-    enqueue_lane(s, ny, timed, s->h_active);
+    enqueue_lane(s, s->lane[0], ny, timed, n);
     if (s->lanes == 2) cudaStreamWaitEvent(q, s->ev_join, 0);
     cudaMemcpyAsync(s->h_active + 1, s->dev.queue, 3 * sizeof(int32_t), cudaMemcpyDeviceToHost, q);
+    return n;
 }
 
 // Marks every candidate that is still live (or was never started) as stopped by the tick cap.
@@ -711,6 +698,12 @@ __global__ void k_mark_tick_cap(const __grid_constant__ TpSolverDev S, int n_sto
     }
 }
 
+// Tick cap: marks lane L's live candidates and, with n_store > 0, the candidates of the store never handed to a slot.
+// Runs after the last batch, when both lanes have joined the solver's stream.
+static void mark_tick_cap(topay_solver* s, const TpLane& L, int n_store) {
+    k_mark_tick_cap<<<(std::max(n_store, s->dev.n_slots) + 127) / 128, 128, 0, s->stream>>>(lane_dev(s, L), n_store);
+}
+
 extern "C" int topay_solver_run(topay_solver* s) {
     if (!s || s->n_cand < 1) return TOPAY_ERR_INVALID_ARG;
     if (!solver_field_ready(s)) {
@@ -730,15 +723,19 @@ extern "C" int topay_solver_run(topay_solver* s) {
     if (D.trace) cudaMemsetAsync(D.trace_len, 0, (size_t)D.max_cand * sizeof(int32_t), q);
     cudaEventRecord(s->ev_begin, q);
     // the store holds the uploaded initial state, so repeated runs do identical work
-    int live = seed_slots(s), live_b = 0;
-    launch_cand(s, TP_MODE_GEN, TP_TICKS, -1, live);
-    s->stats.kernel_launches += 1;
-    s->lanes = (!s->timed && s->lane_min_slots > 0 && live >= s->lane_min_slots) ? 2 : 1;
+    TpLane &A = s->lane[0], &B = s->lane[1];
+    A.live = seed_slots(s);
+    B.live = 0;
+    TpLaunches first;
+    launch_cand(s, A, TP_MODE_GEN, TP_TICKS, -1, A.live, first);
+    first.kernels += 1;   // seed_slots' k_slot_init
+    first.add_to(s->stats);
+    s->lanes = (!s->timed && s->lane_min_slots > 0 && A.live >= s->lane_min_slots) ? 2 : 1;
     if (s->lanes == 2) {
-        const int na = (live + 1) / 2;
-        k_lane_split<<<1, 1024, 0, q>>>(D, s->list_b, s->count_b, na, live);
-        live_b = live - na;
-        live = na;
+        const int na = (A.live + 1) / 2;
+        k_lane_split<<<1, 1024, 0, q>>>(D, B.list, B.count, na, A.live);
+        B.live = A.live - na;
+        A.live = na;
     }
     double ms_eval = 0.0, ms_k[3] = {0.0, 0.0, 0.0}, ms_c[3] = {0.0, 0.0, 0.0}, full_ms_cand = 0.0;
     unsigned long long hist_prev = 0, full_hist = 0;
@@ -763,42 +760,39 @@ extern "C" int topay_solver_run(topay_solver* s) {
         s->graph_max_N = s->max_N;
     }
     while (!done && ticks < max_ticks) {
-        const int ny = grid_bucket(live), ny_b = s->lanes == 2 ? grid_bucket(live_b) : 0;
+        const int ny = grid_bucket(A.live), ny_b = s->lanes == 2 ? grid_bucket(B.live) : 0;
         const int key = ny | (ny_b << 16);
         if (use_graph) {
             auto it = s->graphs.find(key);
             if (it == s->graphs.end()) {
                 cudaGraph_t g = nullptr;
                 cudaGraphExec_t ge = nullptr;
-                const topay_solver_stats keep = s->stats;
                 TP_CUDA_OK(cudaStreamBeginCapture(q, cudaStreamCaptureModeThreadLocal), {});
-                enqueue_batch(s, ny, ny_b, false);
+                const TpLaunches launches = enqueue_batch(s, ny, ny_b, false);
                 TP_CUDA_OK(cudaStreamEndCapture(q, &g), {});
                 TP_CUDA_OK(cudaGraphInstantiate(&ge, g, 0), { cudaGraphDestroy(g); });
                 cudaGraphDestroy(g);
-                s->stats = keep;   // the capture pass launched nothing
-                it = s->graphs.emplace(key, ge).first;
+                it = s->graphs.emplace(key, TpBatchGraph{ge, launches}).first;
             }
-            TP_CUDA_OK(cudaGraphLaunch(it->second, q), {});
-            s->stats.kernel_launches += (ny <= s->fuse_max ? 4 : 6) * TP_TICKS + 1;
-            if (s->lanes == 2) s->stats.kernel_launches += (ny_b <= s->fuse_max ? 4 : 6) * TP_TICKS + 1;
-            s->stats.eval_launches += TP_TICKS * s->lanes;
+            TP_CUDA_OK(cudaGraphLaunch(it->second.exec, q), {});
+            it->second.launches.add_to(s->stats);
         } else {
-            enqueue_batch(s, ny, 0, true);
+            enqueue_batch(s, ny, 0, true).add_to(s->stats);
             cudaMemcpyAsync(s->h_nodes, D.node_count, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, q);
         }
         ticks += TP_TICKS;
-        slot_ticks += (long long)(live + live_b) * TP_TICKS;
-        if (s->spin_sync || g_solves_running.load(std::memory_order_relaxed) <= 2) {
+        slot_ticks += (long long)(A.live + B.live) * TP_TICKS;
+        // spin while at most two solves run in this process (lowest latency, one busy core per plan), else sleep
+        if (g_solves_running.load(std::memory_order_relaxed) <= 2) {
             TP_CUDA_OK(cudaStreamSynchronize(q), {});
         } else {
             cudaEventRecord(s->ev_batch, q);
             TP_CUDA_OK(cudaEventSynchronize(s->ev_batch), {});
         }
-        const int live_after = s->h_active[0];
+        const int live_after = *A.h_live;
         if (!use_graph) {
             // batches in which every slot was still solving: the full-activity figures
-            const bool full = live_after == live;
+            const bool full = live_after == A.live;
             const unsigned long long hist_now = s->h_nodes[1];
             double cand_batch = 0.0, lbfgs_batch = 0.0;
             for (int t = 0; t < TP_TICKS; t++) {
@@ -825,16 +819,13 @@ extern "C" int topay_solver_run(topay_solver* s) {
             }
             hist_prev = hist_now;
         }
-        live = live_after;
-        if (s->lanes == 2) live_b = s->h_active[4];
-        done = live + live_b == 0;
+        A.live = live_after;
+        if (s->lanes == 2) B.live = *B.h_live;
+        done = A.live + B.live == 0;
     }
     if (!done) {
-        if (s->lanes == 2) {
-            TpLaneB lane_b(s);
-            k_mark_tick_cap<<<(D.n_slots + 127) / 128, 128, 0, q>>>(s->dev, 0);
-        }
-        k_mark_tick_cap<<<(std::max(s->n_cand, D.n_slots) + 127) / 128, 128, 0, q>>>(D, s->n_cand);
+        if (s->lanes == 2) mark_tick_cap(s, B, 0);
+        mark_tick_cap(s, A, s->n_cand);
         tp_set_error("tick cap reached: unfinished candidates carry TOPAY_LBFGSERR_TICK_CAP");
     }
     cudaEventRecord(s->ev_end, q);
@@ -859,6 +850,26 @@ extern "C" int topay_solver_run(topay_solver* s) {
     return TOPAY_OK;
 }
 
+// Entry c of `out` from a candidate's final state and its piece durations T[0..N); returns the trajectory's duration
+// (summed in piece order).
+static double fill_result(topay_result_batch* out, int c, const TpCandState& st, const double* T) {
+    double dur = 0.0;
+    for (int i = 0; i < st.N; i++) dur += T[i];
+    out->status[c] = st.status;
+    if (out->lbfgs_code) out->lbfgs_code[c] = st.last_code;
+    if (out->piece_num) out->piece_num[c] = st.N;
+    if (out->iters) out->iters[c] = st.iters_total;
+    if (out->evals) out->evals[c] = st.evals_total;
+    if (out->alm_rounds) out->alm_rounds[c] = st.alm_round;
+    if (out->cost) out->cost[c] = st.cost;
+    if (out->duration) out->duration[c] = dur;
+    if (out->final_xy_err) {
+        out->final_xy_err[2 * c] = st.final_xy[0];
+        out->final_xy_err[2 * c + 1] = st.final_xy[1];
+    }
+    return dur;
+}
+
 extern "C" int topay_solver_download(topay_solver* s, topay_result_batch* out, int32_t* best_by_duration,
                                      int32_t* best_by_cost) {
     if (!s || !out || !out->status || s->n_cand < 1) return TOPAY_ERR_INVALID_ARG;
@@ -873,20 +884,7 @@ extern "C" int topay_solver_download(topay_solver* s, topay_result_batch* out, i
     double bdv = 0, bcv = 0;
     int64_t evals = 0;
     for (int c = 0; c < n; c++) {
-        double dur = 0.0;
-        for (int i = 0; i < st[c].N; i++) dur += T[(size_t)c * NP + i];
-        out->status[c] = st[c].status;
-        if (out->lbfgs_code) out->lbfgs_code[c] = st[c].last_code;
-        if (out->piece_num) out->piece_num[c] = st[c].N;
-        if (out->iters) out->iters[c] = st[c].iters_total;
-        if (out->evals) out->evals[c] = st[c].evals_total;
-        if (out->alm_rounds) out->alm_rounds[c] = st[c].alm_round;
-        if (out->cost) out->cost[c] = st[c].cost;
-        if (out->duration) out->duration[c] = dur;
-        if (out->final_xy_err) {
-            out->final_xy_err[2 * c] = st[c].final_xy[0];
-            out->final_xy_err[2 * c + 1] = st[c].final_xy[1];
-        }
+        const double dur = fill_result(out, c, st[c], &T[(size_t)c * NP]);
         evals += st[c].evals_total;
         if (st[c].status == 1) {
             // planner.cpp:999-1010: first success, replaced only by a strictly shorter duration
@@ -1066,20 +1064,7 @@ extern "C" int topay_solver_download_candidate(topay_solver* s, int cand, topay_
     std::vector<double> xs(out->x ? D.xs : 0);
     if (out->x) TP_CUDA_OK(cudaMemcpyAsync(xs.data(), D.res_x + (size_t)cand * D.xs, (size_t)D.xs * 8, cudaMemcpyDeviceToHost, s->stream), {});
     TP_CUDA_OK(cudaStreamSynchronize(s->stream), {});
-    double dur = 0.0;
-    for (int i = 0; i < st.N; i++) dur += T[i];
-    out->status[0] = st.status;
-    if (out->lbfgs_code) out->lbfgs_code[0] = st.last_code;
-    if (out->piece_num) out->piece_num[0] = st.N;
-    if (out->iters) out->iters[0] = st.iters_total;
-    if (out->evals) out->evals[0] = st.evals_total;
-    if (out->alm_rounds) out->alm_rounds[0] = st.alm_round;
-    if (out->cost) out->cost[0] = st.cost;
-    if (out->duration) out->duration[0] = dur;
-    if (out->final_xy_err) {
-        out->final_xy_err[0] = st.final_xy[0];
-        out->final_xy_err[1] = st.final_xy[1];
-    }
+    fill_result(out, 0, st, T.data());
     if (out->T) memcpy(out->T, T.data(), (size_t)NP * 8);
     if (out->x) memcpy(out->x, xs.data(), (size_t)st.n * 8);
     return TOPAY_OK;
@@ -1157,7 +1142,9 @@ extern "C" int topay_solver_debug_direction(topay_solver* s, int n_vars, int bou
     TP_CUDA_OK(cudaMemcpy(D.list + (size_t)TP_TICKS * D.n_slots, &zero, sizeof(int32_t), cudaMemcpyHostToDevice), {});
     TP_CUDA_OK(cudaMemcpy(D.count + TP_TICKS, &one, sizeof(int32_t), cudaMemcpyHostToDevice), {});
     TP_CUDA_OK(cudaMemcpy(D.queue, queue, sizeof(queue), cudaMemcpyHostToDevice), {});
-    launch_cand(s, TP_MODE_ADVANCE, TP_TICKS, -1, 1);
+    TpLaunches launches;
+    launch_cand(s, s->lane[0], TP_MODE_ADVANCE, TP_TICKS, -1, 1, launches);
+    launches.add_to(s->stats);
     TP_CUDA_OK(cudaStreamSynchronize(q), {});
     TP_CUDA_OK(cudaGetLastError(), {});
     s->n_cand = 0;   // not a solvable upload

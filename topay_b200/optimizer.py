@@ -187,8 +187,9 @@ class MomaTrajOpt:
     def run(self):
         _lib.check(self._l.topay_solver_run(self.h), "topay_solver_run")
 
-    def download(self):
-        n, NP = self._n, self.max_pieces
+    def _result_arrays(self, n):
+        """Result arrays for n candidates and the ResultBatch that points the library at them."""
+        NP = self.max_pieces
         r = dict(status=np.zeros(n, np.int32), lbfgs_code=np.zeros(n, np.int32), piece_num=np.zeros(n, np.int32),
                  iters=np.zeros(n, np.int32), evals=np.zeros(n, np.int32), alm_rounds=np.zeros(n, np.int32),
                  cost=np.zeros(n), duration=np.zeros(n), T=np.zeros((n, NP)), coeff=np.zeros((n, 6 * NP, 9)),
@@ -196,6 +197,10 @@ class MomaTrajOpt:
         rb = ResultBatch(*[_p(r[k], C.c_int32 if r[k].dtype == np.int32 else C.c_double) for k in
                            ("status", "lbfgs_code", "piece_num", "iters", "evals", "alm_rounds", "cost", "duration",
                             "T", "coeff", "final_xy_err", "x")])
+        return r, rb
+
+    def download(self):
+        r, rb = self._result_arrays(self._n)
         bd, bc = C.c_int32(-1), C.c_int32(-1)
         _lib.check(self._l.topay_solver_download(self.h, C.byref(rb), C.byref(bd), C.byref(bc)), "download")
         r["best_by_duration"], r["best_by_cost"] = bd.value, bc.value
@@ -216,14 +221,7 @@ class MomaTrajOpt:
 
     def download_candidate(self, cand):
         """Results of one candidate of the last run (the winner): 28 KB at 64 pieces instead of the whole batch."""
-        NP = self.max_pieces
-        r = dict(status=np.zeros(1, np.int32), lbfgs_code=np.zeros(1, np.int32), piece_num=np.zeros(1, np.int32),
-                 iters=np.zeros(1, np.int32), evals=np.zeros(1, np.int32), alm_rounds=np.zeros(1, np.int32),
-                 cost=np.zeros(1), duration=np.zeros(1), T=np.zeros((1, NP)), coeff=np.zeros((1, 6 * NP, 9)),
-                 final_xy_err=np.zeros((1, 2)), x=np.zeros((1, num_vars(NP))))
-        rb = ResultBatch(*[_p(r[k], C.c_int32 if r[k].dtype == np.int32 else C.c_double) for k in
-                           ("status", "lbfgs_code", "piece_num", "iters", "evals", "alm_rounds", "cost", "duration",
-                            "T", "coeff", "final_xy_err", "x")])
+        r, rb = self._result_arrays(1)
         _lib.check(self._l.topay_solver_download_candidate(self.h, int(cand), C.byref(rb)), "download_candidate")
         out = {k: v[0] for k, v in r.items()}
         out["index"] = int(cand)
