@@ -165,7 +165,8 @@ def test_tick_cap_marks_unfinished_candidates(gpu_scene, monkeypatch, lanes):
 def test_scenarios_with_their_own_fields_share_one_solve():
     """BASELINE configs[4]: the candidates of several scenarios, each with its own field, in ONE upload
     (topay_solver_assign_fields). Every scenario's winner, trajectory and gate verdicts are bit-identical to solving that
-    scenario alone against its field — also when the plans are handed over in another order and with two lanes."""
+    scenario alone against its field — also when the plans are handed over in another order. (16 slots run as one
+    lane; test_gpu_launch_paths.py::test_sweep_pool_in_two_split_lanes runs a sweep in two lanes.)"""
     import topay_b200 as tp
     from topay_b200 import scenes
     opt, rp = tp.opt_params_default(), tp.robot_params_default()

@@ -4,10 +4,12 @@
   golden fixture, incl. empty / full / ragged grids and the accumulate-critical quirk;
 * queries: value and gradient against the oracle (<= 1e-12 absolute; FMA contraction only);
 * one cost/gradient evaluation: <= 1e-9 relative (north_star tolerance) on cost, 13 term costs,
-  gradient and spline coefficients, both stages, K in {5, 12, 32}, ragged piece counts in a batch;
+  gradient and spline coefficients, both stages, K in {1, 2, 3, 4, 5, 8, 12, 16, 31, 32}, ragged piece counts in a
+  batch, candidates of 33..64 pieces;
 * batched solve: identical line-search decisions and f within 1e-9 over the first accepted
   iterations; final cost / duration inside the reference algorithm's own sensitivity band
-  (DESIGN.md "final-trajectory tolerance"); end-point constraint met; selection rule.
+  (DESIGN.md "final-trajectory tolerance"); end-point constraint met; selection rule. Also in timed mode, whose
+  plain launches always split k_cand into its three halves: bit-identical to the graph-mode solve.
 """
 import os
 
@@ -153,20 +155,14 @@ def _eval_batch(solver, stage, prep, xs, lam, rho):
                            [q["init_inner_xy"] for q in prep], xs, lam, rho)
 
 
-@pytest.mark.parametrize("K", [12, 32, 5, 16])
-def test_eval_parity(gpu_scene, small_scene, oracle, K):
+def _check_eval_against_oracle(solver, of, oracle, opt, rp, prep, seed):
+    """One evaluation of every candidate of `prep`, both stages, against the oracle; returns the worst relative
+    deviation."""
     import topay_b200 as tp
-    from topay_b200 import scenes
-    of = small_scene["field"]
-    opt, rp = tp.opt_params_default(), tp.robot_params_default()
-    opt.int_K = K
-    paths, bv, ba = scenes.short_candidates(6, 100 + K)      # ragged: 3..10 pieces in one batch
-    prep = [tp.prepare_candidate(opt, rp, p, bv[0], ba[0], 16) for p in paths]
-    assert len({q["piece_num"] for q in prep}) > 1
-    rng = np.random.default_rng(K)
+    n_c = len(prep)
+    rng = np.random.default_rng(seed)
     xs = [q["x0"] + 0.05 * rng.normal(size=len(q["x0"])) for q in prep]
-    solver = tp.MomaTrajOpt(gpu_scene, max_cand=8, max_pieces=16, opt_param=opt, robot=rp)
-    lam, rho = np.tile([30.0, -20.0], (6, 1)), np.tile([1e4, 2e4], (6, 1))
+    lam, rho = np.tile([30.0, -20.0], (n_c, 1)), np.tile([1e4, 2e4], (n_c, 1))
     worst = 0.0
     for stage in (1, 2):
         ev = _eval_batch(solver, stage, prep, xs, lam, rho)
@@ -182,7 +178,43 @@ def test_eval_parity(gpu_scene, small_scene, oracle, K):
             worst = max(worst, *e)
             assert e[0] <= 1e-10 and e[1] <= 1e-9 and e[2] <= 1e-9 and e[3] <= 1e-9, (stage, c, e)
             assert np.abs(ev["final_xy"][c] - fxy).max() <= 1e-12
+    return worst
+
+
+# K-hat = 4 (K 1..4: eight pieces per warp, 16 values per lane in the transpose-reduce, lane K-hat - 1 owns gdT),
+# K-hat = 8 with and without end-node warps (8, 5), K-hat = 16 (12, 16), K-hat = 32 with and without them (32, 31)
+@pytest.mark.parametrize("K", [12, 32, 5, 16, 1, 2, 3, 4, 8, 31])
+def test_eval_parity(gpu_scene, small_scene, oracle, K):
+    import topay_b200 as tp
+    from topay_b200 import scenes
+    opt, rp = tp.opt_params_default(), tp.robot_params_default()
+    opt.int_K = K
+    paths, bv, ba = scenes.short_candidates(6, 100 + K)      # ragged: 3..10 pieces in one batch
+    prep = [tp.prepare_candidate(opt, rp, p, bv[0], ba[0], 16) for p in paths]
+    assert len({q["piece_num"] for q in prep}) > 1
+    solver = tp.MomaTrajOpt(gpu_scene, max_cand=8, max_pieces=16, opt_param=opt, robot=rp)
+    worst = _check_eval_against_oracle(solver, small_scene["field"], oracle, opt, rp, prep, K)
     print(f"K={K}: worst relative deviation from the oracle {worst:.2e}")
+
+
+@pytest.mark.parametrize("K", [4, 16, 31, 32])
+def test_eval_parity_long_candidates(gpu_scene, small_scene, oracle, K):
+    """Long candidates in one ragged batch (33, 40 and 64 pieces at max_pieces = 64), both stages: more than 32 pieces
+    put the end nodes of K = K-hat on two warps, K-hat = 4 runs 8 piece groups per candidate, and stage 1 runs at
+    64 pieces, which the short candidates above never reach."""
+    import topay_b200 as tp
+    from topay_b200 import scenes
+    opt, rp = tp.opt_params_default(), tp.robot_params_default()
+    opt.int_K, opt.sample_interval = K, 1e9
+    paths, bv, ba = scenes.synthetic_batch(3, 1234 + K)
+    prep = []
+    for p, pieces in zip(paths, (33, 40, 64)):
+        opt.min_piece_num = pieces
+        prep.append(tp.prepare_candidate(opt, rp, p, bv[0], ba[0], 64))
+    assert [q["piece_num"] for q in prep] == [33, 40, 64]
+    solver = tp.MomaTrajOpt(gpu_scene, max_cand=3, max_pieces=64, opt_param=opt, robot=rp)
+    worst = _check_eval_against_oracle(solver, small_scene["field"], oracle, opt, rp, prep, K)
+    print(f"K={K}, 33..64 pieces: worst relative deviation from the oracle {worst:.2e}")
 
 
 def test_eval_golden_and_full_size(gpu_scene, small_scene, oracle):
@@ -221,7 +253,21 @@ def test_eval_golden_and_full_size(gpu_scene, small_scene, oracle):
     assert np.abs(slope - ev["final_xy"].sum(axis=1) - 0.5 * 5.0 * (2.0 / 1e4)).max() <= 1e-6 * (1 + np.abs(slope).max())
 
 
+RESULT_KEYS = ("status", "lbfgs_code", "evals", "iters", "alm_rounds", "cost", "T", "coeff", "x", "final_xy_err")
+
+
 def test_solve_trace_and_band(gpu_scene, small_scene, oracle):
+    _solve_trace_and_band(gpu_scene, small_scene, oracle, timed=False)
+
+
+def test_solve_trace_and_band_timed(gpu_scene, small_scene, oracle):
+    """Timed mode: per-launch CUDA events and plain launches, which always run k_cand as three launches (adjoint,
+    L-BFGS, generate) handing their state over through global memory; graph mode runs this pool as one fused launch.
+    Both must replay the oracle, and the timed solve must equal the graph-mode one bit for bit."""
+    _solve_trace_and_band(gpu_scene, small_scene, oracle, timed=True)
+
+
+def _solve_trace_and_band(gpu_scene, small_scene, oracle, timed):
     import topay_b200 as tp
     z = np.load(os.path.join(G, "solve_cases.npz"))
     n = int(z["n"])
@@ -230,6 +276,18 @@ def test_solve_trace_and_band(gpu_scene, small_scene, oracle):
     solver = tp.MomaTrajOpt(gpu_scene, max_cand=n, max_pieces=16, opt_param=opt, robot=rp)
     solver.set_trace(4000)
     res = solver.optimizeTrajBatch(paths, np.zeros((n, 10, 2)), np.zeros((n, 10, 2)))
+    if timed:
+        graph = res
+        graph_trace = [solver.trace(c) for c in range(n)]
+        solver.set_timed(True)
+        res = solver.optimizeTrajBatch(paths, np.zeros((n, 10, 2)), np.zeros((n, 10, 2)))
+        st = solver.stats()
+        # one lane; every batch split: k_list_roll + 16 ticks x (3 evaluation kernels + 3 halves of k_cand)
+        assert st["eval_launches"] == st["ticks"] and st["kernel_launches"] == 2 + 97 * st["ticks"] // 16, st
+        for k in RESULT_KEYS:
+            assert np.array_equal(res[k], graph[k]), k
+        for c in range(n):
+            assert np.array_equal(solver.trace(c), graph_trace[c]), c
     for c in range(n):
         assert res["status"][c] == int(z[f"s{c}_status"]) == 1
         assert res["piece_num"][c] == int(z[f"s{c}_piece_num"])
