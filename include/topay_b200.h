@@ -230,7 +230,10 @@ int topay_field_line_visible(topay_field* f, const double* p1, const double* p2,
 int topay_field_same_topo_paths(topay_field* f, const double* pts, const int32_t* offsets, int n_paths,
                                 const int32_t* pairs, int n_pairs, double thresh, int use_critical, int8_t* same);
 /* Same queries with DEVICE pointers (inputs and outputs already in HBM), asynchronous
- * on the field's stream; used by the resident benchmark and by the solver. */
+ * on the field's stream; used by the resident benchmark and by the solver. The launch goes to
+ * the field's own non-blocking stream and is not ordered after any work the caller queued on
+ * its streams: the caller must synchronise the stream that wrote pos_dev (or the device)
+ * before the call, and call topay_field_sync before it reads dist_dev / grad_dev. */
 int topay_field_query3d_dev(topay_field* f, const double* pos_dev, int64_t n, double* dist_dev,
                             double* grad_dev);
 int topay_field_sync(topay_field* f);
@@ -484,8 +487,9 @@ typedef struct topay_result_batch {
     int32_t* alm_rounds;    /* [n] */
     double*  cost;          /* [n] traj_cost (moma_traj_opt.cpp:495) */
     double*  duration;      /* [n] sum of piece durations of the returned trajectory */
-    double*  T;             /* [n][max_pieces] */
-    double*  coeff;         /* [n][6*max_pieces][9] minco coefficients of the last evaluation */
+    double*  T;             /* [n][max_pieces], zero past piece_num */
+    double*  coeff;         /* [n][6*max_pieces][9] minco coefficients of the last evaluation, rows past
+                               6*piece_num zero */
     double*  final_xy_err;  /* [n][2] */
     double*  x;             /* [n][10*max_pieces-8] final variables */
 } topay_result_batch;

@@ -13,10 +13,45 @@ def harness(oracle, small_scene):
     return HH.Harness(oracle.opt_defaults(), oracle.robot_defaults(), small_scene["desc"], small_scene["field"])
 
 
+@pytest.fixture(scope="module")
+def fields(oracle, small_scene):
+    """name -> (oracle field, grid_desc, min_boundary, max_boundary, dims): the default grid with its cuboid scene, and
+    the non-square grids A (134 x 80 x 13 @ 0.1) and D (7 x 300 x 5 @ 0.1) of test_gpu_grid_geometry.py with random
+    occupancy. On a square grid a transposed stride or an x bound used for y goes unseen."""
+    from test_gpu_grid_geometry import grid_spec, random_occupancy
+    out = {"default": (small_scene["field"], small_scene["desc"], np.array([-10.0, -10.0, 0.0]),
+                       np.array([10.0, 10.0, 1.6]), (200, 200, 16))}
+    for name in ("A", "D"):
+        desc, lo, hi = grid_spec(name)
+        f = oracle.Field(desc)
+        f.set_occupancy(*random_occupancy(f.dims, 23))
+        f.rebuild()
+        out[name] = (f, desc, lo, hi, f.dims)
+    return out
+
+
+def _grid(oracle, fields, name):
+    f, desc, lo, hi, dims = fields[name]
+    return f, HH.Harness(oracle.opt_defaults(), oracle.robot_defaults(), desc, f), lo, hi, desc.resolution, dims
+
+
 def test_queries_bit_exact(oracle, small_scene, harness):
     f = small_scene["field"]
     rng = np.random.default_rng(0)
     pos = rng.uniform([-10.5, -10.5, -0.2], [10.5, 10.5, 1.8], (20000, 3))
+    _check_queries(f, harness, pos)
+
+
+@pytest.mark.parametrize("grid", ["A", "D"])
+def test_queries_bit_exact_on_other_grids(oracle, fields, grid):
+    """test_queries_bit_exact on the non-square grids, over the map +-5 cells in x and y and +-2 cells in z."""
+    f, harness, lo, hi, res, _ = _grid(oracle, fields, grid)
+    rng = np.random.default_rng(0)
+    pos = rng.uniform(lo - [5 * res, 5 * res, 2 * res], hi + [5 * res, 5 * res, 2 * res], (20000, 3))
+    _check_queries(f, harness, pos)
+
+
+def _check_queries(f, harness, pos):
     d0, g0 = f.query3d(pos)
     d1, g1 = harness.query3d(pos)
     assert np.array_equal(d0, d1) and np.array_equal(g0, g1)
@@ -37,13 +72,15 @@ def test_fk_and_linear_time_adjoint(oracle, harness):
         assert np.abs(a - b).max() <= 1e-13 * np.abs(a).max()
 
 
-@pytest.mark.parametrize("K", [12, 32, 5])
-def test_penalty_dataflow(oracle, small_scene, K):
+@pytest.mark.parametrize("grid,K", [pytest.param("default", K, id=str(K)) for K in (12, 32, 5)] +
+                         [pytest.param("A", K, id=f"A-{K}") for K in (12, 32, 5)])
+def test_penalty_dataflow(oracle, fields, grid, K):
     rp, opt = oracle.robot_defaults(), oracle.opt_defaults()
     opt.int_K = K
-    f = small_scene["field"]
-    H = HH.Harness(opt, rp, small_scene["desc"], f)
+    f, desc = fields[grid][:2]
+    H = HH.Harness(opt, rp, desc, f)
     rng = np.random.default_rng(K)
+    # on grid A (13.4 x 8 m) the candidates' 3-8 m spans cross the map's edges
     paths, bv, ba = scenes.short_candidates(3, 11)
     lam, rho = np.array([30.0, -20.0]), np.array([1e4, 2e4])
     for p in paths:
@@ -107,6 +144,24 @@ def test_field_predicates_bit_exact(oracle, small_scene, harness):
     p2, q2 = rng.uniform(-10.3, 10.3, (n, 2)), rng.uniform(-10.3, 10.3, (n, 2))
     p3 = np.concatenate([rng.uniform(-10.3, 10.3, (n, 2)), rng.uniform(-0.2, 1.8, (n, 1))], axis=1)
     idx = rng.integers(-5, 206, (n, 2))
+    _check_predicates(f, harness, p2, q2, p3, idx)
+
+
+@pytest.mark.parametrize("grid", ["A", "D"])
+def test_field_predicates_bit_exact_on_other_grids(oracle, fields, grid):
+    """test_field_predicates_bit_exact on the non-square grids: positions over the map +-3 cells (z +-2 cells), cell
+    indices -5 .. max(dims) + 5 on both axes."""
+    f, harness, lo, hi, res, dims = _grid(oracle, fields, grid)
+    rng = np.random.default_rng(8)
+    n = 5000
+    p2, q2 = rng.uniform(lo[:2] - 3 * res, hi[:2] + 3 * res, (n, 2)), rng.uniform(lo[:2] - 3 * res, hi[:2] + 3 * res, (n, 2))
+    p3 = np.concatenate([rng.uniform(lo[:2] - 3 * res, hi[:2] + 3 * res, (n, 2)),
+                         rng.uniform(lo[2] - 2 * res, hi[2] + 2 * res, (n, 1))], axis=1)
+    idx = rng.integers(-5, max(dims) + 6, (n, 2))
+    _check_predicates(f, harness, p2, q2, p3, idx)
+
+
+def _check_predicates(f, harness, p2, q2, p3, idx):
     for thr, crit in ((0.0, False), (0.3, True)):
         c2, c3, line, cd, ci = HH.field_misc(harness, p2, q2, p3, idx, thr, crit)
         assert np.array_equal(c2, f.is_collision(p2, thr)) and np.array_equal(c3, f.is_collision(p3, thr))

@@ -870,6 +870,15 @@ static double fill_result(topay_result_batch* out, int c, const TpCandState& st,
     return dur;
 }
 
+// A store row holds its candidate's N pieces; the entries past them are whatever an earlier upload's candidate of that
+// row left there. They leave the library as zeros, so that a candidate's result does not depend on what the solver
+// ran before.
+static void clear_tail(topay_result_batch* out, int c, int N, int NP) {
+    if (out->T) std::fill(out->T + (size_t)c * NP + N, out->T + (size_t)(c + 1) * NP, 0.0);
+    if (out->coeff)
+        std::fill(out->coeff + ((size_t)c * 6 * NP + 6 * N) * 9, out->coeff + (size_t)(c + 1) * 6 * NP * 9, 0.0);
+}
+
 extern "C" int topay_solver_download(topay_solver* s, topay_result_batch* out, int32_t* best_by_duration,
                                      int32_t* best_by_cost) {
     if (!s || !out || !out->status || s->n_cand < 1) return TOPAY_ERR_INVALID_ARG;
@@ -907,6 +916,7 @@ extern "C" int topay_solver_download(topay_solver* s, topay_result_batch* out, i
         const int xstride = topay_num_vars(NP);
         for (int c = 0; c < n; c++) memcpy(out->x + (size_t)c * xstride, &xs[(size_t)c * D.xs], st[c].n * 8);
     }
+    for (int c = 0; c < n; c++) clear_tail(out, c, st[c].N, NP);
     if (best_by_duration) *best_by_duration = bd;
     if (best_by_cost) *best_by_cost = bc;
     return TOPAY_OK;
@@ -1066,6 +1076,7 @@ extern "C" int topay_solver_download_candidate(topay_solver* s, int cand, topay_
     TP_CUDA_OK(cudaStreamSynchronize(s->stream), {});
     fill_result(out, 0, st, T.data());
     if (out->T) memcpy(out->T, T.data(), (size_t)NP * 8);
+    clear_tail(out, 0, st.N, NP);
     if (out->x) memcpy(out->x, xs.data(), (size_t)st.n * 8);
     return TOPAY_OK;
 }
