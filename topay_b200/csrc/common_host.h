@@ -1,4 +1,7 @@
-// Host-side helpers shared by field.cu, edt.cu, rogfield.cu and solver.cu.
+// Host-side helpers shared by the library's objects. Two of them carry every copy between host and device:
+// TpStaging stages one batched call (per-call scratch from the stream-ordered allocator, copies in, copies back,
+// one synchronise of the object's stream), and tp_download is a single download on the object's stream.
+// TpDevBuffers owns an object's device buffers.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -6,6 +9,7 @@
 #include <map>
 #include <mutex>
 #include <string>
+#include <vector>
 
 #include "hd.cuh"
 
@@ -16,6 +20,9 @@ int tp_require_device(int device);
 
 int tp_field_device(const topay_field* f);
 bool tp_field_ready(const topay_field* f);
+// TOPAY_OK when the dense field has been rebuilt since its occupancy last changed, else TOPAY_ERR_NOT_READY with the
+// error text set: the one readiness check of every entry point that reads the field.
+int tp_field_require_ready(const topay_field* f);
 void tp_field_grid(const topay_field* f, TpGrid* out);
 int tp_rogfield_device(const topay_rogfield* f);
 bool tp_rogfield_ready(const topay_rogfield* f);
@@ -64,18 +71,110 @@ inline void tp_pool_keep(int device) {
     }
 }
 
-// cudaMalloc of `count` elements (at least one). On failure *p is null, the error text is set and the result is
-// TOPAY_ERR_ALLOC.
-template <typename T>
-int tp_dev_malloc(T** p, size_t count) {
-    cudaError_t e = cudaMalloc((void**)p, std::max<size_t>(count, 1) * sizeof(T));
+// The staging of one batched call on an object's stream. in() copies a host array to new device scratch, out()
+// allocates scratch that finish() copies back, inout() does both; a null host pointer gives a null device pointer.
+// The first failure is kept with its text (TOPAY_ERR_ALLOC for an allocation, TOPAY_ERR_CUDA for a copy) and every
+// later step does nothing, so the caller launches only while ok(). The scratch is freed on the stream on every path.
+class TpStaging {
+  public:
+    explicit TpStaging(cudaStream_t q) : q_(q) {}
+    TpStaging(const TpStaging&) = delete;
+    TpStaging& operator=(const TpStaging&) = delete;
+    ~TpStaging() {
+        for (const Buf& b : bufs_) cudaFreeAsync(b.dev, q_);
+    }
+    template <typename T>
+    T* in(const T* host, size_t count) { return (T*)stage((void*)host, count * sizeof(T), true, false); }
+    template <typename T>
+    T* out(T* host, size_t count) { return (T*)stage(host, count * sizeof(T), false, true); }
+    template <typename T>
+    T* inout(T* host, size_t count) { return (T*)stage(host, count * sizeof(T), true, true); }
+    bool ok() const { return rc_ == TOPAY_OK; }
+    // Copies the outputs back, waits for the stream and collects a failed launch; returns the call's status.
+    int finish() {
+        for (const Buf& b : bufs_)
+            if (b.back && rc_ == TOPAY_OK)
+                fail(cudaMemcpyAsync(b.host, b.dev, b.bytes, cudaMemcpyDeviceToHost, q_), "copy back");
+        const cudaError_t e = cudaStreamSynchronize(q_);
+        if (rc_ == TOPAY_OK) fail(e, "cudaStreamSynchronize");
+        const cudaError_t l = cudaGetLastError();
+        if (rc_ == TOPAY_OK) fail(l, "kernel launch");
+        return rc_;
+    }
+
+  private:
+    struct Buf {
+        void* dev;
+        void* host;
+        size_t bytes;
+        bool back;
+    };
+    void* stage(void* host, size_t bytes, bool copy_in, bool back) {
+        if (!host || rc_ != TOPAY_OK) return nullptr;
+        void* dev = nullptr;
+        const cudaError_t e = cudaMallocAsync(&dev, std::max<size_t>(bytes, 1), q_);
+        if (e != cudaSuccess) {
+            tp_set_error(std::string("cudaMallocAsync failed: ") + cudaGetErrorString(e));
+            rc_ = TOPAY_ERR_ALLOC;
+            return nullptr;
+        }
+        bufs_.push_back(Buf{dev, host, bytes, back});
+        if (copy_in) fail(cudaMemcpyAsync(dev, host, bytes, cudaMemcpyHostToDevice, q_), "copy in");
+        return rc_ == TOPAY_OK ? dev : nullptr;
+    }
+    void fail(cudaError_t e, const char* what) {
+        if (e == cudaSuccess || rc_ != TOPAY_OK) return;
+        tp_set_error(std::string(what) + ": " + cudaGetErrorString(e));
+        rc_ = TOPAY_ERR_CUDA;
+    }
+    cudaStream_t q_;
+    std::vector<Buf> bufs_;
+    int rc_ = TOPAY_OK;
+};
+
+// Copies `bytes` from the device to the host on `q` and waits for `q`: the host reads `dst` on return.
+inline int tp_download(cudaStream_t q, void* dst, const void* src, size_t bytes) {
+    cudaError_t e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, q);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(q);
     if (e != cudaSuccess) {
-        tp_set_error(std::string("cudaMalloc failed: ") + cudaGetErrorString(e));
-        *p = nullptr;
-        return TOPAY_ERR_ALLOC;
+        tp_set_error(std::string("download: ") + cudaGetErrorString(e));
+        return TOPAY_ERR_CUDA;
     }
     return TOPAY_OK;
 }
+
+// The device buffers of one long-lived object (dense field, ROG ring, probability map, solver). alloc() gives
+// `count` elements (at least one), zeroed on the object's stream; the first failure is kept with its text and later
+// allocations do nothing, so a constructor checks status once. Every buffer is freed with the owner.
+struct TpDevBuffers {
+    cudaStream_t stream = nullptr;
+    int status = TOPAY_OK;
+    std::vector<void*> ptrs;
+    TpDevBuffers() = default;
+    TpDevBuffers(const TpDevBuffers&) = delete;
+    TpDevBuffers& operator=(const TpDevBuffers&) = delete;
+    ~TpDevBuffers() {
+        for (void* p : ptrs) cudaFree(p);
+    }
+    template <typename T>
+    int alloc(T** p, size_t count) {
+        *p = nullptr;
+        if (status != TOPAY_OK) return status;
+        const size_t bytes = std::max<size_t>(count, 1) * sizeof(T);
+        cudaError_t e = cudaMalloc((void**)p, bytes);
+        if (e != cudaSuccess) {
+            *p = nullptr;
+            tp_set_error(std::string("cudaMalloc failed: ") + cudaGetErrorString(e));
+            return status = TOPAY_ERR_ALLOC;
+        }
+        ptrs.push_back(*p);
+        if ((e = cudaMemsetAsync(*p, 0, bytes, stream)) != cudaSuccess) {
+            tp_set_error(std::string("cudaMemsetAsync: ") + cudaGetErrorString(e));
+            return status = TOPAY_ERR_CUDA;
+        }
+        return TOPAY_OK;
+    }
+};
 
 // Raises `kernel`'s max dynamic shared memory to at least `bytes`. The attribute belongs to the kernel, not to one
 // solver or field, and objects of different sizes coexist in a process (bench: 64-piece plans next to 16-piece latency

@@ -65,10 +65,16 @@ struct topay_field {
     bool ready;
     cudaEvent_t ev0, ev1, ev2;
     float ms_total, ms_3d;
+    TpDevBuffers bufs;
 };
 
 int tp_field_device(const topay_field* f) { return f->device; }
 bool tp_field_ready(const topay_field* f) { return f->ready; }
+int tp_field_require_ready(const topay_field* f) {
+    if (f->ready) return TOPAY_OK;
+    tp_set_error("field not built: call topay_field_rebuild first");
+    return TOPAY_ERR_NOT_READY;
+}
 void tp_field_grid(const topay_field* f, TpGrid* out) { *out = f->grid; }
 
 // ------------------------------------------------------------------ kernels
@@ -234,7 +240,6 @@ extern "C" int topay_field_create(const topay_grid_desc* desc, int device, topay
     int rc = tp_require_device(device);
     if (rc != TOPAY_OK) return rc;
     topay_field* f = new topay_field();
-    memset(f, 0, sizeof(*f));
     f->desc = *desc;
     f->device = device;
     f->keep_sq = true;
@@ -265,35 +270,27 @@ extern "C" int topay_field_create(const topay_grid_desc* desc, int device, topay
     f->n2 = (size_t)f->nx * f->ny;
     f->n3 = f->n2 * f->nz;
     TP_CUDA_OK(cudaStreamCreateWithFlags(&f->stream, cudaStreamNonBlocking), { delete f; });
-#define FA(p, n)                                        \
-    if ((rc = tp_dev_malloc(&(p), (n))) != TOPAY_OK) {  \
-        topay_field_destroy(f);                         \
-        return rc;                                      \
+    TpDevBuffers& b = f->bufs;
+    b.stream = f->stream;
+    b.alloc(&f->occ3d, f->n3);
+    b.alloc(&f->occ2d, f->n2);
+    b.alloc(&f->occ2d_crit, f->n2);
+    b.alloc(&f->src2d, f->n2);
+    b.alloc(&f->esdf3d, f->n3);
+    b.alloc(&f->esdf2d, f->n2);
+    b.alloc(&f->esdf2d_inflate, f->n2);
+    b.alloc(&f->esdf2d_crit, f->n2);
+    b.alloc(&f->packed16, f->n3);
+    b.alloc(&f->packed32, f->n3);
+    for (int w = 0; w < 4; w++) {
+        b.alloc(&f->sq_pos[w], w < 3 ? f->n2 : f->n3);
+        b.alloc(&f->sq_neg[w], w < 3 ? f->n2 : f->n3);
     }
-    FA(f->occ3d, f->n3);
-    FA(f->occ2d, f->n2);
-    FA(f->occ2d_crit, f->n2);
-    FA(f->src2d, f->n2);
-    FA(f->esdf3d, f->n3);
-    FA(f->esdf2d, f->n2);
-    FA(f->esdf2d_inflate, f->n2);
-    FA(f->esdf2d_crit, f->n2);
-    FA(f->packed16, f->n3);
-    FA(f->packed32, f->n3);
-    for (int w = 0; w < 3; w++) {
-        FA(f->sq_pos[w], f->n2);
-        FA(f->sq_neg[w], f->n2);
+    if (b.status != TOPAY_OK) {
+        rc = b.status;
+        topay_field_destroy(f);
+        return rc;
     }
-    FA(f->sq_pos[3], f->n3);
-    FA(f->sq_neg[3], f->n3);
-#undef FA
-    cudaMemsetAsync(f->occ3d, 0, f->n3, f->stream);
-    cudaMemsetAsync(f->occ2d, 0, f->n2, f->stream);
-    cudaMemsetAsync(f->occ2d_crit, 0, f->n2, f->stream);
-    cudaMemsetAsync(f->esdf3d, 0, f->n3 * 8, f->stream);
-    cudaMemsetAsync(f->esdf2d, 0, f->n2 * 8, f->stream);
-    cudaMemsetAsync(f->esdf2d_inflate, 0, f->n2 * 8, f->stream);
-    cudaMemsetAsync(f->esdf2d_crit, 0, f->n2 * 8, f->stream);
     g.esdf3d = f->esdf3d;
     g.esdf2d = f->esdf2d;
     g.esdf2d_inflate = f->esdf2d_inflate;
@@ -311,11 +308,6 @@ extern "C" void topay_field_destroy(topay_field* f) {
     if (!f) return;
     cudaSetDevice(f->device);
     if (f->stream) cudaStreamSynchronize(f->stream);
-    void* ptrs[] = {f->occ3d, f->occ2d, f->occ2d_crit, f->src2d, f->esdf3d, f->esdf2d, f->esdf2d_inflate,
-                    f->esdf2d_crit, f->packed16, f->packed32, f->sq_pos[0], f->sq_pos[1], f->sq_pos[2],
-                    f->sq_pos[3], f->sq_neg[0], f->sq_neg[1], f->sq_neg[2], f->sq_neg[3]};
-    for (void* p : ptrs)
-        if (p) cudaFree(p);
     if (f->ev0) cudaEventDestroy(f->ev0);
     if (f->ev1) cudaEventDestroy(f->ev1);
     if (f->ev2) cudaEventDestroy(f->ev2);
@@ -366,14 +358,13 @@ extern "C" int topay_field_rasterize_points(topay_field* f, const float* xyz, in
     if (!f || (!xyz && n > 0) || n < 0) return TOPAY_ERR_INVALID_ARG;
     if (n == 0) return TOPAY_OK;
     cudaSetDevice(f->device);
-    float* d = nullptr;
-    TP_CUDA_OK(cudaMallocAsync(&d, (size_t)n * 3 * sizeof(float), f->stream), {});
-    TP_CUDA_OK(cudaMemcpyAsync(d, xyz, (size_t)n * 3 * sizeof(float), cudaMemcpyHostToDevice, f->stream),
-               { cudaFreeAsync(d, f->stream); });
-    k_rasterize<<<(unsigned)((n + 255) / 256), 256, 0, f->stream>>>(d, n, f->grid, f->desc.chassis_height, f->occ3d,
-                                                                  f->occ2d, f->occ2d_crit);
-    cudaFreeAsync(d, f->stream);
-    TP_CUDA_OK(cudaStreamSynchronize(f->stream), {});
+    TpStaging io(f->stream);
+    const float* d = io.in(xyz, (size_t)n * 3);
+    if (io.ok())
+        k_rasterize<<<(unsigned)((n + 255) / 256), 256, 0, f->stream>>>(d, n, f->grid, f->desc.chassis_height, f->occ3d,
+                                                                      f->occ2d, f->occ2d_crit);
+    const int rc = io.finish();
+    if (rc != TOPAY_OK) return rc;
     f->ready = false;
     f->grid.ready = 0;
     return TOPAY_OK;
@@ -423,36 +414,20 @@ extern "C" int topay_field_last_rebuild_ms(topay_field* f, float* ms_total, floa
 static int query_common(topay_field* f, const double* pos, int64_t n, int dim, int which, double* dist,
                         double* grad, int value_only) {
     if (!f || (!pos && n > 0) || !dist || n < 0) return TOPAY_ERR_INVALID_ARG;
-    if (!f->ready) {
-        tp_set_error("field not built: call topay_field_rebuild first");
-        return TOPAY_ERR_NOT_READY;
-    }
+    const int rc = tp_field_require_ready(f);
+    if (rc != TOPAY_OK) return rc;
     if (n == 0) return TOPAY_OK;
     cudaSetDevice(f->device);
-    double *dpos = nullptr, *dd = nullptr, *dg = nullptr;
-    TP_CUDA_OK(cudaMallocAsync(&dpos, (size_t)n * dim * 8, f->stream), {});
-    TP_CUDA_OK(cudaMallocAsync(&dd, (size_t)n * 8, f->stream), { cudaFreeAsync(dpos, f->stream); });
-    if (grad)
-        TP_CUDA_OK(cudaMallocAsync(&dg, (size_t)n * dim * 8, f->stream),
-                   { cudaFreeAsync(dpos, f->stream); cudaFreeAsync(dd, f->stream); });
-    cudaMemcpyAsync(dpos, pos, (size_t)n * dim * 8, cudaMemcpyHostToDevice, f->stream);
+    TpStaging io(f->stream);
+    const double* dpos = io.in(pos, (size_t)n * dim);
+    double* dd = io.out(dist, (size_t)n);
+    double* dg = io.out(grad, (size_t)n * dim);
     const unsigned blocks = (unsigned)((n + 255) / 256);
-    if (dim == 3)
-        k_query3d<<<blocks, 256, 0, f->stream>>>(f->grid, dpos, n, dd, dg, value_only);
-    else {
-        const double* buf = which == TOPAY_MAP2D_CRITICAL ? f->esdf2d_crit
-                            : which == TOPAY_MAP2D_INFLATE ? f->esdf2d_inflate : f->esdf2d;
-        k_query2d<<<blocks, 256, 0, f->stream>>>(f->grid, buf, dpos, n, dd, dg, value_only);
-    }
-    cudaMemcpyAsync(dist, dd, (size_t)n * 8, cudaMemcpyDeviceToHost, f->stream);
-    if (grad) cudaMemcpyAsync(grad, dg, (size_t)n * dim * 8, cudaMemcpyDeviceToHost, f->stream);
-    cudaFreeAsync(dpos, f->stream);
-    cudaFreeAsync(dd, f->stream);
-    if (dg) cudaFreeAsync(dg, f->stream);
-    cudaError_t e = cudaStreamSynchronize(f->stream);
-    TP_CUDA_OK(e, {});
-    TP_CUDA_OK(cudaGetLastError(), {});
-    return TOPAY_OK;
+    const double* buf = which == TOPAY_MAP2D_CRITICAL ? f->esdf2d_crit
+                        : which == TOPAY_MAP2D_INFLATE ? f->esdf2d_inflate : f->esdf2d;
+    if (io.ok() && dim == 3) k_query3d<<<blocks, 256, 0, f->stream>>>(f->grid, dpos, n, dd, dg, value_only);
+    if (io.ok() && dim == 2) k_query2d<<<blocks, 256, 0, f->stream>>>(f->grid, buf, dpos, n, dd, dg, value_only);
+    return io.finish();
 }
 
 extern "C" int topay_field_query3d(topay_field* f, const double* pos, int64_t n, double* dist, double* grad) {
@@ -473,7 +448,8 @@ extern "C" int topay_field_distance2d(topay_field* f, const double* pos, int64_t
 extern "C" int topay_field_query3d_dev(topay_field* f, const double* pos_dev, int64_t n, double* dist_dev,
                                        double* grad_dev) {
     if (!f || !pos_dev || !dist_dev || n < 0) return TOPAY_ERR_INVALID_ARG;
-    if (!f->ready) return TOPAY_ERR_NOT_READY;
+    const int rc = tp_field_require_ready(f);
+    if (rc != TOPAY_OK) return rc;
     if (n == 0) return TOPAY_OK;
     cudaSetDevice(f->device);
     k_query3d<<<(unsigned)((n + 255) / 256), 256, 0, f->stream>>>(f->grid, pos_dev, n, dist_dev, grad_dev, 0);
@@ -490,7 +466,8 @@ extern "C" int topay_field_sync(topay_field* f) {
 extern "C" int topay_field_whole_body_collision(topay_field* f, const topay_robot_params* robot,
                                                 const double* states, int64_t n, int8_t* out) {
     if (!f || !robot || (!states && n > 0) || !out || n < 0) return TOPAY_ERR_INVALID_ARG;
-    if (!f->ready) return TOPAY_ERR_NOT_READY;
+    const int rc = tp_field_require_ready(f);
+    if (rc != TOPAY_OK) return rc;
     if (n == 0) return TOPAY_OK;
     cudaSetDevice(f->device);
     TpParams P;
@@ -498,18 +475,11 @@ extern "C" int topay_field_whole_body_collision(topay_field* f, const topay_robo
     P.robot = *robot;
     topay_opt_params_default(&P.opt);
     tp_derive_params(P);
-    double* ds = nullptr;
-    int8_t* dout = nullptr;
-    TP_CUDA_OK(cudaMallocAsync(&ds, (size_t)n * 10 * 8, f->stream), {});
-    TP_CUDA_OK(cudaMallocAsync(&dout, (size_t)n, f->stream), { cudaFreeAsync(ds, f->stream); });
-    cudaMemcpyAsync(ds, states, (size_t)n * 10 * 8, cudaMemcpyHostToDevice, f->stream);
-    k_whole_body<<<(unsigned)((n + 127) / 128), 128, 0, f->stream>>>(f->grid, P, ds, n, dout);
-    cudaMemcpyAsync(out, dout, (size_t)n, cudaMemcpyDeviceToHost, f->stream);
-    cudaFreeAsync(ds, f->stream);
-    cudaFreeAsync(dout, f->stream);
-    cudaError_t e = cudaStreamSynchronize(f->stream);
-    TP_CUDA_OK(e, {});
-    return TOPAY_OK;
+    TpStaging io(f->stream);
+    const double* ds = io.in(states, (size_t)n * 10);
+    int8_t* dout = io.out(out, (size_t)n);
+    if (io.ok()) k_whole_body<<<(unsigned)((n + 127) / 128), 128, 0, f->stream>>>(f->grid, P, ds, n, dout);
+    return io.finish();
 }
 
 // kind as k_field_misc; in_a / in_b: n x wa doubles (host), in_i: n x 2 int32 (host)
@@ -518,33 +488,20 @@ static int field_misc(topay_field* f, int kind, const double* in_a, int wa, cons
     if (!f || n < 0 || (n > 0 && ((kind <= 3 && !in_a) || (kind == 2 && !in_b) || (kind == 4 && !in_i) ||
                                   (kind <= 2 && !flag) || (kind >= 3 && !val))))
         return TOPAY_ERR_INVALID_ARG;
-    if (!f->ready) {
-        tp_set_error("field queried before topay_field_rebuild");
-        return TOPAY_ERR_NOT_READY;
-    }
+    const int rc = tp_field_require_ready(f);
+    if (rc != TOPAY_OK) return rc;
     if (n == 0) return TOPAY_OK;
     cudaSetDevice(f->device);
-    const size_t ba = in_a ? (size_t)n * wa * 8 : 0, bb = in_b ? (size_t)n * wa * 8 : 0, bi = in_i ? (size_t)n * 8 : 0;
-    const size_t bv = (size_t)n * 8, bf = (size_t)n;
-    char* d = nullptr;
-    TP_CUDA_OK(cudaMallocAsync(&d, ba + bb + bi + bv + bf + 64, f->stream), {});
-    double* da = (double*)d;
-    double* db = (double*)(d + ba);
-    int32_t* di = (int32_t*)(d + ba + bb);
-    double* dv = (double*)(d + ba + bb + bi);
-    int8_t* df = (int8_t*)(d + ba + bb + bi + bv);
-    if (in_a) cudaMemcpyAsync(da, in_a, ba, cudaMemcpyHostToDevice, f->stream);
-    if (in_b) cudaMemcpyAsync(db, in_b, bb, cudaMemcpyHostToDevice, f->stream);
-    if (in_i) cudaMemcpyAsync(di, in_i, bi, cudaMemcpyHostToDevice, f->stream);
-    k_field_misc<<<(unsigned)((n + 255) / 256), 256, 0, f->stream>>>(f->grid, kind, da, db, di, n, threshold, critical,
-                                                                    df, dv);
-    if (kind <= 2) cudaMemcpyAsync(flag, df, bf, cudaMemcpyDeviceToHost, f->stream);
-    else cudaMemcpyAsync(val, dv, bv, cudaMemcpyDeviceToHost, f->stream);
-    cudaFreeAsync(d, f->stream);
-    cudaError_t e = cudaStreamSynchronize(f->stream);
-    TP_CUDA_OK(e, {});
-    TP_CUDA_OK(cudaGetLastError(), {});
-    return TOPAY_OK;
+    TpStaging io(f->stream);
+    const double* da = io.in(in_a, (size_t)n * wa);
+    const double* db = io.in(in_b, (size_t)n * wa);
+    const int32_t* di = io.in(in_i, (size_t)n * 2);
+    int8_t* df = io.out(kind <= 2 ? flag : nullptr, (size_t)n);
+    double* dv = io.out(kind <= 2 ? nullptr : val, (size_t)n);
+    if (io.ok())
+        k_field_misc<<<(unsigned)((n + 255) / 256), 256, 0, f->stream>>>(f->grid, kind, da, db, di, n, threshold,
+                                                                        critical, df, dv);
+    return io.finish();
 }
 
 extern "C" int topay_field_is_collision2d(topay_field* f, const double* pos, int64_t n, double threshold, int8_t* out) {
@@ -567,28 +524,19 @@ extern "C" int topay_field_dist_coarse2i(topay_field* f, const int32_t* idx, int
 extern "C" int topay_field_line_visible(topay_field* f, const double* p1, const double* p2, int64_t n, double thresh,
                                         int use_critical, int8_t* visible, double* pc) {
     if (!f || n < 0 || (n > 0 && (!p1 || !p2 || !visible || !pc))) return TOPAY_ERR_INVALID_ARG;
-    if (!f->ready) {
-        tp_set_error("field queried before topay_field_rebuild");
-        return TOPAY_ERR_NOT_READY;
-    }
+    const int rc = tp_field_require_ready(f);
+    if (rc != TOPAY_OK) return rc;
     if (n == 0) return TOPAY_OK;
     cudaSetDevice(f->device);
-    const size_t bp = (size_t)n * 3 * 8;
-    char* d = nullptr;
-    TP_CUDA_OK(cudaMallocAsync(&d, 3 * bp + (size_t)n + 64, f->stream), {});
-    double *d1 = (double*)d, *d2 = (double*)(d + bp), *dc = (double*)(d + 2 * bp);
-    int8_t* dv = (int8_t*)(d + 3 * bp);
-    cudaMemcpyAsync(d1, p1, bp, cudaMemcpyHostToDevice, f->stream);
-    cudaMemcpyAsync(d2, p2, bp, cudaMemcpyHostToDevice, f->stream);
-    cudaMemcpyAsync(dc, pc, bp, cudaMemcpyHostToDevice, f->stream);      // pc of a visible segment stays as passed in
-    k_line_visib<<<(unsigned)((n + 127) / 128), 128, 0, f->stream>>>(f->grid, d1, d2, n, thresh, use_critical, dv, dc);
-    cudaMemcpyAsync(visible, dv, (size_t)n, cudaMemcpyDeviceToHost, f->stream);
-    cudaMemcpyAsync(pc, dc, bp, cudaMemcpyDeviceToHost, f->stream);
-    cudaFreeAsync(d, f->stream);
-    cudaError_t e = cudaStreamSynchronize(f->stream);
-    TP_CUDA_OK(e, {});
-    TP_CUDA_OK(cudaGetLastError(), {});
-    return TOPAY_OK;
+    TpStaging io(f->stream);
+    const double* d1 = io.in(p1, (size_t)n * 3);
+    const double* d2 = io.in(p2, (size_t)n * 3);
+    double* dc = io.inout(pc, (size_t)n * 3);      // pc of a visible segment stays as passed in
+    int8_t* dv = io.out(visible, (size_t)n);
+    if (io.ok())
+        k_line_visib<<<(unsigned)((n + 127) / 128), 128, 0, f->stream>>>(f->grid, d1, d2, n, thresh, use_critical, dv,
+                                                                        dc);
+    return io.finish();
 }
 
 extern "C" int topay_discretize_path(const double* path, int n, int pt_num, double* out);
@@ -644,8 +592,7 @@ extern "C" int topay_field_download(topay_field* f, int which, double* esdf_out)
                         : which == TOPAY_MAP2D_CRITICAL ? f->esdf2d_crit
                         : which == TOPAY_MAP2D_INFLATE ? f->esdf2d_inflate : f->esdf2d;
     const size_t n = which == TOPAY_MAP3D ? f->n3 : f->n2;
-    TP_CUDA_OK(cudaMemcpy(esdf_out, src, n * 8, cudaMemcpyDeviceToHost), {});
-    return TOPAY_OK;
+    return tp_download(f->stream, esdf_out, src, n * 8);
 }
 
 extern "C" int topay_field_download_sqdist(topay_field* f, int which, int32_t* pos_sq, int32_t* neg_sq) {
@@ -656,9 +603,10 @@ extern "C" int topay_field_download_sqdist(topay_field* f, int which, int32_t* p
     }
     cudaSetDevice(f->device);
     const size_t n = which == TOPAY_MAP3D ? f->n3 : f->n2;
-    if (pos_sq) TP_CUDA_OK(cudaMemcpy(pos_sq, f->sq_pos[which], n * 4, cudaMemcpyDeviceToHost), {});
-    if (neg_sq) TP_CUDA_OK(cudaMemcpy(neg_sq, f->sq_neg[which], n * 4, cudaMemcpyDeviceToHost), {});
-    return TOPAY_OK;
+    int rc = TOPAY_OK;
+    if (pos_sq) rc = tp_download(f->stream, pos_sq, f->sq_pos[which], n * 4);
+    if (neg_sq && rc == TOPAY_OK) rc = tp_download(f->stream, neg_sq, f->sq_neg[which], n * 4);
+    return rc;
 }
 
 extern "C" int topay_field_download_occupancy(topay_field* f, int which, int8_t* occ_out) {
@@ -666,6 +614,5 @@ extern "C" int topay_field_download_occupancy(topay_field* f, int which, int8_t*
     cudaSetDevice(f->device);
     const int8_t* src = which == TOPAY_MAP3D ? f->occ3d : which == TOPAY_MAP2D_CRITICAL ? f->occ2d_crit : f->occ2d;
     const size_t n = which == TOPAY_MAP3D ? f->n3 : f->n2;
-    TP_CUDA_OK(cudaMemcpy(occ_out, src, n, cudaMemcpyDeviceToHost), {});
-    return TOPAY_OK;
+    return tp_download(f->stream, occ_out, src, n);
 }

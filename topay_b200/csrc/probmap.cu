@@ -301,6 +301,7 @@ struct topay_probmap {
     float4* d_pts;
     double* d_rays;
     size_t cap_pts;
+    TpDevBuffers bufs;       // the ring's buffers; d_pts / d_rays grow with the largest cloud and are freed apart
 };
 
 namespace {
@@ -368,7 +369,6 @@ void pm_apply(topay_probmap* m, int first_frame) {
 extern "C" int topay_probmap_create(topay_rogfield* esdf, const topay_prob_desc* p, topay_probmap** out) {
     if (!esdf || !p || !out) return TOPAY_ERR_INVALID_ARG;
     topay_probmap* m = new topay_probmap();
-    memset(m, 0, sizeof(*m));
     m->esdf = esdf;
     tp_rogfield_counters(esdf, &m->E);
     m->desc = *p;
@@ -412,10 +412,17 @@ extern "C" int topay_probmap_create(topay_rogfield* esdf, const topay_prob_desc*
     }
     m->map_empty = true;
     m->first_frame = true;
-    TP_CUDA_OK(cudaMalloc(&m->V.occ, m->vox * sizeof(float)), { topay_probmap_destroy(m); });
-    TP_CUDA_OK(cudaMalloc(&m->V.cnt, m->vox * sizeof(unsigned int)), { topay_probmap_destroy(m); });
-    TP_CUDA_OK(cudaMalloc(&m->V.cache, m->vox * sizeof(int32_t)), { topay_probmap_destroy(m); });
-    TP_CUDA_OK(cudaMalloc(&m->V.cache_n, sizeof(int32_t)), { topay_probmap_destroy(m); });
+    TpDevBuffers& b = m->bufs;
+    b.stream = m->E.stream;
+    b.alloc(&m->V.occ, m->vox);
+    b.alloc(&m->V.cnt, m->vox);
+    b.alloc(&m->V.cache, m->vox);
+    b.alloc(&m->V.cache_n, 1);
+    if (b.status != TOPAY_OK) {
+        const int rc = b.status;
+        topay_probmap_destroy(m);
+        return rc;
+    }
     pm_reset_local_map(m);
     if (!m->sliding_en) {
         // sliding_map.cpp:58-61 + prob_map.cpp:73-77
@@ -440,8 +447,7 @@ extern "C" void topay_probmap_destroy(topay_probmap* m) {
     if (!m) return;
     cudaSetDevice(m->E.device);
     cudaStreamSynchronize(m->E.stream);
-    void* ptrs[] = {m->V.occ, m->V.cnt, m->V.cache, m->V.cache_n, m->d_pts, m->d_rays};
-    for (void* p : ptrs)
+    for (void* p : {(void*)m->d_pts, (void*)m->d_rays})
         if (p) cudaFree(p);
     delete m;
 }
@@ -564,17 +570,14 @@ extern "C" int topay_probmap_update(topay_probmap* m, const float* cloud, int64_
                     counts[k]++;
                 }
         if (!cells.empty()) {
-            int32_t* d_l = nullptr;
             const size_t nc = cells.size();
-            TP_CUDA_OK(cudaMalloc(&d_l, 2 * nc * sizeof(int32_t)), {});
-            cudaMemcpyAsync(d_l, cells.data(), nc * sizeof(int32_t), cudaMemcpyHostToDevice, q);
-            cudaMemcpyAsync(d_l + nc, counts.data(), nc * sizeof(int32_t), cudaMemcpyHostToDevice, q);
-            k_prob_first<<<(unsigned)((nc + 127) / 128), 128, 0, q>>>(m->V, m->E.view, m->E.occ_cnt, m->E.unk_cnt, d_l, d_l + nc,
-                                                                     (int)nc);
-            cudaError_t e = cudaStreamSynchronize(q);
-            cudaFree(d_l);
-            TP_CUDA_OK(e, {});
-            TP_CUDA_OK(cudaGetLastError(), {});
+            TpStaging io(q);
+            const int32_t* d_cells = io.in(cells.data(), nc);
+            const int32_t* d_counts = io.in(counts.data(), nc);
+            if (io.ok())
+                k_prob_first<<<(unsigned)((nc + 127) / 128), 128, 0, q>>>(m->V, m->E.view, m->E.occ_cnt, m->E.unk_cnt,
+                                                                         d_cells, d_counts, (int)nc);
+            return io.finish();
         }
     }
     return TOPAY_OK;

@@ -41,6 +41,7 @@ struct topay_rogfield {
     cudaEvent_t ev0, ev1, ev2;
     float ms_total, ms_3d;
     bool updated;               // updateESDF3D ran at least once
+    TpDevBuffers bufs;
 };
 
 namespace {
@@ -251,7 +252,6 @@ extern "C" int topay_rogfield_create(const topay_rog_desc* d, int device, topay_
     int rc = tp_require_device(device);
     if (rc != TOPAY_OK) return rc;
     topay_rogfield* f = new topay_rogfield();
-    memset(f, 0, sizeof(*f));
     f->desc = *d;
     f->device = device;
     cudaSetDevice(device);
@@ -282,29 +282,20 @@ extern "C" int topay_rogfield_create(const topay_rog_desc* d, int device, topay_
     f->n2 = (size_t)f->size[0] * f->size[1];
     f->n3 = f->n2 * f->size[2];
     TP_CUDA_OK(cudaStreamCreateWithFlags(&f->stream, cudaStreamNonBlocking), { delete f; });
-#define RA(p, n)                                        \
-    if ((rc = tp_dev_malloc(&(p), (n))) != TOPAY_OK) {  \
-        topay_rogfield_destroy(f);                      \
-        return rc;                                      \
-    }
-    RA(f->occ_cnt, f->n3 + 1);   // +1: the 16-bit atomics work on aligned 32-bit words
-    RA(f->unk_cnt, f->n3 + 1);
-    RA(f->dist3, f->n3);
-    RA(f->neg3, f->n3);
-    RA(f->crit, f->n2);
-    RA(f->flat, f->n2);
-    RA(f->neg2, f->n2);
-    RA(f->box_occ, f->n3);
-    RA(f->col_occ, 2 * f->n2);
-    RA(f->packed16, f->n3);
-    RA(f->packed32, f->n3);
-#undef RA
-    cudaMemsetAsync(f->dist3, 0, f->n3 * 8, f->stream);
-    cudaMemsetAsync(f->neg3, 0, f->n3 * 8, f->stream);
-    cudaMemsetAsync(f->crit, 0, f->n2 * 8, f->stream);
-    cudaMemsetAsync(f->flat, 0, f->n2 * 8, f->stream);
-    cudaMemsetAsync(f->unk_cnt, 0, (f->n3 + 1) * 2, f->stream);
-    if ((rc = reset_counters(f)) != TOPAY_OK) {
+    TpDevBuffers& b = f->bufs;
+    b.stream = f->stream;
+    b.alloc(&f->occ_cnt, f->n3 + 1);   // +1: the 16-bit atomics work on aligned 32-bit words
+    b.alloc(&f->unk_cnt, f->n3 + 1);
+    b.alloc(&f->dist3, f->n3);
+    b.alloc(&f->neg3, f->n3);
+    b.alloc(&f->crit, f->n2);
+    b.alloc(&f->flat, f->n2);
+    b.alloc(&f->neg2, f->n2);
+    b.alloc(&f->box_occ, f->n3);
+    b.alloc(&f->col_occ, 2 * f->n2);
+    b.alloc(&f->packed16, f->n3);
+    b.alloc(&f->packed32, f->n3);
+    if ((rc = b.status) != TOPAY_OK || (rc = reset_counters(f)) != TOPAY_OK) {
         topay_rogfield_destroy(f);
         return rc;
     }
@@ -320,10 +311,6 @@ extern "C" void topay_rogfield_destroy(topay_rogfield* f) {
     if (!f) return;
     cudaSetDevice(f->device);
     if (f->stream) cudaStreamSynchronize(f->stream);
-    void* ptrs[] = {f->occ_cnt, f->unk_cnt, f->dist3, f->neg3, f->crit, f->flat, f->neg2, f->box_occ,
-                    f->col_occ, f->packed16, f->packed32};
-    for (void* p : ptrs)
-        if (p) cudaFree(p);
     if (f->ev0) cudaEventDestroy(f->ev0);
     if (f->ev1) cudaEventDestroy(f->ev1);
     if (f->ev2) cudaEventDestroy(f->ev2);
@@ -382,21 +369,14 @@ extern "C" int topay_rogfield_update_counters(topay_rogfield* f, const double* p
     if (!f || n < 0 || (n > 0 && (!pos || !from_type || !to_type))) return TOPAY_ERR_INVALID_ARG;
     if (n == 0) return TOPAY_OK;
     cudaSetDevice(f->device);
-    double* dp = nullptr;
-    uint8_t* dt = nullptr;
-    TP_CUDA_OK(cudaMallocAsync(&dp, (size_t)n * 24, f->stream), {});
-    TP_CUDA_OK(cudaMallocAsync(&dt, (size_t)n * 2, f->stream), { cudaFreeAsync(dp, f->stream); });
-    cudaMemcpyAsync(dp, pos, (size_t)n * 24, cudaMemcpyHostToDevice, f->stream);
-    cudaMemcpyAsync(dt, from_type, (size_t)n, cudaMemcpyHostToDevice, f->stream);
-    cudaMemcpyAsync(dt + n, to_type, (size_t)n, cudaMemcpyHostToDevice, f->stream);
-    k_rog_counters<<<(unsigned)((n + 255) / 256), 256, 0, f->stream>>>(rog_view(f), dp, dt, dt + n, n, f->occ_cnt,
-                                                                      f->unk_cnt);
-    cudaFreeAsync(dp, f->stream);
-    cudaFreeAsync(dt, f->stream);
-    cudaError_t e = cudaStreamSynchronize(f->stream);
-    TP_CUDA_OK(e, {});
-    TP_CUDA_OK(cudaGetLastError(), {});
-    return TOPAY_OK;
+    TpStaging io(f->stream);
+    const double* dp = io.in(pos, (size_t)n * 3);
+    const uint8_t* dfrom = io.in(from_type, (size_t)n);
+    const uint8_t* dto = io.in(to_type, (size_t)n);
+    if (io.ok())
+        k_rog_counters<<<(unsigned)((n + 255) / 256), 256, 0, f->stream>>>(rog_view(f), dp, dfrom, dto, n, f->occ_cnt,
+                                                                          f->unk_cnt);
+    return io.finish();
 }
 
 extern "C" int topay_rogfield_set_occupied_cnt(topay_rogfield* f, const int16_t* cnt) {
@@ -516,20 +496,13 @@ extern "C" int topay_rogfield_query(topay_rogfield* f, int kind, const double* p
         return TOPAY_ERR_INVALID_ARG;
     if (n == 0) return TOPAY_OK;
     cudaSetDevice(f->device);
-    double* d = nullptr;
-    TP_CUDA_OK(cudaMallocAsync(&d, (size_t)n * 7 * 8, f->stream), {});
-    double *dpos = d, *ddist = d + 3 * n, *dgrad = d + 4 * n;
-    cudaMemcpyAsync(dpos, pos, (size_t)n * 24, cudaMemcpyHostToDevice, f->stream);
-    if (grad) cudaMemcpyAsync(dgrad, grad, (size_t)n * 24, cudaMemcpyHostToDevice, f->stream);   // cell kinds leave it
-    k_rog_query<<<(unsigned)((n + 255) / 256), 256, 0, f->stream>>>(rog_view(f), kind, dpos, n, ddist,
-                                                                   grad ? dgrad : nullptr);
-    cudaMemcpyAsync(dist, ddist, (size_t)n * 8, cudaMemcpyDeviceToHost, f->stream);
-    if (grad) cudaMemcpyAsync(grad, dgrad, (size_t)n * 24, cudaMemcpyDeviceToHost, f->stream);
-    cudaFreeAsync(d, f->stream);
-    cudaError_t e = cudaStreamSynchronize(f->stream);
-    TP_CUDA_OK(e, {});
-    TP_CUDA_OK(cudaGetLastError(), {});
-    return TOPAY_OK;
+    TpStaging io(f->stream);
+    const double* dpos = io.in(pos, (size_t)n * 3);
+    double* ddist = io.out(dist, (size_t)n);
+    double* dgrad = io.inout(grad, (size_t)n * 3);   // the cell kinds leave it as passed in
+    if (io.ok())
+        k_rog_query<<<(unsigned)((n + 255) / 256), 256, 0, f->stream>>>(rog_view(f), kind, dpos, n, ddist, dgrad);
+    return io.finish();
 }
 
 extern "C" int topay_rogfield_is_line_free2d(topay_rogfield* f, const double* start, const double* end, int64_t n,
@@ -537,18 +510,13 @@ extern "C" int topay_rogfield_is_line_free2d(topay_rogfield* f, const double* st
     if (!f || n < 0 || (n > 0 && (!start || !end || !out))) return TOPAY_ERR_INVALID_ARG;
     if (n == 0) return TOPAY_OK;
     cudaSetDevice(f->device);
-    double* d = nullptr;
-    TP_CUDA_OK(cudaMallocAsync(&d, (size_t)n * 4 * 8 + (size_t)n, f->stream), {});
-    int8_t* dout = reinterpret_cast<int8_t*>(d + 4 * n);
-    cudaMemcpyAsync(d, start, (size_t)n * 16, cudaMemcpyHostToDevice, f->stream);
-    cudaMemcpyAsync(d + 2 * n, end, (size_t)n * 16, cudaMemcpyHostToDevice, f->stream);
-    k_rog_line<<<(unsigned)((n + 127) / 128), 128, 0, f->stream>>>(rog_view(f), d, d + 2 * n, n, threshold, dout);
-    cudaMemcpyAsync(out, dout, (size_t)n, cudaMemcpyDeviceToHost, f->stream);
-    cudaFreeAsync(d, f->stream);
-    cudaError_t e = cudaStreamSynchronize(f->stream);
-    TP_CUDA_OK(e, {});
-    TP_CUDA_OK(cudaGetLastError(), {});
-    return TOPAY_OK;
+    TpStaging io(f->stream);
+    const double* ds = io.in(start, (size_t)n * 2);
+    const double* de = io.in(end, (size_t)n * 2);
+    int8_t* dout = io.out(out, (size_t)n);
+    if (io.ok())
+        k_rog_line<<<(unsigned)((n + 127) / 128), 128, 0, f->stream>>>(rog_view(f), ds, de, n, threshold, dout);
+    return io.finish();
 }
 
 extern "C" int topay_rogfield_download(topay_rogfield* f, int which, double* out) {
@@ -558,7 +526,5 @@ extern "C" int topay_rogfield_download(topay_rogfield* f, int which, double* out
                         : which == TOPAY_ROG_BUF_NEG3 ? f->neg3
                         : which == TOPAY_ROG_BUF_CRITICAL ? f->crit : f->flat;
     const size_t n = which <= TOPAY_ROG_BUF_NEG3 ? f->n3 : f->n2;
-    TP_CUDA_OK(cudaMemcpyAsync(out, src, n * 8, cudaMemcpyDeviceToHost, f->stream), {});
-    TP_CUDA_OK(cudaStreamSynchronize(f->stream), {});
-    return TOPAY_OK;
+    return tp_download(f->stream, out, src, n * 8);
 }

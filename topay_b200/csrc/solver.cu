@@ -68,7 +68,7 @@ struct topay_solver {
     char* h_pin;
     TpCandState* h_state;
     double *p_head, *p_tail, *p_sxy, *p_exy, *p_ixy;
-    std::vector<void*> allocs;
+    TpDevBuffers bufs;   // every device buffer of the solver but the trace and phase-clock buffers
     int32_t* h_active;   // pinned: [0] lane A's live slots after the batch, [1..3] queue state, [4] lane B's live slots
     unsigned long long* h_nodes;  // pinned
     int n_slots_used;    // slots seeded by the last run (min(n_slots, n_cand))
@@ -114,22 +114,14 @@ void solver_grid(const topay_solver* s, TpGrid* G) {
     if (s->rog) tp_rogfield_grid(s->rog, G);
     else tp_field_grid(s->field, G);
 }
-bool solver_field_ready(const topay_solver* s) {
-    if (s->dev.n_fields > 1) {
-        for (const topay_field* f : s->fields)
-            if (!tp_field_ready(f)) return false;
-        return true;
-    }
-    return s->rog ? tp_rogfield_ready(s->rog) : tp_field_ready(s->field);
-}
-
-template <typename T>
-int dev_alloc(topay_solver* s, T** p, size_t count) {
-    const int rc = tp_dev_malloc(p, count);
-    if (rc != TOPAY_OK) return rc;
-    cudaMemsetAsync(*p, 0, std::max<size_t>(count, 1) * sizeof(T), s->stream);
-    s->allocs.push_back(*p);
-    return TOPAY_OK;
+// TOPAY_OK when every field the solver reads is built, else TOPAY_ERR_NOT_READY with the error text set.
+int solver_require_ready(const topay_solver* s) {
+    const bool ready = s->dev.n_fields > 1 ? std::all_of(s->fields.begin(), s->fields.end(), tp_field_ready)
+                       : s->rog            ? tp_rogfield_ready(s->rog)
+                                           : tp_field_ready(s->field);
+    if (ready) return TOPAY_OK;
+    tp_set_error("field not built: call topay_field_rebuild first");
+    return TOPAY_ERR_NOT_READY;
 }
 
 int kpad_of(int K) {
@@ -286,6 +278,7 @@ static int solver_create(const topay_opt_params* opt, const topay_robot_params* 
     cudaSetDevice(s->device);
     tp_pool_keep(s->device);
     TP_CUDA_OK(cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking), { delete s; });
+    s->bufs.stream = s->stream;
     memset(&s->params, 0, sizeof(s->params));
     s->params.robot = *robot;
     s->params.opt = *opt;
@@ -302,58 +295,57 @@ static int solver_create(const topay_opt_params* opt, const topay_robot_params* 
     D.xs = (topay_num_vars(max_pieces) + 3) & ~3;
     D.mem = std::max(1, std::max(opt->s1_lbfgs.mem_size, opt->s2_lbfgs.mem_size));
     const size_t G = max_cand, C = n_slots, NP = max_pieces, K = D.K;
-#define ALLOC(ptr, count)                                    \
-    if ((rc = dev_alloc(s, &(ptr), (count))) != TOPAY_OK) {  \
-        topay_solver_destroy(s);                             \
-        return rc;                                           \
-    }
+    TpDevBuffers& b = s->bufs;
     // store
-    ALLOC(D.head_pva, G * 27);
-    ALLOC(D.tail_pva, G * 27);
-    ALLOC(D.start_xy, G * 2);
-    ALLOC(D.end_xy, G * 2);
-    ALLOC(D.init_inner_xy, G * NP * 2);
-    ALLOC(D.x0, G * D.xs);
-    ALLOC(D.st0, G);
-    ALLOC(D.res_st, G);
-    ALLOC(D.res_T, G * NP);
-    ALLOC(D.res_coeff, G * 6 * NP * 9);
-    ALLOC(D.res_x, G * D.xs);
+    b.alloc(&D.head_pva, G * 27);
+    b.alloc(&D.tail_pva, G * 27);
+    b.alloc(&D.start_xy, G * 2);
+    b.alloc(&D.end_xy, G * 2);
+    b.alloc(&D.init_inner_xy, G * NP * 2);
+    b.alloc(&D.x0, G * D.xs);
+    b.alloc(&D.st0, G);
+    b.alloc(&D.res_st, G);
+    b.alloc(&D.res_T, G * NP);
+    b.alloc(&D.res_coeff, G * 6 * NP * 9);
+    b.alloc(&D.res_x, G * D.xs);
     // scheduling
-    ALLOC(D.slot_gid, C);
-    ALLOC(D.list, (size_t)(TP_TICKS + 1) * C);
-    ALLOC(D.count, (size_t)TP_TICKS + 1);
-    ALLOC(s->lane[1].list, (size_t)(TP_TICKS + 1) * C);
-    ALLOC(s->lane[1].count, (size_t)TP_TICKS + 1);
-    ALLOC(D.queue, 4);
+    b.alloc(&D.slot_gid, C);
+    b.alloc(&D.list, (size_t)(TP_TICKS + 1) * C);
+    b.alloc(&D.count, (size_t)TP_TICKS + 1);
+    b.alloc(&s->lane[1].list, (size_t)(TP_TICKS + 1) * C);
+    b.alloc(&s->lane[1].count, (size_t)TP_TICKS + 1);
+    b.alloc(&D.queue, 4);
     // slots
-    ALLOC(D.st, C);
-    ALLOC(D.x, C * D.xs);
-    ALLOC(D.g, C * D.xs);
-    ALLOC(D.xp, C * D.xs);
-    ALLOC(D.gp, C * D.xs);
-    ALLOC(D.d, C * D.xs);
-    ALLOC(D.lm_s, C * D.mem * D.xs);
-    ALLOC(D.lm_y, C * D.mem * D.xs);
-    ALLOC(D.lm_ys, C * D.mem);
-    ALLOC(D.lm_alpha, C * D.mem);
-    ALLOC(D.T, C * NP);
-    ALLOC(D.coeff, C * 6 * NP * 9);
-    ALLOC(D.lu, C * 6 * NP * TP_BAND);
-    ALLOC(D.Ixy, C * NP * K * 2);
-    ALLOC(D.tot, C * NP * 2);
-    ALLOC(D.gnode, C * NP * (K + 1) * 2);
-    ALLOC(D.gsum, C * NP * 2);
-    ALLOC(D.gdC, C * 6 * NP * 9);
-    ALLOC(D.gdC_end, C * NP * 54);
-    ALLOC(D.gdT, C * NP);
-    ALLOC(D.gdT_end, C * NP);
-    ALLOC(D.terms, C * NP * TOPAY_NTERMS);
-    ALLOC(D.terms_end, C * NP * TOPAY_NTERMS);
-    ALLOC(D.f, C);
-    ALLOC(D.term_out, C * TOPAY_NTERMS);
-    ALLOC(D.node_count, 2);
-#undef ALLOC
+    b.alloc(&D.st, C);
+    b.alloc(&D.x, C * D.xs);
+    b.alloc(&D.g, C * D.xs);
+    b.alloc(&D.xp, C * D.xs);
+    b.alloc(&D.gp, C * D.xs);
+    b.alloc(&D.d, C * D.xs);
+    b.alloc(&D.lm_s, C * D.mem * D.xs);
+    b.alloc(&D.lm_y, C * D.mem * D.xs);
+    b.alloc(&D.lm_ys, C * D.mem);
+    b.alloc(&D.lm_alpha, C * D.mem);
+    b.alloc(&D.T, C * NP);
+    b.alloc(&D.coeff, C * 6 * NP * 9);
+    b.alloc(&D.lu, C * 6 * NP * TP_BAND);
+    b.alloc(&D.Ixy, C * NP * K * 2);
+    b.alloc(&D.tot, C * NP * 2);
+    b.alloc(&D.gnode, C * NP * (K + 1) * 2);
+    b.alloc(&D.gsum, C * NP * 2);
+    b.alloc(&D.gdC, C * 6 * NP * 9);
+    b.alloc(&D.gdC_end, C * NP * 54);
+    b.alloc(&D.gdT, C * NP);
+    b.alloc(&D.gdT_end, C * NP);
+    b.alloc(&D.terms, C * NP * TOPAY_NTERMS);
+    b.alloc(&D.terms_end, C * NP * TOPAY_NTERMS);
+    b.alloc(&D.f, C);
+    b.alloc(&D.term_out, C * TOPAY_NTERMS);
+    b.alloc(&D.node_count, 2);
+    if ((rc = b.status) != TOPAY_OK) {
+        topay_solver_destroy(s);
+        return rc;
+    }
     {
         const size_t b_state = ((G * sizeof(TpCandState) + 15) / 16) * 16;
         const size_t n_dbl = G * D.xs + G * (27 + 27 + 2 + 2) + G * NP * 2;
@@ -423,7 +415,6 @@ extern "C" void topay_solver_destroy(topay_solver* s) {
     if (s->stream) cudaStreamSynchronize(s->stream);
     drop_graphs(s);
     delete s->checker;
-    for (void* p : s->allocs) cudaFree(p);
     if (s->dev.trace) cudaFree(s->dev.trace);
     if (s->dev.trace_len) cudaFree(s->dev.trace_len);
     if (s->dev.prof) cudaFree(s->dev.prof);
@@ -521,18 +512,16 @@ extern "C" int topay_solver_eval(topay_solver* s, int stage, const topay_problem
                                  int x_stride, double* cost, double* grad, double* term_costs, double* coeff_out,
                                  double* final_xy_out) {
     if (!s || !prob || !x || !cost || !grad || (stage != 1 && stage != 2)) return TOPAY_ERR_INVALID_ARG;
-    if (!solver_field_ready(s)) {
-        tp_set_error("field not built: call topay_field_rebuild first");
-        return TOPAY_ERR_NOT_READY;
-    }
+    int rc = solver_require_ready(s);
+    if (rc != TOPAY_OK) return rc;
     if (prob->n_cand > s->dev.n_slots) {
         tp_set_error("topay_solver_eval evaluates at most n_slots candidates at a time");
         return TOPAY_ERR_TOO_LARGE;
     }
     if (s->dev.n_fields > 1) topay_solver_assign_fields(s, nullptr, 0, nullptr);   // evaluations read the solver's own field
-    int rc = upload_problem(s, prob->n_cand, prob->piece_num, prob->head_pva, prob->tail_pva, prob->start_xy,
-                            prob->end_xy, prob->init_inner_xy, x, x_stride, nullptr, stage, prob->alm_lambda,
-                            prob->alm_rho);
+    rc = upload_problem(s, prob->n_cand, prob->piece_num, prob->head_pva, prob->tail_pva, prob->start_xy,
+                        prob->end_xy, prob->init_inner_xy, x, x_stride, nullptr, stage, prob->alm_lambda,
+                        prob->alm_rho);
     if (rc != TOPAY_OK) return rc;
     const TpSolverDev& D = s->dev;
     const int n = prob->n_cand;
@@ -545,17 +534,19 @@ extern "C" int topay_solver_eval(topay_solver* s, int stage, const topay_problem
     TP_CUDA_OK(cudaStreamSynchronize(s->stream), {});
     TP_CUDA_OK(cudaGetLastError(), {});
     s->n_cand = 0;   // the uploaded problem carried the evaluation's phase / multipliers: not a solvable upload
+    const cudaStream_t q = s->stream;
     std::vector<double> g((size_t)n * D.xs);
-    TP_CUDA_OK(cudaMemcpy(cost, D.f, n * 8, cudaMemcpyDeviceToHost), {});
-    TP_CUDA_OK(cudaMemcpy(g.data(), D.g, g.size() * 8, cudaMemcpyDeviceToHost), {});
+    if ((rc = tp_download(q, cost, D.f, n * 8)) != TOPAY_OK) return rc;
+    if ((rc = tp_download(q, g.data(), D.g, g.size() * 8)) != TOPAY_OK) return rc;
     for (int c = 0; c < n; c++)
         memcpy(grad + (size_t)c * x_stride, &g[(size_t)c * D.xs], topay_num_vars(prob->piece_num[c]) * 8);
-    if (term_costs) TP_CUDA_OK(cudaMemcpy(term_costs, D.term_out, (size_t)n * TOPAY_NTERMS * 8, cudaMemcpyDeviceToHost), {});
-    if (coeff_out)
-        TP_CUDA_OK(cudaMemcpy(coeff_out, D.coeff, (size_t)n * 6 * D.max_pieces * 9 * 8, cudaMemcpyDeviceToHost), {});
+    if (term_costs && (rc = tp_download(q, term_costs, D.term_out, (size_t)n * TOPAY_NTERMS * 8)) != TOPAY_OK)
+        return rc;
+    if (coeff_out && (rc = tp_download(q, coeff_out, D.coeff, (size_t)n * 6 * D.max_pieces * 9 * 8)) != TOPAY_OK)
+        return rc;
     if (final_xy_out) {
         std::vector<TpCandState> st(n);
-        TP_CUDA_OK(cudaMemcpy(st.data(), D.st, n * sizeof(TpCandState), cudaMemcpyDeviceToHost), {});
+        if ((rc = tp_download(q, st.data(), D.st, n * sizeof(TpCandState))) != TOPAY_OK) return rc;
         for (int c = 0; c < n; c++) {
             final_xy_out[2 * c] = st[c].final_xy[0];
             final_xy_out[2 * c + 1] = st[c].final_xy[1];
@@ -589,8 +580,8 @@ extern "C" int topay_solver_assign_fields(topay_solver* s, topay_field* const* f
         if (field_of[c] < 0 || field_of[c] >= n_fields) return TOPAY_ERR_INVALID_ARG;
     int rc;
     if (!s->d_grids) {
-        if ((rc = dev_alloc(s, &s->d_grids, (size_t)D.max_cand)) != TOPAY_OK) return rc;
-        if ((rc = dev_alloc(s, &s->d_field_of, (size_t)D.max_cand)) != TOPAY_OK) return rc;
+        if ((rc = s->bufs.alloc(&s->d_grids, (size_t)D.max_cand)) != TOPAY_OK) return rc;
+        if ((rc = s->bufs.alloc(&s->d_field_of, (size_t)D.max_cand)) != TOPAY_OK) return rc;
     }
     TP_CUDA_OK(cudaMemcpyAsync(s->d_grids, hg.data(), (size_t)n_fields * sizeof(TpGrid), cudaMemcpyHostToDevice, s->stream), {});
     TP_CUDA_OK(cudaMemcpyAsync(s->d_field_of, field_of, (size_t)s->n_cand * sizeof(int32_t), cudaMemcpyHostToDevice, s->stream), {});
@@ -706,10 +697,8 @@ static void mark_tick_cap(topay_solver* s, const TpLane& L, int n_store) {
 
 extern "C" int topay_solver_run(topay_solver* s) {
     if (!s || s->n_cand < 1) return TOPAY_ERR_INVALID_ARG;
-    if (!solver_field_ready(s)) {
-        tp_set_error("field not built: call topay_field_rebuild first");
-        return TOPAY_ERR_NOT_READY;
-    }
+    const int rc = solver_require_ready(s);
+    if (rc != TOPAY_OK) return rc;
     if (s->dev.n_fields > 1 && s->fields_n_cand != s->n_cand) {
         tp_set_error("the field assignment was made for an upload of another size: call topay_solver_assign_fields again");
         return TOPAY_ERR_NOT_READY;
@@ -885,10 +874,12 @@ extern "C" int topay_solver_download(topay_solver* s, topay_result_batch* out, i
     cudaSetDevice(s->device);
     const TpSolverDev& D = s->dev;
     const int n = s->n_cand, NP = D.max_pieces;
+    const cudaStream_t q = s->stream;
+    int rc;
     std::vector<TpCandState> st(n);
-    TP_CUDA_OK(cudaMemcpy(st.data(), D.res_st, n * sizeof(TpCandState), cudaMemcpyDeviceToHost), {});
+    if ((rc = tp_download(q, st.data(), D.res_st, n * sizeof(TpCandState))) != TOPAY_OK) return rc;
     std::vector<double> T((size_t)n * NP);
-    TP_CUDA_OK(cudaMemcpy(T.data(), D.res_T, T.size() * 8, cudaMemcpyDeviceToHost), {});
+    if ((rc = tp_download(q, T.data(), D.res_T, T.size() * 8)) != TOPAY_OK) return rc;
     int bd = -1, bc = -1;
     double bdv = 0, bcv = 0;
     int64_t evals = 0;
@@ -909,10 +900,10 @@ extern "C" int topay_solver_download(topay_solver* s, topay_result_batch* out, i
     }
     s->stats.evals_total = evals;
     if (out->T) memcpy(out->T, T.data(), T.size() * 8);
-    if (out->coeff) TP_CUDA_OK(cudaMemcpy(out->coeff, D.res_coeff, (size_t)n * 6 * NP * 9 * 8, cudaMemcpyDeviceToHost), {});
+    if (out->coeff && (rc = tp_download(q, out->coeff, D.res_coeff, (size_t)n * 6 * NP * 9 * 8)) != TOPAY_OK) return rc;
     if (out->x) {
         std::vector<double> xs((size_t)n * D.xs);
-        TP_CUDA_OK(cudaMemcpy(xs.data(), D.res_x, xs.size() * 8, cudaMemcpyDeviceToHost), {});
+        if ((rc = tp_download(q, xs.data(), D.res_x, xs.size() * 8)) != TOPAY_OK) return rc;
         const int xstride = topay_num_vars(NP);
         for (int c = 0; c < n; c++) memcpy(out->x + (size_t)c * xstride, &xs[(size_t)c * D.xs], st[c].n * 8);
     }
@@ -951,8 +942,8 @@ extern "C" int topay_solver_check_feasible(topay_solver* s, topay_feasibility* o
     const int n = s->n_cand, NP = D.max_pieces;
     int rc;
     if (!s->checker) {
-        if ((rc = dev_alloc(s, &s->d_pn, (size_t)D.max_cand)) != TOPAY_OK) return rc;
-        if ((rc = dev_alloc(s, &s->d_start, (size_t)D.max_cand * 3)) != TOPAY_OK) return rc;
+        if ((rc = s->bufs.alloc(&s->d_pn, (size_t)D.max_cand)) != TOPAY_OK) return rc;
+        if ((rc = s->bufs.alloc(&s->d_start, (size_t)D.max_cand * 3)) != TOPAY_OK) return rc;
         s->checker = new TpTrajChecker();
         if ((rc = s->checker->init(s->device, s->stream)) != TOPAY_OK) return rc;
     }
@@ -1038,18 +1029,15 @@ extern "C" int topay_solver_select(topay_solver* s, int n_plans, const int32_t* 
     }
     cudaSetDevice(s->device);
     const TpSolverDev& D = s->dev;
-    int32_t* d = nullptr;
-    TP_CUDA_OK(cudaMallocAsync(&d, (size_t)(3 * n_plans + 1) * sizeof(int32_t), s->stream), {});
-    int32_t* d_off = d + 2 * n_plans;
-    TP_CUDA_OK(cudaMemcpyAsync(d_off, plan_offset, (size_t)(n_plans + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, s->stream),
-               { cudaFreeAsync(d, s->stream); });
-    k_select<<<n_plans, 128, 0, s->stream>>>(D.res_st, D.res_T, D.max_pieces, use_gate ? s->checker->feas : nullptr, d_off, d);
     std::vector<int32_t> h((size_t)2 * n_plans);
-    TP_CUDA_OK(cudaMemcpyAsync(h.data(), d, h.size() * sizeof(int32_t), cudaMemcpyDeviceToHost, s->stream),
-               { cudaFreeAsync(d, s->stream); });
-    cudaFreeAsync(d, s->stream);
-    TP_CUDA_OK(cudaStreamSynchronize(s->stream), {});
-    TP_CUDA_OK(cudaGetLastError(), {});
+    TpStaging io(s->stream);
+    const int32_t* d_off = io.in(plan_offset, (size_t)n_plans + 1);
+    int32_t* d = io.out(h.data(), h.size());
+    if (io.ok())
+        k_select<<<n_plans, 128, 0, s->stream>>>(D.res_st, D.res_T, D.max_pieces, use_gate ? s->checker->feas : nullptr,
+                                                 d_off, d);
+    const int rc = io.finish();
+    if (rc != TOPAY_OK) return rc;
     for (int i = 0; i < n_plans; i++) {
         if (best_by_duration) best_by_duration[i] = h[2 * i];
         if (best_by_cost) best_by_cost[i] = h[2 * i + 1];
@@ -1103,8 +1091,8 @@ extern "C" int64_t topay_solver_debug_download(topay_solver* s, int which, doubl
         default: return TOPAY_ERR_INVALID_ARG;
     }
     if ((int64_t)n > cap) n = (size_t)cap;
-    TP_CUDA_OK(cudaMemcpy(out, src, n * sizeof(double), cudaMemcpyDeviceToHost), {});
-    return (int64_t)n;
+    const int rc = tp_download(s->stream, out, src, n * sizeof(double));
+    return rc != TOPAY_OK ? rc : (int64_t)n;
 }
 
 // Parity hook for the L-BFGS direction update (lbfgs.hpp:657-710). Loads a history into slot 0 and runs ONE launch
@@ -1136,7 +1124,7 @@ extern "C" int topay_solver_debug_direction(topay_solver* s, int n_vars, int bou
     auto up = [&](double* dst, const double* src, size_t rows, size_t row_len) {
         std::vector<double> pad(rows * D.xs, 0.0);
         for (size_t r = 0; r < rows; r++) memcpy(&pad[r * D.xs], src + r * row_len, row_len * sizeof(double));
-        return cudaMemcpy(dst, pad.data(), pad.size() * sizeof(double), cudaMemcpyHostToDevice);
+        return cudaMemcpyAsync(dst, pad.data(), pad.size() * sizeof(double), cudaMemcpyHostToDevice, q);
     };
     TP_CUDA_OK(up(D.x, x, 1, n_vars), {});
     TP_CUDA_OK(up(D.xp, xp, 1, n_vars), {});
@@ -1144,23 +1132,25 @@ extern "C" int topay_solver_debug_direction(topay_solver* s, int n_vars, int bou
     TP_CUDA_OK(up(D.gp, gp, 1, n_vars), {});
     TP_CUDA_OK(up(D.lm_s, S_rows, m, n_vars), {});
     TP_CUDA_OK(up(D.lm_y, Y_rows, m, n_vars), {});
-    TP_CUDA_OK(cudaMemcpy(D.lm_ys, ys, m * sizeof(double), cudaMemcpyHostToDevice), {});
+    TP_CUDA_OK(cudaMemcpyAsync(D.lm_ys, ys, m * sizeof(double), cudaMemcpyHostToDevice, q), {});
     const double f = 1.0;
     const int32_t zero = 0, one = 1, queue[3] = {1, 1, 0};
-    TP_CUDA_OK(cudaMemcpy(D.f, &f, sizeof(double), cudaMemcpyHostToDevice), {});
-    TP_CUDA_OK(cudaMemcpy(D.st, &st, sizeof(st), cudaMemcpyHostToDevice), {});
-    TP_CUDA_OK(cudaMemcpy(D.slot_gid, &zero, sizeof(int32_t), cudaMemcpyHostToDevice), {});
-    TP_CUDA_OK(cudaMemcpy(D.list + (size_t)TP_TICKS * D.n_slots, &zero, sizeof(int32_t), cudaMemcpyHostToDevice), {});
-    TP_CUDA_OK(cudaMemcpy(D.count + TP_TICKS, &one, sizeof(int32_t), cudaMemcpyHostToDevice), {});
-    TP_CUDA_OK(cudaMemcpy(D.queue, queue, sizeof(queue), cudaMemcpyHostToDevice), {});
+    TP_CUDA_OK(cudaMemcpyAsync(D.f, &f, sizeof(double), cudaMemcpyHostToDevice, q), {});
+    TP_CUDA_OK(cudaMemcpyAsync(D.st, &st, sizeof(st), cudaMemcpyHostToDevice, q), {});
+    TP_CUDA_OK(cudaMemcpyAsync(D.slot_gid, &zero, sizeof(int32_t), cudaMemcpyHostToDevice, q), {});
+    TP_CUDA_OK(cudaMemcpyAsync(D.list + (size_t)TP_TICKS * D.n_slots, &zero, sizeof(int32_t), cudaMemcpyHostToDevice, q),
+               {});
+    TP_CUDA_OK(cudaMemcpyAsync(D.count + TP_TICKS, &one, sizeof(int32_t), cudaMemcpyHostToDevice, q), {});
+    TP_CUDA_OK(cudaMemcpyAsync(D.queue, queue, sizeof(queue), cudaMemcpyHostToDevice, q), {});
     TpLaunches launches;
     launch_cand(s, s->lane[0], TP_MODE_ADVANCE, TP_TICKS, -1, 1, launches);
     launches.add_to(s->stats);
     TP_CUDA_OK(cudaStreamSynchronize(q), {});
     TP_CUDA_OK(cudaGetLastError(), {});
     s->n_cand = 0;   // not a solvable upload
-    TP_CUDA_OK(cudaMemcpy(d_out, D.d, n_vars * sizeof(double), cudaMemcpyDeviceToHost), {});
-    TP_CUDA_OK(cudaMemcpy(&st, D.st, sizeof(st), cudaMemcpyDeviceToHost), {});
+    int rc = tp_download(q, d_out, D.d, n_vars * sizeof(double));
+    if (rc == TOPAY_OK) rc = tp_download(q, &st, D.st, sizeof(st));
+    if (rc != TOPAY_OK) return rc;
     if (st.phase != 2) {
         tp_set_error("debug_direction: the crafted iteration did not reach the two-loop (ys <= cautious bound or "
                      "an ascent direction)");
@@ -1179,11 +1169,12 @@ extern "C" int topay_solver_phase_clocks(topay_solver* s, int enable, long long*
     drop_graphs(s);   // captured kernel arguments change
     if (enable && !D.prof) {
         TP_CUDA_OK(cudaMalloc(&D.prof, 16 * sizeof(long long)), {});
-        cudaMemset(D.prof, 0, 16 * sizeof(long long));
+        TP_CUDA_OK(cudaMemsetAsync(D.prof, 0, 16 * sizeof(long long), s->stream), {});
     }
     if (out16 && D.prof) {
-        TP_CUDA_OK(cudaMemcpy(out16, D.prof, 16 * sizeof(long long), cudaMemcpyDeviceToHost), {});
-        cudaMemset(D.prof, 0, 16 * sizeof(long long));
+        const int rc = tp_download(s->stream, out16, D.prof, 16 * sizeof(long long));
+        if (rc != TOPAY_OK) return rc;
+        TP_CUDA_OK(cudaMemsetAsync(D.prof, 0, 16 * sizeof(long long), s->stream), {});
     }
     if (!enable && D.prof) {
         cudaFree(D.prof);
@@ -1213,7 +1204,7 @@ extern "C" int topay_solver_set_trace(topay_solver* s, int cap) {
     if (cap > 0) {
         TP_CUDA_OK(cudaMalloc(&D.trace, (size_t)D.max_cand * cap * 4 * sizeof(double)), {});
         TP_CUDA_OK(cudaMalloc(&D.trace_len, (size_t)D.max_cand * sizeof(int32_t)), {});
-        cudaMemset(D.trace_len, 0, (size_t)D.max_cand * sizeof(int32_t));
+        TP_CUDA_OK(cudaMemsetAsync(D.trace_len, 0, (size_t)D.max_cand * sizeof(int32_t), s->stream), {});
     }
     return TOPAY_OK;
 }
@@ -1221,13 +1212,17 @@ extern "C" int topay_solver_set_trace(topay_solver* s, int cap) {
 extern "C" int topay_solver_download_trace(topay_solver* s, int cand, double* out, int cap, int32_t* len) {
     if (!s || !out || !len || cand < 0 || cand >= s->dev.max_cand) return TOPAY_ERR_INVALID_ARG;
     const TpSolverDev& D = s->dev;
-    if (!D.trace) return TOPAY_ERR_NOT_READY;
+    if (!D.trace) {
+        tp_set_error("no trace recorded: call topay_solver_set_trace first");
+        return TOPAY_ERR_NOT_READY;
+    }
     cudaSetDevice(s->device);
     int32_t n = 0;
-    TP_CUDA_OK(cudaMemcpy(&n, D.trace_len + cand, sizeof(int32_t), cudaMemcpyDeviceToHost), {});
+    int rc = tp_download(s->stream, &n, D.trace_len + cand, sizeof(int32_t));
+    if (rc != TOPAY_OK) return rc;
     n = std::min(n, cap);
-    TP_CUDA_OK(cudaMemcpy(out, D.trace + (size_t)cand * D.trace_cap * 4, (size_t)n * 4 * sizeof(double),
-                          cudaMemcpyDeviceToHost), {});
+    rc = tp_download(s->stream, out, D.trace + (size_t)cand * D.trace_cap * 4, (size_t)n * 4 * sizeof(double));
+    if (rc != TOPAY_OK) return rc;
     *len = n;
     return TOPAY_OK;
 }

@@ -361,57 +361,41 @@ int TpTrajChecker::check(const TpTrajView& V, const TpParams& P, const TpGrid& g
 
 namespace {
 
-// host batch -> device copy + view; owns the device memory for the duration of one call
-struct HostBatchOnDevice {
-    void* buf = nullptr;
-    TpTrajView V{};
-    ~HostBatchOnDevice() {
-        if (buf) cudaFree(buf);
+// Checks a host batch and stages it through `io`; *V views the device copy.
+int stage_batch(const topay_traj_batch* b, TpStaging& io, TpTrajView* V) {
+    if (!b || b->n_traj < 1 || b->max_pieces < 1 || !b->piece_num || !b->T || !b->coeff || !b->start_se2) {
+        tp_set_error("trajectory batch: null pointer or empty batch");
+        return TOPAY_ERR_INVALID_ARG;
     }
-    int upload(const topay_traj_batch* b, cudaStream_t q) {
-        if (!b || b->n_traj < 1 || b->max_pieces < 1 || !b->piece_num || !b->T || !b->coeff || !b->start_se2) {
-            tp_set_error("trajectory batch: null pointer or empty batch");
+    const size_t n = b->n_traj, NP = b->max_pieces;
+    for (size_t i = 0; i < n; i++)
+        if (b->piece_num[i] < 1 || b->piece_num[i] > (int)NP) {
+            tp_set_error("trajectory batch: piece_num outside 1..max_pieces");
             return TOPAY_ERR_INVALID_ARG;
         }
-        const size_t n = b->n_traj, NP = b->max_pieces;
-        for (size_t i = 0; i < n; i++)
-            if (b->piece_num[i] < 1 || b->piece_num[i] > (int)NP) {
-                tp_set_error("trajectory batch: piece_num outside 1..max_pieces");
-                return TOPAY_ERR_INVALID_ARG;
-            }
-        const size_t bT = n * NP * 8, bC = n * 6 * NP * 9 * 8, bS = n * 3 * 8, bN = ((n * 4 + 7) / 8) * 8;
-        TP_CUDA_OK(cudaMalloc(&buf, bT + bC + bS + bN), {});
-        char* p = (char*)buf;
-        cudaMemcpyAsync(p, b->T, bT, cudaMemcpyHostToDevice, q);
-        cudaMemcpyAsync(p + bT, b->coeff, bC, cudaMemcpyHostToDevice, q);
-        cudaMemcpyAsync(p + bT + bC, b->start_se2, bS, cudaMemcpyHostToDevice, q);
-        cudaMemcpyAsync(p + bT + bC + bS, b->piece_num, n * 4, cudaMemcpyHostToDevice, q);
-        V.n = (int)n;
-        V.max_pieces = (int)NP;
-        V.T = (const double*)p;
-        V.coeff = (const double*)(p + bT);
-        V.start = (const double*)(p + bT + bC);
-        V.piece_num = (const int32_t*)(p + bT + bC + bS);
-        return TOPAY_OK;
-    }
-};
+    V->n = (int)n;
+    V->max_pieces = (int)NP;
+    V->T = io.in(b->T, n * NP);
+    V->coeff = io.in(b->coeff, n * 6 * NP * 9);
+    V->start = io.in(b->start_se2, n * 3);
+    V->piece_num = io.in(b->piece_num, n);
+    return io.ok() ? TOPAY_OK : io.finish();
+}
 
 }  // namespace
 
 extern "C" int topay_traj_check_feasible(topay_field* f, const topay_robot_params* robot, const topay_traj_batch* trajs,
                                          topay_feasibility* out) {
     if (!f || !robot || !out || !out->feasible) return TOPAY_ERR_INVALID_ARG;
-    if (!tp_field_ready(f)) {
-        tp_set_error("feasibility check on a field that was not rebuilt");
-        return TOPAY_ERR_NOT_READY;
-    }
+    int rc = tp_field_require_ready(f);
+    if (rc != TOPAY_OK) return rc;
     const int dev = tp_field_device(f);
     cudaSetDevice(dev);
     cudaStream_t q;
     TP_CUDA_OK(cudaStreamCreateWithFlags(&q, cudaStreamNonBlocking), {});
-    int rc;
     {
-        HostBatchOnDevice hb;
+        TpStaging io(q);
+        TpTrajView V{};
         TpTrajChecker ck;
         TpParams P;
         memset(&P, 0, sizeof(P));
@@ -420,9 +404,9 @@ extern "C" int topay_traj_check_feasible(topay_field* f, const topay_robot_param
         tp_derive_params(P);
         TpGrid g;
         tp_field_grid(f, &g);
-        rc = hb.upload(trajs, q);
+        rc = stage_batch(trajs, io, &V);
         if (rc == TOPAY_OK) rc = ck.init(dev, q);
-        if (rc == TOPAY_OK) rc = ck.check(hb.V, P, g, out);
+        if (rc == TOPAY_OK) rc = ck.check(V, P, g, out);
         cudaStreamSynchronize(q);
     }
     cudaStreamDestroy(q);
@@ -437,13 +421,14 @@ extern "C" int topay_traj_car_seq(int device, const topay_traj_batch* trajs, int
     cudaStream_t q;
     TP_CUDA_OK(cudaStreamCreateWithFlags(&q, cudaStreamNonBlocking), {});
     {
-        HostBatchOnDevice hb;
+        TpStaging io(q);
+        TpTrajView V{};
         TpTrajChecker ck;
-        rc = hb.upload(trajs, q);
+        rc = stage_batch(trajs, io, &V);
         if (rc == TOPAY_OK) rc = ck.init(device, q);
-        if (rc == TOPAY_OK) rc = ck.prepare(hb.V);
+        if (rc == TOPAY_OK) rc = ck.prepare(V);
         if (rc == TOPAY_OK) {
-            for (int i = 0; i < hb.V.n && rc == TOPAY_OK; i++) {
+            for (int i = 0; i < V.n && rc == TOPAY_OK; i++) {
                 len[i] = ck.h_meta[i].n_seq;
                 if (len[i] > cap) {
                     tp_set_error("car_seq longer than cap");
@@ -473,31 +458,20 @@ extern "C" int topay_traj_sample(int device, const topay_traj_batch* trajs, cons
     cudaStream_t q;
     TP_CUDA_OK(cudaStreamCreateWithFlags(&q, cudaStreamNonBlocking), {});
     {
-        HostBatchOnDevice hb;
+        TpStaging io(q);
+        TpTrajView V{};
         TpTrajChecker ck;
-        double* d = nullptr;
-        rc = hb.upload(trajs, q);
+        rc = stage_batch(trajs, io, &V);
         if (rc == TOPAY_OK) rc = ck.init(device, q);
-        if (rc == TOPAY_OK) rc = ck.prepare(hb.V);
+        if (rc == TOPAY_OK) rc = ck.prepare(V);
         if (rc == TOPAY_OK) {
-            const size_t nm = (size_t)hb.V.n * m;
-            if (cudaMallocAsync(&d, nm * 21 * 8, q) != cudaSuccess) {
-                tp_set_error("traj_sample: cudaMalloc failed");
-                rc = TOPAY_ERR_ALLOC;
-            } else {
-                cudaMemcpyAsync(d, t, nm * 8, cudaMemcpyHostToDevice, q);
-                dim3 grid((m + 127) / 128, hb.V.n);
-                k_traj_sample<<<grid, 128, 0, q>>>(hb.V, ck.meta, ck.car_seq, d, m, state ? d + nm : nullptr,
-                                                   dstate ? d + nm * 11 : nullptr);
-                if (state) cudaMemcpyAsync(state, d + nm, nm * 80, cudaMemcpyDeviceToHost, q);
-                if (dstate) cudaMemcpyAsync(dstate, d + nm * 11, nm * 80, cudaMemcpyDeviceToHost, q);
-            }
-        }
-        if (d) cudaFreeAsync(d, q);
-        cudaError_t e = cudaStreamSynchronize(q);
-        if (rc == TOPAY_OK && e != cudaSuccess) {
-            tp_set_error(std::string("traj_sample: ") + cudaGetErrorString(e));
-            rc = TOPAY_ERR_CUDA;
+            const size_t nm = (size_t)V.n * m;
+            const double* dt = io.in(t, nm);
+            double* ds = io.out(state, nm * 10);
+            double* dd = io.out(dstate, nm * 10);
+            if (io.ok())
+                k_traj_sample<<<dim3((m + 127) / 128, V.n), 128, 0, q>>>(V, ck.meta, ck.car_seq, dt, m, ds, dd);
+            rc = io.finish();
         }
     }
     cudaStreamDestroy(q);
