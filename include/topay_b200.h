@@ -71,7 +71,10 @@ enum {
     TOPAY_LBFGSERR_INCREASEGRADIENT = -1005,
     /* not a reference code: the device solve stopped this candidate at its hard cap on evaluations
      * (topay_solver_run); the candidate comes back with status 0 */
-    TOPAY_LBFGSERR_TICK_CAP = -2000
+    TOPAY_LBFGSERR_TICK_CAP = -2000,
+    /* not a reference code: the candidate was cancelled because its plan had succeeded more than the grace period
+     * earlier (topay_solver_set_plans); it comes back with status 0 */
+    TOPAY_LBFGSERR_PLAN_GRACE = -2001
 };
 
 /* ------------------------------------------------------------------ params */
@@ -518,6 +521,23 @@ int topay_solver_run(topay_solver* s);          /* device solve of the uploaded 
  * group of scenarios shares the launches of one solve. The assignment holds for uploads of the same size until it is
  * changed; n_fields <= 1 returns to the solver's own field. Call after topay_solver_upload. */
 int topay_solver_assign_fields(topay_solver* s, topay_field* const* fields, int n_fields, const int32_t* field_of);
+/* First success + grace of the planner's worker pool (planner.cpp:931-952), with the grace counted in evaluations
+ * instead of the reference's 100 ms of wall-clock time, so that the outcome does not depend on scheduling. The upload
+ * is read as n_plans plans, plan p = candidates plan_offset[p] .. plan_offset[p+1]-1 (n_plans + 1 entries, starting
+ * at 0, non-decreasing, ending at the uploaded n_cand). All candidates of a plan count as started together.
+ *   A candidate succeeds when it ends with status 1 and, with use_gate != 0, printConstraintsSituations passes
+ *   (feasible_print, planner.cpp:877-880). S_p = the fewest evaluations (result `evals`) among the candidates of plan p
+ *   that succeed when nothing is cancelled; no success: S_p = infinity.
+ *   A candidate with evals <= S_p + grace_evals in that unbounded run is KEPT: its results, trace and gate metrics
+ *   are bit-identical to the unbounded run. Every other candidate of the plan is CANCELLED: status 0, lbfgs_code
+ *   TOPAY_LBFGSERR_PLAN_GRACE, piece_num kept, iters, evals, alm_rounds, cost, duration, T, coeff, final_xy_err and x
+ *   zero, an empty trace, both gate verdicts, n_samples and every gate metric zero.
+ * So a plan has a winner if and only if it has one unbounded (its earliest success is never cancelled), and the
+ * result depends on each candidate's own evaluation count only: not on slots, lanes, timed mode or queue order.
+ * Cancelled candidates free their slots at once. The setting holds for uploads of the same size until it is changed
+ * (topay_solver_run refuses an upload of another size with TOPAY_ERR_NOT_READY); n_plans == 0 turns it off. Call after
+ * topay_solver_upload. Malformed offsets, grace_evals < 0 or n_plans > n_cand: TOPAY_ERR_INVALID_ARG. */
+int topay_solver_set_plans(topay_solver* s, int n_plans, const int32_t* plan_offset, int use_gate, int32_t grace_evals);
 int topay_solver_download(topay_solver* s, topay_result_batch* out, int32_t* best_by_duration,
                           int32_t* best_by_cost);
 

@@ -320,10 +320,26 @@ public:
         topay_result_batch out = {};
         out.status = status_.data(); out.piece_num = pieces_.data(); out.cost = cost_.data();
         out.T = T_.data(); out.coeff = coeff_.data();
-        topay_check(topay_solver_solve_batch(s_, n, len.data(), all.data(), bvel, bacc, &out, &best_by_duration,
-                                             &best_by_cost), "topay_solver_solve_batch");
+        if (grace_evals_ < 0) {
+            topay_check(topay_solver_solve_batch(s_, n, len.data(), all.data(), bvel, bacc, &out, &best_by_duration,
+                                                 &best_by_cost), "topay_solver_solve_batch");
+        } else {   // the batch is one plan: its first success + grace under the planner's success test
+            topay_check(topay_solver_upload(s_, n, len.data(), all.data(), bvel, bacc), "topay_solver_upload");
+            const int32_t off[2] = {0, n};
+            topay_check(topay_solver_set_plans(s_, 1, off, 1, grace_evals_), "topay_solver_set_plans");
+            topay_check(topay_solver_run(s_), "topay_solver_run");
+            topay_check(topay_solver_download(s_, &out, &best_by_duration, &best_by_cost), "topay_solver_download");
+        }
         traj_cost = cost_[0];
         return std::vector<int>(status_.begin(), status_.end());
+    }
+    // First success + grace of the planner's worker pool (planner.cpp:931-952), counted in evaluations: from the next
+    // optimizeTrajBatch on, once a candidate passes optimizeTraj && printConstraintsSituations, the candidates that
+    // need more than `evals` evaluations beyond it are cancelled (status 0, TOPAY_LBFGSERR_PLAN_GRACE), and
+    // selectFeasible sees them as failed. evals < 0 turns it off (the default).
+    void setGrace(int evals) {
+        if (evals < 0 && grace_evals_ >= 0) topay_check(topay_solver_set_plans(s_, 0, nullptr, 0, 0), "topay_solver_set_plans");
+        grace_evals_ = evals < 0 ? -1 : evals;
     }
     // MomaTraj getTraj() const (moma_traj_opt.h:943-946)
     MomaTraj getTraj(int idx = 0) const {
@@ -386,6 +402,7 @@ private:
     GridMap::Ptr grid_map;
     topay_solver* s_ = nullptr;
     int max_cand_, max_pieces_;
+    int grace_evals_ = -1;
     std::vector<int32_t> status_, pieces_;
     std::vector<double> cost_, T_, coeff_, starts_;
 };

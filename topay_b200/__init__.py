@@ -4,7 +4,7 @@ The product is topay_b200/libtopay_b200.so (kernels in csrc/, C ABI in include/t
 this package is the host-side mirror of the two reference interfaces it replaces:
 GridMap (field.py), rog_map::ESDFMap (rog.py) and MomaTrajOpt (optimizer.py).
 """
-from ._structs import (LBFGSERR_TICK_CAP, MAP2D_CRITICAL, MAP2D_FLAT, MAP2D_INFLATE, MAP3D, TERM_NAMES, GridDesc, OptParams,
+from ._structs import (LBFGSERR_PLAN_GRACE, LBFGSERR_TICK_CAP, MAP2D_CRITICAL, MAP2D_FLAT, MAP2D_INFLATE, MAP3D, TERM_NAMES, GridDesc, OptParams,
                        RobotParams, RogDesc, grid_desc, num_vars, prob_desc, rog_desc)
 from .field import GridMap, robot_params_default
 from .rog import ESDFMap, ProbMap
@@ -13,4 +13,5 @@ from .optimizer import (MomaTraj, MomaTrajOpt, discretizePath, getDensePath, opt
 
 __all__ = ["GridMap", "ESDFMap", "ProbMap", "prob_desc", "rog_desc", "RogDesc", "MomaTrajOpt", "MomaTraj", "grid_desc", "GridDesc", "OptParams", "RobotParams",
            "robot_params_default", "opt_params_default", "prepare_candidate", "getDensePath", "discretizePath", "pathLength", "num_vars", "TERM_NAMES",
-           "MAP2D_FLAT", "MAP2D_INFLATE", "MAP2D_CRITICAL", "MAP3D", "LBFGSERR_TICK_CAP"]
+           "MAP2D_FLAT", "MAP2D_INFLATE", "MAP2D_CRITICAL", "MAP3D", "LBFGSERR_TICK_CAP",
+           "LBFGSERR_PLAN_GRACE"]

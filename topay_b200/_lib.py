@@ -113,6 +113,7 @@ PROTOTYPES = {
     "topay_solver_upload": (C.c_int, [C.c_void_p, C.c_int, _ip, _dp, _dp, _dp]),
     "topay_solver_run": (C.c_int, [C.c_void_p]),
     "topay_solver_assign_fields": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.c_int, _ip]),
+    "topay_solver_set_plans": (C.c_int, [C.c_void_p, C.c_int, _ip, C.c_int, C.c_int32]),
     "topay_solver_download": (C.c_int, [C.c_void_p, C.POINTER(ResultBatch), _ip, _ip]),
     "topay_solver_set_trace": (C.c_int, [C.c_void_p, C.c_int]),
     "topay_solver_download_trace": (C.c_int, [C.c_void_p, C.c_int, _dp, C.c_int, _ip]),

@@ -8,6 +8,7 @@ TERM_NAMES = ["jerk", "time", "chassis_colli", "moment", "acc", "domega", "mani_
               "self_colli", "mani_pos", "mani_vel", "mani_acc", "mean_time", "endp"]
 MAP2D_FLAT, MAP2D_INFLATE, MAP2D_CRITICAL, MAP3D = 0, 1, 2, 3
 LBFGSERR_TICK_CAP = -2000      # TOPAY_LBFGSERR_TICK_CAP: stopped by the solver's hard cap on ticks
+LBFGSERR_PLAN_GRACE = -2001    # TOPAY_LBFGSERR_PLAN_GRACE: cancelled by its plan's first success + grace
 
 
 class RobotParams(C.Structure):

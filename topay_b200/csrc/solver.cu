@@ -106,6 +106,11 @@ struct topay_solver {
     TpTrajChecker* checker;
     int32_t* d_pn;
     double* d_start;
+    // first success + grace (topay_solver_set_plans): dev.plan_of points at d_plan_of while it is on
+    int n_plans;
+    int plans_n_cand;           // the upload size the plans were set for
+    int32_t *d_plan_of, *d_plan_first, *d_pending;   // [max_cand], [max_cand], [1 + max_cand]; allocated on first use
+    bool grace_ran;             // the last run cancelled by the grace rule (check_feasible clears their verdicts)
 };
 
 namespace {
@@ -274,6 +279,10 @@ static int solver_create(const topay_opt_params* opt, const topay_robot_params* 
     s->checker = nullptr;
     s->d_pn = nullptr;
     s->d_start = nullptr;
+    s->n_plans = 0;
+    s->plans_n_cand = 0;
+    s->d_plan_of = s->d_plan_first = s->d_pending = nullptr;
+    s->grace_ran = false;
     memset(&s->stats, 0, sizeof(s->stats));
     cudaSetDevice(s->device);
     tp_pool_keep(s->device);
@@ -695,12 +704,151 @@ static void mark_tick_cap(topay_solver* s, const TpLane& L, int n_store) {
     k_mark_tick_cap<<<(std::max(n_store, s->dev.n_slots) + 127) / 128, 128, 0, s->stream>>>(lane_dev(s, L), n_store);
 }
 
+// Piece counts live in the per-candidate state and the start pose is split over start_xy and the
+// yaw slot of head_pva; gather both into the layout the trajectory kernels read.
+__global__ void k_solver_traj_view(const TpCandState* __restrict__ st, const double* __restrict__ start_xy,
+                                   const double* __restrict__ head_pva, int n, int32_t* pn, double* start) {
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= n) return;
+    pn[c] = st[c].N;
+    start[3 * c] = start_xy[2 * c];
+    start[3 * c + 1] = start_xy[2 * c + 1];
+    start[3 * c + 2] = head_pva[(size_t)c * 27];
+}
+
+// The success gate's checker and its staging buffers, built on first use.
+static int solver_checker(topay_solver* s) {
+    if (s->checker) return TOPAY_OK;
+    int rc;
+    if ((rc = s->bufs.alloc(&s->d_pn, (size_t)s->dev.max_cand)) != TOPAY_OK) return rc;
+    if ((rc = s->bufs.alloc(&s->d_start, (size_t)s->dev.max_cand * 3)) != TOPAY_OK) return rc;
+    s->checker = new TpTrajChecker();
+    return s->checker->init(s->device, s->stream);
+}
+
+// ---- first success + grace (topay_solver_set_plans)
+
+// Start of a run: no plan has a success yet, nothing waits for the gate.
+__global__ void k_plan_reset(const __grid_constant__ TpSolverDev S, int n_plans) {
+    for (int p = threadIdx.x; p < n_plans; p += blockDim.x) S.plan_first[p] = INT32_MAX;
+    if (threadIdx.x == 0) S.pending[0] = 0;
+}
+
+// After the gate of the m waiting successes (verdict i = S.pending[1 + i]): the ones that pass publish their
+// evaluation count to their plan; the list is emptied.
+__global__ void k_plan_publish(const __grid_constant__ TpSolverDev S, const TpFeasOut* __restrict__ feas, int m) {
+    for (int i = threadIdx.x; i < m; i += blockDim.x)
+        if (feas[i].feasible_print) {
+            const int gid = S.pending[1 + i];
+            atomicMin(S.plan_first + S.plan_of[gid], S.res_st[gid].evals_total);
+        }
+    __syncthreads();
+    if (threadIdx.x == 0) S.pending[0] = 0;
+}
+
+// End of a run, one CTA per candidate: every candidate of the store with more evaluations than its plan's first
+// success + grace leaves with the cancelled values, whether the device stopped it or it finished before the
+// plan's first success was known.
+__global__ void k_plan_fixup(const __grid_constant__ TpSolverDev S) {
+    const int gid = blockIdx.x;
+    const TpCandState st = S.res_st[gid];
+    const bool cancel = st.evals_total - S.grace > S.plan_first[S.plan_of[gid]];
+    __syncthreads();   // every thread has read res_st before thread 0 rewrites it
+    if (!cancel) return;
+    for (int i = threadIdx.x; i < S.max_pieces; i += blockDim.x) S.res_T[(size_t)gid * S.max_pieces + i] = 0.0;
+    for (int i = threadIdx.x; i < 6 * S.max_pieces * 9; i += blockDim.x)
+        S.res_coeff[(size_t)gid * 6 * S.max_pieces * 9 + i] = 0.0;
+    for (int i = threadIdx.x; i < S.xs; i += blockDim.x) S.res_x[(size_t)gid * S.xs + i] = 0.0;
+    if (threadIdx.x == 0) {
+        TpCandState z{};
+        z.N = st.N;
+        z.n = st.n;
+        z.last_code = TOPAY_LBFGSERR_PLAN_GRACE;
+        S.res_st[gid] = z;
+        if (S.trace) S.trace_len[gid] = 0;
+    }
+}
+
+// Gate verdicts of a candidate the grace rule cancelled: all zero.
+__global__ void k_plan_clear_gate(const TpCandState* __restrict__ st, TpFeasOut* feas, int n) {
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c < n && st[c].last_code == TOPAY_LBFGSERR_PLAN_GRACE) feas[c] = TpFeasOut{};
+}
+
+// use_gate: the m successes waiting in S.pending go through the same checker as topay_solver_check_feasible, and
+// those that pass printConstraintsSituations publish. Enqueued between two batches, outside their graph.
+static int gate_pending(topay_solver* s, int m, TpLaunches& n) {
+    int rc = solver_checker(s);
+    if (rc != TOPAY_OK) return rc;
+    const TpSolverDev& D = s->dev;
+    k_solver_traj_view<<<(s->n_cand + 127) / 128, 128, 0, s->stream>>>(D.res_st, D.start_xy, D.head_pva, s->n_cand,
+                                                                       s->d_pn, s->d_start);
+    const TpTrajView V{m, D.max_pieces, s->d_pn, D.res_T, D.res_coeff, s->d_start, D.pending + 1};
+    TpGrid G;
+    solver_grid(s, &G);
+    rc = s->checker->run(V, s->params, G, D.n_fields > 1 ? D.grids : nullptr, D.field_of);
+    s->checker->checked_n = 0;   // `feas` now holds these m verdicts, not those of a whole solve
+    if (rc != TOPAY_OK) return rc;
+    k_plan_publish<<<1, 256, 0, s->stream>>>(D, s->checker->feas, m);
+    n.kernels += 5;   // traj view, the checker's three, publish
+    return TOPAY_OK;
+}
+
+extern "C" int topay_solver_set_plans(topay_solver* s, int n_plans, const int32_t* plan_offset, int use_gate,
+                                      int32_t grace_evals) {
+    if (!s || n_plans < 0) return TOPAY_ERR_INVALID_ARG;
+    cudaSetDevice(s->device);
+    TpSolverDev& D = s->dev;
+    if (n_plans == 0) {
+        if (D.plan_of) drop_graphs(s);   // the captured kernel arguments change
+        D.plan_of = nullptr;
+        D.grace = D.plan_gate = 0;
+        s->n_plans = 0;
+        return TOPAY_OK;
+    }
+    const int n = s->n_cand;
+    if (n < 1 || n_plans > n || !plan_offset || grace_evals < 0) {
+        tp_set_error("topay_solver_set_plans: needs an upload, at most n_cand plans and grace_evals >= 0");
+        return TOPAY_ERR_INVALID_ARG;
+    }
+    bool ok = plan_offset[0] == 0 && plan_offset[n_plans] == n;
+    for (int p = 0; ok && p < n_plans; p++) ok = plan_offset[p] <= plan_offset[p + 1];
+    if (!ok) {
+        tp_set_error("topay_solver_set_plans: plan_offset must start at 0, never decrease and end at n_cand");
+        return TOPAY_ERR_INVALID_ARG;
+    }
+    int rc;
+    if (!s->d_plan_of) {
+        if ((rc = s->bufs.alloc(&s->d_plan_of, (size_t)D.max_cand)) != TOPAY_OK) return rc;
+        if ((rc = s->bufs.alloc(&s->d_plan_first, (size_t)D.max_cand)) != TOPAY_OK) return rc;
+        if ((rc = s->bufs.alloc(&s->d_pending, (size_t)D.max_cand + 1)) != TOPAY_OK) return rc;
+    }
+    std::vector<int32_t> plan_of(n);
+    for (int p = 0; p < n_plans; p++) std::fill(plan_of.begin() + plan_offset[p], plan_of.begin() + plan_offset[p + 1], p);
+    TP_CUDA_OK(cudaMemcpyAsync(s->d_plan_of, plan_of.data(), (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, s->stream), {});
+    TP_CUDA_OK(cudaStreamSynchronize(s->stream), {});
+    const int gate = use_gate != 0;
+    if (D.plan_of != s->d_plan_of || D.grace != grace_evals || D.plan_gate != gate) drop_graphs(s);
+    D.plan_of = s->d_plan_of;
+    D.plan_first = s->d_plan_first;
+    D.pending = s->d_pending;
+    D.grace = grace_evals;
+    D.plan_gate = gate;
+    s->n_plans = n_plans;
+    s->plans_n_cand = n;
+    return TOPAY_OK;
+}
+
 extern "C" int topay_solver_run(topay_solver* s) {
     if (!s || s->n_cand < 1) return TOPAY_ERR_INVALID_ARG;
     const int rc = solver_require_ready(s);
     if (rc != TOPAY_OK) return rc;
     if (s->dev.n_fields > 1 && s->fields_n_cand != s->n_cand) {
         tp_set_error("the field assignment was made for an upload of another size: call topay_solver_assign_fields again");
+        return TOPAY_ERR_NOT_READY;
+    }
+    if (s->dev.plan_of && s->plans_n_cand != s->n_cand) {
+        tp_set_error("the plans were set for an upload of another size: call topay_solver_set_plans again");
         return TOPAY_ERR_NOT_READY;
     }
     cudaSetDevice(s->device);
@@ -713,9 +861,15 @@ extern "C" int topay_solver_run(topay_solver* s) {
     cudaEventRecord(s->ev_begin, q);
     // the store holds the uploaded initial state, so repeated runs do identical work
     TpLane &A = s->lane[0], &B = s->lane[1];
+    TpLaunches first;
+    s->grace_ran = D.plan_of != nullptr;
+    const bool gate = D.plan_of && D.plan_gate;   // successes wait for the gate between batches
+    if (D.plan_of) {
+        k_plan_reset<<<1, 256, 0, q>>>(D, s->n_plans);
+        first.kernels += 1;
+    }
     A.live = seed_slots(s);
     B.live = 0;
-    TpLaunches first;
     launch_cand(s, A, TP_MODE_GEN, TP_TICKS, -1, A.live, first);
     first.kernels += 1;   // seed_slots' k_slot_init
     first.add_to(s->stats);
@@ -769,6 +923,7 @@ extern "C" int topay_solver_run(topay_solver* s) {
             enqueue_batch(s, ny, 0, true).add_to(s->stats);
             cudaMemcpyAsync(s->h_nodes, D.node_count, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, q);
         }
+        if (gate) cudaMemcpyAsync(s->h_active + 5, D.pending, sizeof(int32_t), cudaMemcpyDeviceToHost, q);
         ticks += TP_TICKS;
         slot_ticks += (long long)(A.live + B.live) * TP_TICKS;
         // spin while at most two solves run in this process (lowest latency, one busy core per plan), else sleep
@@ -811,11 +966,21 @@ extern "C" int topay_solver_run(topay_solver* s) {
         A.live = live_after;
         if (s->lanes == 2) B.live = *B.h_live;
         done = A.live + B.live == 0;
+        if (gate && s->h_active[5] > 0) {   // also after the last batch: nothing waits when the run ends
+            TpLaunches g;
+            const int grc = gate_pending(s, s->h_active[5], g);
+            if (grc != TOPAY_OK) return grc;
+            g.add_to(s->stats);
+        }
     }
     if (!done) {
         if (s->lanes == 2) mark_tick_cap(s, B, 0);
         mark_tick_cap(s, A, s->n_cand);
         tp_set_error("tick cap reached: unfinished candidates carry TOPAY_LBFGSERR_TICK_CAP");
+    }
+    if (D.plan_of) {   // last, so that a candidate past its plan's first success + grace carries the grace code
+        k_plan_fixup<<<s->n_cand, 128, 0, q>>>(D);
+        s->stats.kernel_launches += 1;
     }
     cudaEventRecord(s->ev_end, q);
     cudaMemcpyAsync(s->h_nodes, D.node_count, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, q);
@@ -923,30 +1088,13 @@ extern "C" int topay_solver_solve_batch(topay_solver* s, int n_cand, const int32
     return topay_solver_download(s, out, best_by_duration, best_by_cost);
 }
 
-// Piece counts live in the per-candidate state and the start pose is split over start_xy and the
-// yaw slot of head_pva; gather both into the layout the trajectory kernels read.
-__global__ void k_solver_traj_view(const TpCandState* __restrict__ st, const double* __restrict__ start_xy,
-                                   const double* __restrict__ head_pva, int n, int32_t* pn, double* start) {
-    const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= n) return;
-    pn[c] = st[c].N;
-    start[3 * c] = start_xy[2 * c];
-    start[3 * c + 1] = start_xy[2 * c + 1];
-    start[3 * c + 2] = head_pva[(size_t)c * 27];
-}
-
 extern "C" int topay_solver_check_feasible(topay_solver* s, topay_feasibility* out, int32_t* best_success) {
     if (!s || !out || !out->feasible || s->n_cand < 1) return TOPAY_ERR_INVALID_ARG;
     cudaSetDevice(s->device);
     TpSolverDev& D = s->dev;
     const int n = s->n_cand, NP = D.max_pieces;
     int rc;
-    if (!s->checker) {
-        if ((rc = s->bufs.alloc(&s->d_pn, (size_t)D.max_cand)) != TOPAY_OK) return rc;
-        if ((rc = s->bufs.alloc(&s->d_start, (size_t)D.max_cand * 3)) != TOPAY_OK) return rc;
-        s->checker = new TpTrajChecker();
-        if ((rc = s->checker->init(s->device, s->stream)) != TOPAY_OK) return rc;
-    }
+    if ((rc = solver_checker(s)) != TOPAY_OK) return rc;
     k_solver_traj_view<<<(n + 127) / 128, 128, 0, s->stream>>>(D.res_st, D.start_xy, D.head_pva, n, s->d_pn, s->d_start);
     TpTrajView V{n, NP, s->d_pn, D.res_T, D.res_coeff, s->d_start};
     TpGrid G;
@@ -957,7 +1105,10 @@ extern "C" int topay_solver_check_feasible(topay_solver* s, topay_feasibility* o
         fp.resize(n);
         out->feasible_print = fp.data();
     }
-    rc = s->checker->check(V, s->params, G, out, D.n_fields > 1 ? D.grids : nullptr, D.field_of);
+    rc = s->checker->run(V, s->params, G, D.n_fields > 1 ? D.grids : nullptr, D.field_of);
+    if (rc == TOPAY_OK && s->grace_ran)
+        k_plan_clear_gate<<<(n + 127) / 128, 128, 0, s->stream>>>(D.res_st, s->checker->feas, n);
+    if (rc == TOPAY_OK) rc = s->checker->fetch(n, out);
     s->checker->checked_n = rc == TOPAY_OK ? n : 0;
     out->feasible_print = keep_fp;
     if (rc == TOPAY_OK && best_success) {
@@ -1143,7 +1294,10 @@ extern "C" int topay_solver_debug_direction(topay_solver* s, int n_vars, int bou
     TP_CUDA_OK(cudaMemcpyAsync(D.count + TP_TICKS, &one, sizeof(int32_t), cudaMemcpyHostToDevice, q), {});
     TP_CUDA_OK(cudaMemcpyAsync(D.queue, queue, sizeof(queue), cudaMemcpyHostToDevice, q), {});
     TpLaunches launches;
+    const int32_t* plan_of = s->dev.plan_of;
+    s->dev.plan_of = nullptr;   // the crafted state belongs to no plan
     launch_cand(s, s->lane[0], TP_MODE_ADVANCE, TP_TICKS, -1, 1, launches);
+    s->dev.plan_of = plan_of;
     launches.add_to(s->stats);
     TP_CUDA_OK(cudaStreamSynchronize(q), {});
     TP_CUDA_OK(cudaGetLastError(), {});

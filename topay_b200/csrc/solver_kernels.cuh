@@ -104,7 +104,21 @@ struct TpSolverDev {
     int32_t *trace_len;   // [store]
     int32_t trace_cap;
     long long *prof;      // optional phase clocks of candidate 0 (dev profiling), [16] or null
+    // first success + grace (topay_solver_set_plans); plan_of is null when it is off, and then nothing else is read
+    const int32_t* plan_of;   // [store] plan of the candidate
+    int32_t* plan_first;      // [plan] fewest evaluations of a success of the plan published so far (INT32_MAX: none)
+    int32_t* pending;         // [0] count, [1 + i] status-1 candidates waiting for the gate (plan_gate only)
+    int32_t grace;            // evaluations a plan's candidates may run past its first success
+    int32_t plan_gate;        // a success counts once printConstraintsSituations passed (published by the host's gate)
 };
+
+// plan_first[] is lowered by other CTAs and by the host's gate while the solve runs; it only ever decreases, so a value
+// read at any moment is an upper bound of the final one and a cancellation made against it stands.
+__device__ __forceinline__ int32_t tp_load_relaxed(const int32_t* p) {
+    int32_t v;
+    asm volatile("ld.relaxed.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+    return v;
+}
 
 // ------------------------------------------------------------------ warp helpers
 __device__ __forceinline__ double tp_shfl_xor(double v, int m) { return __shfl_xor_sync(0xffffffffu, v, m); }
@@ -1437,7 +1451,19 @@ k_cand(const __grid_constant__ TpSolverDev S, const __grid_constant__ TpParams P
         int ret = 0;
         enum { A_NONE, A_BEGIN_LS, A_LS_DONE, A_FINISH } action = A_NONE;
         const double f = (mode & TP_MODE_ADJ) ? f_eval : S.f[cand];   // a separate adjoint launch left it in S.f
-        if (st.ls_init) {
+        // first success + grace: past grace evaluations after its plan's earliest success the candidate is cancelled
+        // (one thread reads the bound, so that the whole CTA takes the same branch)
+        bool cancel = false;
+        if (S.plan_of) {
+            __shared__ int s_cancel;
+            if (tid == 0) s_cancel = st.evals_total - S.grace > tp_load_relaxed(S.plan_first + S.plan_of[gid]);
+            __syncthreads();
+            cancel = s_cancel != 0;
+        }
+        if (cancel) {
+            ret = TOPAY_LBFGSERR_PLAN_GRACE;
+            action = A_FINISH;
+        } else if (st.ls_init) {
             // lbfgs.hpp:522-554
             st.ls_init = 0;
             st.fx = f;
@@ -1899,7 +1925,10 @@ k_cand(const __grid_constant__ TpSolverDev S, const __grid_constant__ TpParams P
             st.last_code = ret;
             st.cost = st.fx;
             bool next_round = false;
-            if (st.phase == 1) {
+            if (cancel) {
+                st.status = 0;
+                st.phase = 0;
+            } else if (st.phase == 1) {
                 if (tp_ok_code(ret)) {
                     st.phase = 2;
                     st.lambda[0] = P.opt.alm_init_lambda[0];
@@ -1956,6 +1985,10 @@ k_cand(const __grid_constant__ TpSolverDev S, const __grid_constant__ TpParams P
             __shared__ int s_next;
             if (tid == 0) {
                 S.res_st[gid] = st;
+                if (S.plan_of && st.status == 1) {   // publish the success (through the host's gate with plan_gate)
+                    if (S.plan_gate) S.pending[1 + atomicAdd(S.pending, 1)] = gid;
+                    else atomicMin(S.plan_first + S.plan_of[gid], st.evals_total);
+                }
                 atomicAdd(S.queue + 2, 1);
                 const int q = atomicAdd(S.queue, 1);
                 s_next = q < S.queue[1] ? q : -1;

@@ -30,7 +30,10 @@
 
 namespace {
 
+__device__ __forceinline__ int traj_of(const TpTrajView& V, int i) { return V.idx ? V.idx[i] : i; }
+
 __device__ __forceinline__ TpPoly poly_of(const TpTrajView& V, int i) {
+    i = traj_of(V, i);
     TpPoly p;
     p.N = V.piece_num[i];
     p.T = V.T + (size_t)i * V.max_pieces;
@@ -70,11 +73,12 @@ k_car_seq(TpTrajView V, const TpTrajMeta* __restrict__ meta, double* __restrict_
     const TpTrajMeta m = meta[i];
     double* out = car_seq + (size_t)m.seq_off * 4;
     const double r = TP_SEQ_RES / TP_APPROX_RES, half = r / 2.0, r16 = r / 6.0;
-    double cx = V.start[3 * i], cy = V.start[3 * i + 1];
+    const double* start = V.start + 3 * traj_of(V, i);
+    double cx = start[0], cy = start[1];
     if (threadIdx.x == 0) {
         out[0] = cx;
         out[1] = cy;
-        out[2] = V.start[3 * i + 2];
+        out[2] = start[2];
         out[3] = 0.0;
     }
     for (int base = 0; base < m.seq_num; base += TP_TRAJ_THREADS) {
@@ -155,7 +159,7 @@ k_feasible(TpTrajView V, const __grid_constant__ TpParams P, const __grid_consta
     // scenario sweeps: trajectory i is checked against the field of its own scenario, grids[field_of[i]]
     __shared__ TpGrid s_grid;
     if (grids) {
-        const double* src = reinterpret_cast<const double*>(grids + field_of[blockIdx.x]);
+        const double* src = reinterpret_cast<const double*>(grids + field_of[traj_of(V, blockIdx.x)]);
         double* dst = reinterpret_cast<double*>(&s_grid);
         for (int w = threadIdx.x; w < (int)(sizeof(TpGrid) / sizeof(double)); w += TP_TRAJ_THREADS) dst[w] = src[w];
         __syncthreads();
@@ -331,14 +335,24 @@ int TpTrajChecker::prepare(const TpTrajView& V) {
 
 int TpTrajChecker::check(const TpTrajView& V, const TpParams& P, const TpGrid& g, topay_feasibility* out,
                          const TpGrid* grids, const int32_t* field_of) {
+    const int rc = run(V, P, g, grids, field_of);
+    return rc != TOPAY_OK ? rc : fetch(V.n, out);
+}
+
+int TpTrajChecker::run(const TpTrajView& V, const TpParams& P, const TpGrid& g, const TpGrid* grids,
+                       const int32_t* field_of) {
     int rc = prepare(V);
     if (rc != TOPAY_OK) return rc;
     k_feasible<<<V.n, TP_TRAJ_THREADS, 0, stream>>>(V, P, g, grids, field_of, meta, car_seq, ttab, feas);
-    std::vector<TpFeasOut> h(V.n);
-    TP_CUDA_OK(cudaMemcpyAsync(h.data(), feas, (size_t)V.n * sizeof(TpFeasOut), cudaMemcpyDeviceToHost, stream), {});
+    return TOPAY_OK;
+}
+
+int TpTrajChecker::fetch(int n, topay_feasibility* out) {
+    std::vector<TpFeasOut> h(n);
+    TP_CUDA_OK(cudaMemcpyAsync(h.data(), feas, (size_t)n * sizeof(TpFeasOut), cudaMemcpyDeviceToHost, stream), {});
     TP_CUDA_OK(cudaStreamSynchronize(stream), {});
     TP_CUDA_OK(cudaGetLastError(), {});
-    for (int i = 0; i < V.n; i++) {
+    for (int i = 0; i < n; i++) {
         const TpFeasOut& F = h[i];
         out->feasible[i] = F.feasible;
         if (out->feasible_print) out->feasible_print[i] = F.feasible_print;

@@ -26,6 +26,7 @@ struct TpTrajView {
     const double* T;            // [n][max_pieces]
     const double* coeff;        // [n][6*max_pieces][9]
     const double* start;        // [n][3]
+    const int32_t* idx;         // null, or [n]: trajectory i of the check is entry idx[i] of the arrays above
 };
 
 struct TpTrajChecker {
@@ -49,4 +50,8 @@ struct TpTrajChecker {
     int prepare(const TpTrajView& V);
     int check(const TpTrajView& V, const TpParams& P, const TpGrid& g, topay_feasibility* out,
               const TpGrid* grids = nullptr, const int32_t* field_of = nullptr);   // per-trajectory fields (sweeps)
+    // check() in two steps: the verdicts of V into `feas` on the device (field_of is indexed like V's arrays) ...
+    int run(const TpTrajView& V, const TpParams& P, const TpGrid& g, const TpGrid* grids, const int32_t* field_of);
+    // ... and the first n of them to the host
+    int fetch(int n, topay_feasibility* out);
 };

@@ -184,6 +184,20 @@ class MomaTrajOpt:
         _lib.check(self._l.topay_solver_assign_fields(self.h, hs, len(fields), _p(fo, C.c_int32)), "topay_solver_assign_fields")
         self._fields = list(fields)       # keep them alive
 
+    def set_plans(self, plan_offset=None, grace_evals=None, use_gate=False):
+        """topay_solver_set_plans: first success + grace of the planner's worker pool (planner.cpp:931-952), counted
+        in evaluations. plan_offset: first candidate of each plan + the total (default: one plan = the whole upload).
+        Once a plan has a success (status 1 and, with use_gate, printConstraintsSituations), its candidates that need
+        more than grace_evals evaluations beyond that success's are cancelled (status 0, lbfgs_code
+        LBFGSERR_PLAN_GRACE, results zero); the others are bit-identical to a run without plans. grace_evals=None
+        turns it off. The setting holds for uploads of the same size until it is changed."""
+        if grace_evals is None:
+            _lib.check(self._l.topay_solver_set_plans(self.h, 0, None, 0, 0), "topay_solver_set_plans")
+            return
+        off = np.ascontiguousarray([0, self._n] if plan_offset is None else plan_offset, dtype=np.int32)
+        _lib.check(self._l.topay_solver_set_plans(self.h, len(off) - 1, _p(off, C.c_int32), int(use_gate),
+                                                  int(grace_evals)), "topay_solver_set_plans")
+
     def run(self):
         _lib.check(self._l.topay_solver_run(self.h), "topay_solver_run")
 
@@ -228,19 +242,22 @@ class MomaTrajOpt:
         out["nbytes"] = int(sum(v.nbytes for v in r.values()))
         return out
 
-    def planWinners(self, plans, use_gate=True, fields=None):
+    def planWinners(self, plans, use_gate=True, fields=None, grace_evals=None):
         """The worker loop of planner.cpp:847-1010 for several plans in one device solve: every candidate is optimised
         (continuous batching), passed through the success gate (optimizeTraj && printConstraintsSituations,
         :877-880) and the shortest trajectory of each plan is picked (:999-1010) — all on the device; only each
         plan's winner crosses the bus. Returns a list with one entry per plan: the winner's result dict
         (download_candidate, `index` inside the plan) or None. `fields`: one GridMap per plan (scenario sweeps: every
-        plan is solved and gated against its own scenario's field, all plans share the launches of one solve)."""
+        plan is solved and gated against its own scenario's field, all plans share the launches of one solve).
+        grace_evals: first success + grace per plan (set_plans; None = off)."""
         paths = [q for p in plans for q in p[0]]
         bv = np.concatenate([np.asarray(p[1], dtype=np.float64).reshape(len(p[0]), 10, 2) for p in plans])
         ba = np.concatenate([np.asarray(p[2], dtype=np.float64).reshape(len(p[0]), 10, 2) for p in plans])
         self.upload(paths, bv, ba)
         if fields is not None:      # plan i against its own scenario's field (scenario sweeps)
             self.assign_fields(fields, np.repeat(np.arange(len(plans)), [len(p[0]) for p in plans]))
+        off = np.cumsum([0] + [len(p[0]) for p in plans]).astype(np.int32)
+        self.set_plans(off, grace_evals, use_gate)
         self.run()
         self.d2h_bytes = 0
         if use_gate:
@@ -248,7 +265,6 @@ class MomaTrajOpt:
             _lib.check(self._l.topay_solver_check_feasible(self.h, C.byref(f), None), "topay_solver_check_feasible")
             self.constraints = arrs
             self.d2h_bytes += self._n * 352     # what the gate itself reads back: per-trajectory metrics + sizes
-        off = np.cumsum([0] + [len(p[0]) for p in plans]).astype(np.int32)
         bd, _ = self.select(off, use_gate)
         self.d2h_bytes += int(bd.nbytes * 2)
         out = []
@@ -263,25 +279,29 @@ class MomaTrajOpt:
         self._last = None
         return out
 
-    def optimizeTrajBatch(self, paths, boundary_vel, boundary_acc):
-        """All candidates of a plan in one device solve; returns the result dict of download()."""
+    def optimizeTrajBatch(self, paths, boundary_vel, boundary_acc, grace_evals=None):
+        """All candidates of a plan in one device solve; returns the result dict of download(). grace_evals: first
+        success + grace over the batch as one plan (set_plans; None = off)."""
         self.upload(paths, boundary_vel, boundary_acc)
+        self.set_plans(None, grace_evals)
         self.run()
         return self.download()
 
-    def optimizeTrajPlans(self, plans):
+    def optimizeTrajPlans(self, plans, grace_evals=None):
         """Several plans through one device solve with continuous batching: `plans` is a list of
         (paths, boundary_vel, boundary_acc); their candidates are queued back to back and flow through the solver's
         slots (n_slots in flight, the next waiting candidate takes a slot the moment one finishes). Returns the
         result dict of download() over all candidates plus `plan_offset` (first candidate of each plan) and the
-        per-plan winners `plan_best_by_duration` / `plan_best_by_cost` (index inside the plan, -1 if none)."""
+        per-plan winners `plan_best_by_duration` / `plan_best_by_cost` (index inside the plan, -1 if none).
+        grace_evals: first success + grace per plan (set_plans; None = off)."""
         paths = [q for p in plans for q in p[0]]
         bv = np.concatenate([np.asarray(p[1], dtype=np.float64).reshape(len(p[0]), 10, 2) for p in plans])
         ba = np.concatenate([np.asarray(p[2], dtype=np.float64).reshape(len(p[0]), 10, 2) for p in plans])
         self.upload(paths, bv, ba)
+        off = np.cumsum([0] + [len(p[0]) for p in plans])
+        self.set_plans(off, grace_evals)
         self.run()
         r = self.download()
-        off = np.cumsum([0] + [len(p[0]) for p in plans])
         bd, bc = [], []
         for i in range(len(plans)):
             ok = np.flatnonzero(r["status"][off[i]:off[i + 1]] == 1)
