@@ -519,7 +519,8 @@ int topay_solver_run(topay_solver* s);          /* device solve of the uploaded 
  * `fields` (dense fields on the solver's device, rebuilt before the run); the solve, the success gate
  * (topay_solver_check_feasible) and the selection then read every candidate against its own field, so that a whole
  * group of scenarios shares the launches of one solve. The assignment holds for uploads of the same size until it is
- * changed; n_fields <= 1 returns to the solver's own field. Call after topay_solver_upload. */
+ * changed; n_fields <= 1 returns to the solver's own field. Call after topay_solver_upload. Rebuild the fields first;
+ * in a streaming session, a plan's field must stay as it is until the plan has finished (topay_solver_stream_submit). */
 int topay_solver_assign_fields(topay_solver* s, topay_field* const* fields, int n_fields, const int32_t* field_of);
 /* First success + grace of the planner's worker pool (planner.cpp:931-952), with the grace counted in evaluations
  * instead of the reference's 100 ms of wall-clock time, so that the outcome does not depend on scheduling. The upload
@@ -587,6 +588,44 @@ int topay_solver_select(topay_solver* s, int n_plans, const int32_t* plan_offset
 /* Results of ONE candidate of the last run (e.g. the winner): `out`'s arrays have length 1 (T: max_pieces,
  * coeff: 6 max_pieces x 9, x: topay_num_vars(max_pieces)). 28 KB at 64 pieces instead of the whole batch. */
 int topay_solver_download_candidate(topay_solver* s, int cand, topay_result_batch* out);
+
+/* Streaming session: plans are submitted while the solve runs, and each plan's winners come back as soon as that plan's
+ * last candidate has finished — the worker pool of planner.cpp:921-952 with plans arriving while it works. Every
+ * streamed plan is bit-identical to the same plan solved alone through the batch API on a fresh upload (results, gate
+ * metrics and winners): a candidate's result depends on its own inputs only, not on slots, lanes, timed mode or when
+ * its plan arrived. One host thread per solver, as for every other call.
+ *   stream_begin starts a session on an empty pool; it drops the uploaded batch and turns first success + grace off.
+ *     Both stages need bounded max_iterations (else TOPAY_ERR_INVALID_ARG), so every candidate ends; TOPAY_MAX_TICKS
+ *     does not apply. use_gate != 0: a candidate counts for its plan's winners only if printConstraintsSituations
+ *     passes (as topay_solver_select with use_gate). Two lanes when n_slots reaches the batch run's threshold.
+ *   stream_submit prepares every candidate on the host (a failure changes nothing), writes them into free store rows
+ *     and queues them; *plan_id names the plan until it is taken. Not enough free rows: TOPAY_ERR_TOO_LARGE, nothing
+ *     changed. `field` (NULL: the solver's own) is a built dense field on the solver's device; every candidate of the
+ *     plan is solved and gated against it. A ROG solver takes NULL only.
+ *   stream_advance runs up to max_batches batches of 16 ticks (graph replays, or plain launches in timed mode); idle
+ *     slots take the newly queued candidates first. *n_live (may be NULL) = candidates in the slots afterwards; 0 means
+ *     every submitted candidate has finished. Returns at once when nothing is live.
+ *   stream_poll writes up to cap finished plans, each reported once, with their winners by duration and by cost (index
+ *     inside the plan, -1: none; planner.cpp:999-1010, ties to the earliest candidate); returns the number written.
+ *   stream_take downloads the results of candidate `cand` of a finished plan (-1: all of them, in submission order;
+ *     topay_result_batch layout, entries past piece_num zero) and, if gate is not NULL, their gate metrics; then the
+ *     plan's rows and its id are free. An unknown, unfinished or already taken plan: TOPAY_ERR_INVALID_ARG.
+ *   stream_end ends the session and drops every plan not taken; the next upload / run gives what a fresh solver gives.
+ * Inside a session upload, run, solve_batch, eval, the download calls, select, check_feasible, assign_fields, set_plans,
+ * set_timed, set_trace and debug_direction return TOPAY_ERR_NOT_READY, and so do stream calls outside one.
+ * topay_solver_last_stats counts the session since stream_begin (evals_total: the candidates taken so far).
+ * A field a live plan reads must not be rebuilt, slid or updated until that plan has finished; the library does not
+ * check this. */
+int topay_solver_stream_begin(topay_solver* s, int use_gate);
+int topay_solver_stream_submit(topay_solver* s, int n_cand, const int32_t* path_len, const double* init_paths,
+                               const double* bvel, const double* bacc, topay_field* field, int32_t* plan_id);
+int topay_solver_stream_advance(topay_solver* s, int max_batches, int32_t* n_live);
+int topay_solver_stream_poll(topay_solver* s, int cap, int32_t* plan_id, int32_t* best_by_duration,
+                             int32_t* best_by_cost);
+int topay_solver_stream_take(topay_solver* s, int32_t plan_id, int cand, topay_result_batch* out,
+                             topay_feasibility* gate);
+int topay_solver_stream_end(topay_solver* s);
+
 /* timed != 0: every k_penalty launch is bracketed by CUDA events (stats.ms_eval) and the ticks are
  * plain launches; timed == 0 (default): a batch of 16 ticks is replayed as one CUDA graph, which
  * removes the per-launch host cost that dominates small plans; stats.ms_eval is then 0. */

@@ -8,6 +8,7 @@
 // Eigen::VectorXd / Eigen::MatrixXd / Eigen::Vector3d satisfy these directly.
 #pragma once
 #include <cmath>
+#include <map>
 #include <memory>
 #include <stdexcept>
 #include <string>
@@ -385,6 +386,70 @@ public:
         for (GridMap* g : fields) h.push_back(g->handle());
         topay_check(topay_solver_assign_fields(s_, h.data(), (int)h.size(), field_of.data()), "topay_solver_assign_fields");
     }
+
+    // Streaming session (topay_solver_stream_*): plans are submitted while the solve runs, and each plan's winners
+    // come back as soon as that plan is done — the worker pool of planner.cpp:921-952 with plans arriving while it
+    // works. The batch calls above are refused between streamBegin and streamEnd.
+    struct StreamDone { int32_t plan_id, best_by_duration, best_by_cost; };
+    void streamBegin(bool use_gate = true) {
+        topay_check(topay_solver_stream_begin(s_, use_gate ? 1 : 0), "topay_solver_stream_begin");
+        stream_starts_.clear();
+    }
+    // One plan (paths, bvel and bacc as in optimizeTrajBatch); `field` (nullptr: the solver's own) must stay as it is
+    // until the plan is done. Returns the plan id.
+    int32_t streamSubmit(const std::vector<std::vector<double>>& paths, const double* bvel, const double* bacc,
+                         GridMap* field = nullptr) {
+        const int n = (int)paths.size();
+        std::vector<int32_t> len(n);
+        std::vector<double> all, starts;
+        for (int c = 0; c < n; c++) {
+            len[c] = (int32_t)(paths[c].size() / 10);
+            all.insert(all.end(), paths[c].begin(), paths[c].end());
+            starts.insert(starts.end(), paths[c].begin(), paths[c].begin() + 3);
+        }
+        int32_t id = -1;
+        topay_check(topay_solver_stream_submit(s_, n, len.data(), all.data(), bvel, bacc,
+                                               field ? field->handle() : nullptr, &id), "topay_solver_stream_submit");
+        stream_starts_[id] = starts;
+        return id;
+    }
+    // Runs up to max_batches batches of 16 ticks; returns the candidates still in the slots (0: every plan is done).
+    int streamAdvance(int max_batches = 1) {
+        int32_t live = 0;
+        topay_check(topay_solver_stream_advance(s_, max_batches, &live), "topay_solver_stream_advance");
+        return live;
+    }
+    // The plans that finished since the last call, with their winners (index inside the plan, -1: none).
+    std::vector<StreamDone> streamPoll() {
+        std::vector<int32_t> id(max_cand_), bd(max_cand_), bc(max_cand_);
+        const int k = topay_solver_stream_poll(s_, max_cand_, id.data(), bd.data(), bc.data());
+        if (k < 0) topay_check(k, "topay_solver_stream_poll");
+        std::vector<StreamDone> out;
+        for (int i = 0; i < k; i++) out.push_back(StreamDone{id[i], bd[i], bc[i]});
+        return out;
+    }
+    // Takes a finished plan's candidates (all of them, or only `cand`): getTraj(i) then returns the i-th one taken.
+    // The plan's id is free afterwards.
+    void streamTake(int32_t plan_id, int cand = -1) {
+        auto it = stream_starts_.find(plan_id);
+        if (it == stream_starts_.end()) topay_check(TOPAY_ERR_INVALID_ARG, "topay_solver_stream_take");
+        const int n = cand < 0 ? (int)it->second.size() / 3 : 1;
+        status_.assign(n, 0); pieces_.assign(n, 0); cost_.assign(n, 0.0);
+        T_.assign((size_t)n * max_pieces_, 0.0);
+        coeff_.assign((size_t)n * 6 * max_pieces_ * 9, 0.0);
+        topay_result_batch out = {};
+        out.status = status_.data(); out.piece_num = pieces_.data(); out.cost = cost_.data();
+        out.T = T_.data(); out.coeff = coeff_.data();
+        topay_check(topay_solver_stream_take(s_, plan_id, cand, &out, nullptr), "topay_solver_stream_take");
+        starts_.assign(it->second.begin() + (cand < 0 ? 0 : 3 * cand),
+                       it->second.begin() + (cand < 0 ? it->second.size() : 3 * cand + 3));
+        stream_starts_.erase(it);
+        traj_cost = cost_[0];
+    }
+    void streamEnd() {
+        topay_check(topay_solver_stream_end(s_), "topay_solver_stream_end");
+        stream_starts_.clear();
+    }
 private:
     bool gate(const MomaTraj& traj, bool print_rule) {
         int32_t pn, f = 0, fp = 0;
@@ -405,6 +470,7 @@ private:
     int grace_evals_ = -1;
     std::vector<int32_t> status_, pieces_;
     std::vector<double> cost_, T_, coeff_, starts_;
+    std::map<int32_t, std::vector<double>> stream_starts_;   // start poses of the submitted plans, by plan id
 };
 
 }  // namespace nmoma_planner

@@ -121,6 +121,13 @@ PROTOTYPES = {
     "topay_solver_debug_direction": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, _dp, _dp, _dp, _dp,
                                                _dp, _ip, _ip]),
     "topay_solver_phase_clocks": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_longlong)]),
+    "topay_solver_stream_begin": (C.c_int, [C.c_void_p, C.c_int]),
+    "topay_solver_stream_submit": (C.c_int, [C.c_void_p, C.c_int, _ip, _dp, _dp, _dp, C.c_void_p, _ip]),
+    "topay_solver_stream_advance": (C.c_int, [C.c_void_p, C.c_int, _ip]),
+    "topay_solver_stream_poll": (C.c_int, [C.c_void_p, C.c_int, _ip, _ip, _ip]),
+    "topay_solver_stream_take": (C.c_int, [C.c_void_p, C.c_int32, C.c_int, C.POINTER(ResultBatch),
+                                           C.POINTER(Feasibility)]),
+    "topay_solver_stream_end": (C.c_int, [C.c_void_p]),
     "topay_solver_set_timed": (C.c_int, [C.c_void_p, C.c_int]),
     "topay_solver_last_stats": (C.c_int, [C.c_void_p, C.POINTER(SolverStats)]),
 }

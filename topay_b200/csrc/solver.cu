@@ -6,6 +6,7 @@
 #include <cstring>
 #include <cstdlib>
 #include <ctime>
+#include <deque>
 #include <map>
 #include <string>
 #include <vector>
@@ -52,6 +53,40 @@ struct TpLaunches {
 struct TpBatchGraph {
     cudaGraphExec_t exec;
     TpLaunches launches;
+};
+
+// Ticks and timed-mode figures of a run or of a streaming session, summed batch by batch.
+struct TpRunSums {
+    long long ticks = 0;
+    long long slot_ticks = 0;   // live slots summed over the batches (upper bound of the evaluations done)
+    double ms_eval = 0.0, ms_k[3] = {0.0, 0.0, 0.0}, ms_c[3] = {0.0, 0.0, 0.0}, full_ms_cand = 0.0;
+    unsigned long long hist_prev = 0, full_hist = 0;
+    long long full_ticks = 0;
+};
+
+// A plan of a streaming session: its store rows in submission order and, once its last candidate has finished, its
+// winners by duration and by cost (index inside the plan, -1: none).
+enum { TP_PLAN_FREE, TP_PLAN_LIVE, TP_PLAN_DONE };
+struct TpStreamPlan {
+    std::vector<int32_t> rows;
+    int state = TP_PLAN_FREE;
+    int32_t best[2] = {-1, -1};
+};
+
+// Host side of a streaming session (topay_solver_stream_begin .. _end). Store rows and plan ids are handed out here;
+// the queue, the refill of idle slots and the per-plan completion count run on the device.
+struct TpStream {
+    bool on = false;
+    bool gate = false;          // winners count only candidates that pass printConstraintsSituations
+    bool refill = false;        // rows were queued since idle slots last took any
+    int na = 0;                 // slots [0, na) belong to lane A, the others to lane B
+    int live_rows = 0;          // rows of the plans that have not finished
+    std::vector<int32_t> free_rows, free_plans;   // handed out from the back
+    std::vector<TpStreamPlan> plans;              // [max_cand], by plan id
+    std::deque<int32_t> ready;                    // finished plans not reported by topay_solver_stream_poll yet
+    TpRunSums sums;
+    double* trace = nullptr;    // the batch mode's L-BFGS trace, set aside for the session
+    int32_t* trace_len = nullptr;
 };
 
 struct topay_solver {
@@ -111,6 +146,9 @@ struct topay_solver {
     int plans_n_cand;           // the upload size the plans were set for
     int32_t *d_plan_of, *d_plan_first, *d_pending;   // [max_cand], [max_cand], [1 + max_cand]; allocated on first use
     bool grace_ran;             // the last run cancelled by the grace rule (check_feasible clears their verdicts)
+    // streaming session (topay_solver_stream_begin): dev.qrow and the pointers after it point here while one runs
+    TpStream sess;
+    int32_t *d_qrow, *d_row_plan, *d_plan_size, *d_plan_done, *d_done_ring;   // [max_cand] each, allocated on first use
 };
 
 namespace {
@@ -126,6 +164,11 @@ int solver_require_ready(const topay_solver* s) {
                                            : tp_field_ready(s->field);
     if (ready) return TOPAY_OK;
     tp_set_error("field not built: call topay_field_rebuild first");
+    return TOPAY_ERR_NOT_READY;
+}
+// What a batch-mode call returns while a streaming session owns the store and the slots.
+int in_session() {
+    tp_set_error("not available during a streaming session: call topay_solver_stream_end first");
     return TOPAY_ERR_NOT_READY;
 }
 
@@ -423,6 +466,10 @@ extern "C" void topay_solver_destroy(topay_solver* s) {
     cudaSetDevice(s->device);
     if (s->stream) cudaStreamSynchronize(s->stream);
     drop_graphs(s);
+    if (s->sess.on) {   // the trace the session set aside
+        s->dev.trace = s->sess.trace;
+        s->dev.trace_len = s->sess.trace_len;
+    }
     delete s->checker;
     if (s->dev.trace) cudaFree(s->dev.trace);
     if (s->dev.trace_len) cudaFree(s->dev.trace_len);
@@ -439,6 +486,22 @@ extern "C" void topay_solver_destroy(topay_solver* s) {
     if (s->lane[1].stream) cudaStreamDestroy(s->lane[1].stream);
     if (s->stream) cudaStreamDestroy(s->stream);
     delete s;
+}
+
+// Initial state of a candidate of N pieces entering `phase`; lambda / rho (two each) default to the ALM's initial values.
+static void init_state(const topay_solver* s, TpCandState& st, int phase, int N, int s1_past, const double* lambda,
+                       const double* rho) {
+    const topay_opt_params& op = s->params.opt;
+    memset(&st, 0, sizeof(st));
+    st.phase = phase;
+    st.N = N;
+    st.n = topay_num_vars(N);
+    st.ls_init = 1;
+    st.s1_past = s1_past;
+    st.lambda[0] = lambda ? lambda[0] : op.alm_init_lambda[0];
+    st.lambda[1] = lambda ? lambda[1] : op.alm_init_lambda[1];
+    st.rho[0] = rho ? rho[0] : op.alm_init_rho[0];
+    st.rho[1] = rho ? rho[1] : op.alm_init_rho[1];
 }
 
 // Uploads problem data + x of n_cand candidates into the store and their initial per-candidate state.
@@ -467,16 +530,8 @@ static int upload_problem(topay_solver* s, int n_cand, const int32_t* piece_num,
     s->h_x0_count = (size_t)n_cand * D.xs;
     for (int c = 0; c < n_cand; c++) {
         TpCandState& st = s->h_state[c];
-        memset(&st, 0, sizeof(st));
-        st.phase = phase;
-        st.N = piece_num[c];
-        st.n = topay_num_vars(piece_num[c]);
-        st.ls_init = 1;
-        st.s1_past = s1_past ? s1_past[c] : s->params.opt.s1_lbfgs.past;
-        st.lambda[0] = lambda ? lambda[2 * c] : s->params.opt.alm_init_lambda[0];
-        st.lambda[1] = lambda ? lambda[2 * c + 1] : s->params.opt.alm_init_lambda[1];
-        st.rho[0] = rho ? rho[2 * c] : s->params.opt.alm_init_rho[0];
-        st.rho[1] = rho ? rho[2 * c + 1] : s->params.opt.alm_init_rho[1];
+        init_state(s, st, phase, piece_num[c], s1_past ? s1_past[c] : s->params.opt.s1_lbfgs.past,
+                   lambda ? lambda + 2 * c : nullptr, rho ? rho + 2 * c : nullptr);
         memcpy(&xs[(size_t)c * D.xs], x + (size_t)c * x_stride, st.n * sizeof(double));
     }
     // the packed problem goes through the pinned staging block
@@ -521,6 +576,7 @@ extern "C" int topay_solver_eval(topay_solver* s, int stage, const topay_problem
                                  int x_stride, double* cost, double* grad, double* term_costs, double* coeff_out,
                                  double* final_xy_out) {
     if (!s || !prob || !x || !cost || !grad || (stage != 1 && stage != 2)) return TOPAY_ERR_INVALID_ARG;
+    if (s->sess.on) return in_session();
     int rc = solver_require_ready(s);
     if (rc != TOPAY_OK) return rc;
     if (prob->n_cand > s->dev.n_slots) {
@@ -571,6 +627,7 @@ extern "C" int topay_solver_eval(topay_solver* s, int stage, const topay_problem
 extern "C" int topay_solver_assign_fields(topay_solver* s, topay_field* const* fields, int n_fields,
                                           const int32_t* field_of) {
     if (!s) return TOPAY_ERR_INVALID_ARG;
+    if (s->sess.on) return in_session();
     cudaSetDevice(s->device);
     TpSolverDev& D = s->dev;
     if (n_fields <= 1) {
@@ -607,6 +664,7 @@ extern "C" int topay_solver_assign_fields(topay_solver* s, topay_field* const* f
 extern "C" int topay_solver_upload(topay_solver* s, int n_cand, const int32_t* path_len, const double* init_paths,
                                    const double* bvel, const double* bacc) {
     if (!s || !path_len || !init_paths || !bvel || !bacc) return TOPAY_ERR_INVALID_ARG;
+    if (s->sess.on) return in_session();
     const TpSolverDev& D = s->dev;
     if (n_cand < 1 || n_cand > D.max_cand) {
         tp_set_error("n_cand above the solver capacity");
@@ -704,6 +762,105 @@ static void mark_tick_cap(topay_solver* s, const TpLane& L, int n_store) {
     k_mark_tick_cap<<<(std::max(n_store, s->dev.n_slots) + 127) / 128, 128, 0, s->stream>>>(lane_dev(s, L), n_store);
 }
 
+// One batch of TP_TICKS ticks of both lanes at their live counts: a replay of the graph of its launch grids (captured
+// on first use), or plain launches with per-launch events in timed mode. Waits for it and reads the lanes' live
+// counts back into A.live / B.live; the pinned words of the grace gate and of a session's done ring come back too.
+static int run_batch(topay_solver* s, TpRunSums& m) {
+    const TpSolverDev& D = s->dev;
+    cudaStream_t q = s->stream;
+    TpLane &A = s->lane[0], &B = s->lane[1];
+    const bool use_graph = !s->timed;
+    const int ny = grid_bucket(A.live), ny_b = s->lanes == 2 ? grid_bucket(B.live) : 0;
+    const int key = ny | (ny_b << 16);
+    if (use_graph) {
+        auto it = s->graphs.find(key);
+        if (it == s->graphs.end()) {
+            cudaGraph_t g = nullptr;
+            cudaGraphExec_t ge = nullptr;
+            TP_CUDA_OK(cudaStreamBeginCapture(q, cudaStreamCaptureModeThreadLocal), {});
+            const TpLaunches launches = enqueue_batch(s, ny, ny_b, false);
+            TP_CUDA_OK(cudaStreamEndCapture(q, &g), {});
+            TP_CUDA_OK(cudaGraphInstantiate(&ge, g, 0), { cudaGraphDestroy(g); });
+            cudaGraphDestroy(g);
+            it = s->graphs.emplace(key, TpBatchGraph{ge, launches}).first;
+        }
+        TP_CUDA_OK(cudaGraphLaunch(it->second.exec, q), {});
+        it->second.launches.add_to(s->stats);
+    } else {
+        enqueue_batch(s, ny, 0, true).add_to(s->stats);
+        cudaMemcpyAsync(s->h_nodes, D.node_count, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, q);
+    }
+    if (D.plan_of && D.plan_gate) cudaMemcpyAsync(s->h_active + 5, D.pending, sizeof(int32_t), cudaMemcpyDeviceToHost, q);
+    if (D.qrow) cudaMemcpyAsync(s->h_active + 6, D.queue + 3, sizeof(int32_t), cudaMemcpyDeviceToHost, q);
+    m.ticks += TP_TICKS;
+    m.slot_ticks += (long long)(A.live + B.live) * TP_TICKS;
+    // spin while at most two solves run in this process (lowest latency, one busy core per plan), else sleep
+    if (g_solves_running.load(std::memory_order_relaxed) <= 2) {
+        TP_CUDA_OK(cudaStreamSynchronize(q), {});
+    } else {
+        cudaEventRecord(s->ev_batch, q);
+        TP_CUDA_OK(cudaEventSynchronize(s->ev_batch), {});
+    }
+    const int live_after = *A.h_live;
+    if (!use_graph) {
+        // batches in which every slot was still solving: the full-activity figures
+        const bool full = live_after == A.live;
+        const unsigned long long hist_now = s->h_nodes[1];
+        double cand_batch = 0.0, lbfgs_batch = 0.0;
+        for (int t = 0; t < TP_TICKS; t++) {
+            float ms = 0.f;
+            cudaEventElapsedTime(&ms, s->ev[TP_EV * t + 1], s->ev[TP_EV * t + 2]);
+            m.ms_eval += ms;
+            cudaEventElapsedTime(&ms, s->ev[TP_EV * t], s->ev[TP_EV * t + 1]);
+            m.ms_k[0] += ms;
+            cudaEventElapsedTime(&ms, s->ev[TP_EV * t + 2], s->ev[TP_EV * t + 3]);
+            m.ms_k[1] += ms;
+            cudaEventElapsedTime(&ms, s->ev[TP_EV * t + 3], s->ev[TP_EV * t + 6]);
+            m.ms_k[2] += ms;
+            cand_batch += ms;
+            for (int k = 0; k < 3; k++) {
+                cudaEventElapsedTime(&ms, s->ev[TP_EV * t + 3 + k], s->ev[TP_EV * t + 4 + k]);
+                m.ms_c[k] += ms;
+                if (k == 1) lbfgs_batch += ms;
+            }
+        }
+        if (full) {
+            m.full_ms_cand += lbfgs_batch;
+            m.full_hist += hist_now - m.hist_prev;
+            m.full_ticks += TP_TICKS;
+        }
+        m.hist_prev = hist_now;
+    }
+    A.live = live_after;
+    if (s->lanes == 2) B.live = *B.h_live;
+    return TOPAY_OK;
+}
+
+// End of a run, or of a session's advance: waits for the stream and writes the figures since ev_begin to stats.
+static int finish_stats(topay_solver* s, const TpRunSums& m) {
+    cudaStream_t q = s->stream;
+    cudaEventRecord(s->ev_end, q);
+    cudaMemcpyAsync(s->h_nodes, s->dev.node_count, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, q);
+    TP_CUDA_OK(cudaStreamSynchronize(q), {});
+    TP_CUDA_OK(cudaGetLastError(), {});
+    cudaEventElapsedTime(&s->stats.ms_total, s->ev_begin, s->ev_end);
+    s->stats.ms_eval = (float)m.ms_eval;
+    s->stats.ms_integrate = (float)m.ms_k[0];
+    s->stats.ms_chain = (float)m.ms_k[1];
+    s->stats.ms_cand = (float)m.ms_k[2];
+    s->stats.ms_adj = (float)m.ms_c[0];
+    s->stats.ms_lbfgs = (float)m.ms_c[1];
+    s->stats.ms_gen = (float)m.ms_c[2];
+    s->stats.ticks = m.ticks;
+    s->stats.slot_ticks = m.slot_ticks;
+    s->stats.eval_nodes = (int64_t)s->h_nodes[0];
+    s->stats.hist_bytes = (int64_t)s->h_nodes[1] * 16;
+    s->stats.full_ticks = m.full_ticks;
+    s->stats.full_hist_bytes = (int64_t)m.full_hist * 16;
+    s->stats.full_ms_cand = (float)m.full_ms_cand;   // one s_j and one y_j element per row element
+    return TOPAY_OK;
+}
+
 // Piece counts live in the per-candidate state and the start pose is split over start_xy and the
 // yaw slot of head_pva; gather both into the layout the trajectory kernels read.
 __global__ void k_solver_traj_view(const TpCandState* __restrict__ st, const double* __restrict__ start_xy,
@@ -797,6 +954,7 @@ static int gate_pending(topay_solver* s, int m, TpLaunches& n) {
 extern "C" int topay_solver_set_plans(topay_solver* s, int n_plans, const int32_t* plan_offset, int use_gate,
                                       int32_t grace_evals) {
     if (!s || n_plans < 0) return TOPAY_ERR_INVALID_ARG;
+    if (s->sess.on) return in_session();
     cudaSetDevice(s->device);
     TpSolverDev& D = s->dev;
     if (n_plans == 0) {
@@ -840,6 +998,7 @@ extern "C" int topay_solver_set_plans(topay_solver* s, int n_plans, const int32_
 }
 
 extern "C" int topay_solver_run(topay_solver* s) {
+    if (s && s->sess.on) return in_session();
     if (!s || s->n_cand < 1) return TOPAY_ERR_INVALID_ARG;
     const int rc = solver_require_ready(s);
     if (rc != TOPAY_OK) return rc;
@@ -880,9 +1039,7 @@ extern "C" int topay_solver_run(topay_solver* s) {
         B.live = A.live - na;
         A.live = na;
     }
-    double ms_eval = 0.0, ms_k[3] = {0.0, 0.0, 0.0}, ms_c[3] = {0.0, 0.0, 0.0}, full_ms_cand = 0.0;
-    unsigned long long hist_prev = 0, full_hist = 0;
-    long long full_ticks = 0;
+    TpRunSums sums;
     // Hard cap on ticks: no candidate does more evaluations than this (max_iterations == 0 means unbounded in
     // lbfgs.hpp; the cap then only guards against a runaway loop), times the number of refills of a slot.
     const topay_opt_params& op = s->params.opt;
@@ -894,77 +1051,14 @@ extern "C" int topay_solver_run(topay_solver* s) {
     const double waves = std::ceil((double)s->n_cand / std::max(1, s->n_slots_used));
     long long max_ticks = (long long)std::min(per_cand * waves, 4e15);
     if (const char* e = getenv("TOPAY_MAX_TICKS")) max_ticks = std::max(1LL, atoll(e));   // tests: force the cap
-    long long ticks = 0;
-    long long slot_ticks = 0;      // live slots summed over the batches (upper bound of the evaluations done)
     bool done = false;
-    const bool use_graph = !s->timed;
     if (s->graph_max_N != s->max_N) {
         drop_graphs(s);
         s->graph_max_N = s->max_N;
     }
-    while (!done && ticks < max_ticks) {
-        const int ny = grid_bucket(A.live), ny_b = s->lanes == 2 ? grid_bucket(B.live) : 0;
-        const int key = ny | (ny_b << 16);
-        if (use_graph) {
-            auto it = s->graphs.find(key);
-            if (it == s->graphs.end()) {
-                cudaGraph_t g = nullptr;
-                cudaGraphExec_t ge = nullptr;
-                TP_CUDA_OK(cudaStreamBeginCapture(q, cudaStreamCaptureModeThreadLocal), {});
-                const TpLaunches launches = enqueue_batch(s, ny, ny_b, false);
-                TP_CUDA_OK(cudaStreamEndCapture(q, &g), {});
-                TP_CUDA_OK(cudaGraphInstantiate(&ge, g, 0), { cudaGraphDestroy(g); });
-                cudaGraphDestroy(g);
-                it = s->graphs.emplace(key, TpBatchGraph{ge, launches}).first;
-            }
-            TP_CUDA_OK(cudaGraphLaunch(it->second.exec, q), {});
-            it->second.launches.add_to(s->stats);
-        } else {
-            enqueue_batch(s, ny, 0, true).add_to(s->stats);
-            cudaMemcpyAsync(s->h_nodes, D.node_count, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, q);
-        }
-        if (gate) cudaMemcpyAsync(s->h_active + 5, D.pending, sizeof(int32_t), cudaMemcpyDeviceToHost, q);
-        ticks += TP_TICKS;
-        slot_ticks += (long long)(A.live + B.live) * TP_TICKS;
-        // spin while at most two solves run in this process (lowest latency, one busy core per plan), else sleep
-        if (g_solves_running.load(std::memory_order_relaxed) <= 2) {
-            TP_CUDA_OK(cudaStreamSynchronize(q), {});
-        } else {
-            cudaEventRecord(s->ev_batch, q);
-            TP_CUDA_OK(cudaEventSynchronize(s->ev_batch), {});
-        }
-        const int live_after = *A.h_live;
-        if (!use_graph) {
-            // batches in which every slot was still solving: the full-activity figures
-            const bool full = live_after == A.live;
-            const unsigned long long hist_now = s->h_nodes[1];
-            double cand_batch = 0.0, lbfgs_batch = 0.0;
-            for (int t = 0; t < TP_TICKS; t++) {
-                float ms = 0.f;
-                cudaEventElapsedTime(&ms, s->ev[TP_EV * t + 1], s->ev[TP_EV * t + 2]);
-                ms_eval += ms;
-                cudaEventElapsedTime(&ms, s->ev[TP_EV * t], s->ev[TP_EV * t + 1]);
-                ms_k[0] += ms;
-                cudaEventElapsedTime(&ms, s->ev[TP_EV * t + 2], s->ev[TP_EV * t + 3]);
-                ms_k[1] += ms;
-                cudaEventElapsedTime(&ms, s->ev[TP_EV * t + 3], s->ev[TP_EV * t + 6]);
-                ms_k[2] += ms;
-                cand_batch += ms;
-                for (int k = 0; k < 3; k++) {
-                    cudaEventElapsedTime(&ms, s->ev[TP_EV * t + 3 + k], s->ev[TP_EV * t + 4 + k]);
-                    ms_c[k] += ms;
-                    if (k == 1) lbfgs_batch += ms;
-                }
-            }
-            if (full) {
-                full_ms_cand += lbfgs_batch;
-                full_hist += hist_now - hist_prev;
-                full_ticks += TP_TICKS;
-            }
-            hist_prev = hist_now;
-        }
-        A.live = live_after;
-        if (s->lanes == 2) B.live = *B.h_live;
+    while (!done && sums.ticks < max_ticks) {
+        const int brc = run_batch(s, sums);
+        if (brc != TOPAY_OK) return brc;
         done = A.live + B.live == 0;
         if (gate && s->h_active[5] > 0) {   // also after the last batch: nothing waits when the run ends
             TpLaunches g;
@@ -982,26 +1076,7 @@ extern "C" int topay_solver_run(topay_solver* s) {
         k_plan_fixup<<<s->n_cand, 128, 0, q>>>(D);
         s->stats.kernel_launches += 1;
     }
-    cudaEventRecord(s->ev_end, q);
-    cudaMemcpyAsync(s->h_nodes, D.node_count, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, q);
-    TP_CUDA_OK(cudaStreamSynchronize(q), {});
-    TP_CUDA_OK(cudaGetLastError(), {});
-    cudaEventElapsedTime(&s->stats.ms_total, s->ev_begin, s->ev_end);
-    s->stats.ms_eval = (float)ms_eval;
-    s->stats.ms_integrate = (float)ms_k[0];
-    s->stats.ms_chain = (float)ms_k[1];
-    s->stats.ms_cand = (float)ms_k[2];
-    s->stats.ms_adj = (float)ms_c[0];
-    s->stats.ms_lbfgs = (float)ms_c[1];
-    s->stats.ms_gen = (float)ms_c[2];
-    s->stats.ticks = ticks;
-    s->stats.slot_ticks = slot_ticks;
-    s->stats.eval_nodes = (int64_t)s->h_nodes[0];
-    s->stats.hist_bytes = (int64_t)s->h_nodes[1] * 16;
-    s->stats.full_ticks = full_ticks;
-    s->stats.full_hist_bytes = (int64_t)full_hist * 16;
-    s->stats.full_ms_cand = (float)full_ms_cand;   // one s_j and one y_j element per row element
-    return TOPAY_OK;
+    return finish_stats(s, sums);
 }
 
 // Entry c of `out` from a candidate's final state and its piece durations T[0..N); returns the trajectory's duration
@@ -1035,6 +1110,7 @@ static void clear_tail(topay_result_batch* out, int c, int N, int NP) {
 
 extern "C" int topay_solver_download(topay_solver* s, topay_result_batch* out, int32_t* best_by_duration,
                                      int32_t* best_by_cost) {
+    if (s && s->sess.on) return in_session();
     if (!s || !out || !out->status || s->n_cand < 1) return TOPAY_ERR_INVALID_ARG;
     cudaSetDevice(s->device);
     const TpSolverDev& D = s->dev;
@@ -1089,6 +1165,7 @@ extern "C" int topay_solver_solve_batch(topay_solver* s, int n_cand, const int32
 }
 
 extern "C" int topay_solver_check_feasible(topay_solver* s, topay_feasibility* out, int32_t* best_success) {
+    if (s && s->sess.on) return in_session();
     if (!s || !out || !out->feasible || s->n_cand < 1) return TOPAY_ERR_INVALID_ARG;
     cudaSetDevice(s->device);
     TpSolverDev& D = s->dev;
@@ -1122,25 +1199,29 @@ extern "C" int topay_solver_check_feasible(topay_solver* s, topay_feasibility* o
 // Selection on the device (planner.cpp:999-1010: the first success, replaced only by a strictly shorter duration;
 // the same rule on the cost): one block per plan walks its candidates, `ok` = optimizeTraj's status and, when the
 // gate ran, printConstraintsSituations' verdict (planner.cpp:877-880). Durations are summed in piece order like the
-// host loop of topay_solver_download, ties go to the lowest index.
+// host loop of topay_solver_download, ties go to the lowest index. Entry c of a plan is store row c, or rows[c] when a
+// row list is given (a streaming session's plans, whose rows need not be contiguous); feas is indexed by entry, and
+// ties go to the lowest entry, i.e. the earliest candidate of the plan.
 __global__ void __launch_bounds__(128)
 k_select(const TpCandState* __restrict__ st, const double* __restrict__ T, int max_pieces,
-         const TpFeasOut* __restrict__ feas, const int32_t* __restrict__ plan_off, int32_t* __restrict__ out) {
+         const TpFeasOut* __restrict__ feas, const int32_t* __restrict__ plan_off, const int32_t* __restrict__ rows,
+         int32_t* __restrict__ out) {
     const int plan = blockIdx.x, c0 = plan_off[plan], c1 = plan_off[plan + 1];
     int bd = INT32_MAX, bc = INT32_MAX;
     double bdv = 0.0, bcv = 0.0;
     for (int c = c0 + threadIdx.x; c < c1; c += blockDim.x) {
-        const bool ok = st[c].status == 1 && (!feas || feas[c].feasible_print != 0);
+        const int r = rows ? rows[c] : c;   // store row of entry c
+        const bool ok = st[r].status == 1 && (!feas || feas[c].feasible_print != 0);
         if (!ok) continue;
         double dur = 0.0;
-        for (int i = 0; i < st[c].N; i++) dur += T[(size_t)c * max_pieces + i];
+        for (int i = 0; i < st[r].N; i++) dur += T[(size_t)r * max_pieces + i];
         if (bd == INT32_MAX || dur < bdv) {
             bd = c;
             bdv = dur;
         }
-        if (bc == INT32_MAX || st[c].cost < bcv) {
+        if (bc == INT32_MAX || st[r].cost < bcv) {
             bc = c;
-            bcv = st[c].cost;
+            bcv = st[r].cost;
         }
     }
     __shared__ double s_v[2][128];
@@ -1169,6 +1250,7 @@ k_select(const TpCandState* __restrict__ st, const double* __restrict__ T, int m
 
 extern "C" int topay_solver_select(topay_solver* s, int n_plans, const int32_t* plan_offset, int use_gate,
                                    int32_t* best_by_duration, int32_t* best_by_cost) {
+    if (s && s->sess.on) return in_session();
     if (!s || s->n_cand < 1 || n_plans < 1 || !plan_offset || (!best_by_duration && !best_by_cost))
         return TOPAY_ERR_INVALID_ARG;
     for (int i = 0; i < n_plans; i++)
@@ -1186,7 +1268,7 @@ extern "C" int topay_solver_select(topay_solver* s, int n_plans, const int32_t* 
     int32_t* d = io.out(h.data(), h.size());
     if (io.ok())
         k_select<<<n_plans, 128, 0, s->stream>>>(D.res_st, D.res_T, D.max_pieces, use_gate ? s->checker->feas : nullptr,
-                                                 d_off, d);
+                                                 d_off, nullptr, d);
     const int rc = io.finish();
     if (rc != TOPAY_OK) return rc;
     for (int i = 0; i < n_plans; i++) {
@@ -1199,6 +1281,7 @@ extern "C" int topay_solver_select(topay_solver* s, int n_plans, const int32_t* 
 // Results of ONE candidate of the last run (the winner): the arrays of `out` have length 1 (T: max_pieces,
 // coeff: 6 max_pieces x 9, x: num_vars(max_pieces)).
 extern "C" int topay_solver_download_candidate(topay_solver* s, int cand, topay_result_batch* out) {
+    if (s && s->sess.on) return in_session();
     if (!s || !out || !out->status || cand < 0 || cand >= s->n_cand) return TOPAY_ERR_INVALID_ARG;
     cudaSetDevice(s->device);
     const TpSolverDev& D = s->dev;
@@ -1225,6 +1308,7 @@ extern "C" int topay_solver_download_candidate(topay_solver* s, int cand, topay_
 // doubles written (<= cap) or a negative status.
 extern "C" int64_t topay_solver_debug_download(topay_solver* s, int which, double* out, int64_t cap) {
     if (!s || !out) return TOPAY_ERR_INVALID_ARG;
+    if (s->sess.on) return in_session();
     cudaSetDevice(s->device);
     const TpSolverDev& D = s->dev;
     const size_t C_ = (size_t)D.n_slots, NP = (size_t)D.max_pieces, K = (size_t)D.K;
@@ -1254,6 +1338,7 @@ extern "C" int topay_solver_debug_direction(topay_solver* s, int n_vars, int bou
                                             const double* g, const double* gp, double* d_out, int32_t* bound_out,
                                             int32_t* end_out) {
     if (!s || !S_rows || !Y_rows || !ys || !x || !xp || !g || !gp || !d_out) return TOPAY_ERR_INVALID_ARG;
+    if (s->sess.on) return in_session();
     cudaSetDevice(s->device);
     const TpSolverDev& D = s->dev;
     const int m = std::min(s->params.opt.s2_lbfgs.mem_size, D.mem);
@@ -1339,12 +1424,14 @@ extern "C" int topay_solver_phase_clocks(topay_solver* s, int enable, long long*
 
 extern "C" int topay_solver_set_timed(topay_solver* s, int timed) {
     if (!s) return TOPAY_ERR_INVALID_ARG;
+    if (s->sess.on) return in_session();   // a session's lanes were laid out for the launch mode it began in
     s->timed = timed != 0;
     return TOPAY_OK;
 }
 
 extern "C" int topay_solver_set_trace(topay_solver* s, int cap) {
     if (!s || cap < 0) return TOPAY_ERR_INVALID_ARG;
+    if (s->sess.on) return in_session();
     cudaSetDevice(s->device);
     TpSolverDev& D = s->dev;
     drop_graphs(s);   // captured kernel arguments change
@@ -1365,6 +1452,7 @@ extern "C" int topay_solver_set_trace(topay_solver* s, int cap) {
 
 extern "C" int topay_solver_download_trace(topay_solver* s, int cand, double* out, int cap, int32_t* len) {
     if (!s || !out || !len || cand < 0 || cand >= s->dev.max_cand) return TOPAY_ERR_INVALID_ARG;
+    if (s->sess.on) return in_session();
     const TpSolverDev& D = s->dev;
     if (!D.trace) {
         tp_set_error("no trace recorded: call topay_solver_set_trace first");
@@ -1378,6 +1466,443 @@ extern "C" int topay_solver_download_trace(topay_solver* s, int cand, double* ou
     rc = tp_download(s->stream, out, D.trace + (size_t)cand * D.trace_cap * 4, (size_t)n * 4 * sizeof(double));
     if (rc != TOPAY_OK) return rc;
     *len = n;
+    return TOPAY_OK;
+}
+
+// ---- streaming session (topay_solver_stream_*)
+//
+// The store's rows are handed to plans on the host; the queue holds row ids (dev.qrow), so a slot that finishes pops
+// the next queued row on the device exactly as in batch mode. Between batches, rows of new plans are queued, idle
+// slots take them, and the plans whose last candidate finished get their winners.
+
+// Size of a candidate's staged record, in doubles: x0 [xs], head and tail [27 each], start and end [2 each], the
+// stage-1 targets [max_pieces x 2].
+__host__ __device__ inline int stream_record(const TpSolverDev& D) { return D.xs + 58 + 2 * D.max_pieces; }
+
+// The m candidates staged for `plan` go to their store rows; each row gets the plan and, on a dense solver (grids
+// non-null), the grid of the plan's field.
+__global__ void k_stream_scatter(const __grid_constant__ TpSolverDev S, const TpCandState* __restrict__ st,
+                                 const double* __restrict__ rec, const int32_t* __restrict__ rows, int m, int plan,
+                                 int32_t* row_plan, int32_t* plan_size, TpGrid* grids, int32_t* field_of,
+                                 const __grid_constant__ TpGrid g) {
+    const int c = blockIdx.x, row = rows[c], NP = S.max_pieces;
+    const double* r = rec + (size_t)c * stream_record(S);
+    for (int i = threadIdx.x; i < S.xs; i += blockDim.x) S.x0[(size_t)row * S.xs + i] = r[i];
+    r += S.xs;
+    for (int i = threadIdx.x; i < 27; i += blockDim.x) {
+        S.head_pva[(size_t)row * 27 + i] = r[i];
+        S.tail_pva[(size_t)row * 27 + i] = r[27 + i];
+    }
+    r += 54;
+    if (threadIdx.x < 2) {
+        S.start_xy[(size_t)row * 2 + threadIdx.x] = r[threadIdx.x];
+        S.end_xy[(size_t)row * 2 + threadIdx.x] = r[2 + threadIdx.x];
+    }
+    r += 4;
+    for (int i = threadIdx.x; i < 2 * NP; i += blockDim.x) S.init_inner_xy[(size_t)row * NP * 2 + i] = r[i];
+    if (threadIdx.x == 0) {
+        S.st0[row] = st[c];
+        row_plan[row] = plan;
+        if (grids) {
+            grids[row] = g;
+            field_of[row] = row;
+        }
+        if (c == 0) {
+            plan_size[plan] = m;
+            S.plan_done[plan] = 0;
+        }
+    }
+}
+
+// Appends m rows to the queue. Pops that found the queue empty left queue[0] past queue[1]; the head is brought back
+// to the tail, and both counters drop by whole rings, which keeps every q % max_cand and bounds them. One CTA.
+__global__ void k_stream_push(const __grid_constant__ TpSolverDev S, const int32_t* __restrict__ rows, int m) {
+    __shared__ int s_tail;
+    if (threadIdx.x == 0) {
+        const int q1 = S.queue[1], q0 = min(S.queue[0], q1), wrap = q0 - q0 % S.max_cand;
+        S.queue[0] = q0 - wrap;
+        S.queue[1] = q1 - wrap + m;
+        s_tail = q1 - wrap;
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < m; i += blockDim.x) S.qrow[(s_tail + i) % S.max_cand] = rows[i];
+}
+
+// Between batches, both lanes joined: every idle slot (never used, or its last pop found the queue empty) takes the
+// next queued row and joins the live list of its own lane (slots [0, na): lane A's), and list 0 of lane A, over which
+// k_stream_load and the generate half then run. One CTA.
+__global__ void k_stream_refill(const __grid_constant__ TpSolverDev S, int32_t* list_b, int32_t* count_b, int na) {
+    if (threadIdx.x == 0) S.count[0] = 0;
+    __syncthreads();
+    for (int slot = threadIdx.x; slot < S.n_slots; slot += blockDim.x) {
+        if (S.st[slot].phase != 0) continue;
+        const int q = atomicAdd(S.queue, 1);
+        if (q >= S.queue[1]) continue;
+        S.slot_gid[slot] = S.qrow[q % S.max_cand];
+        int32_t* list = slot < na ? S.list : list_b;
+        int32_t* count = slot < na ? S.count : count_b;
+        list[(size_t)TP_TICKS * S.n_slots + atomicAdd(count + TP_TICKS, 1)] = slot;
+        S.list[atomicAdd(S.count, 1)] = slot;
+    }
+}
+
+// The refilled slots (lane A's list 0) load their row's initial state, as k_cand's pop does.
+__global__ void k_stream_load(const __grid_constant__ TpSolverDev S) {
+    const int slot = tp_live_slot(S, 0, blockIdx.x);
+    if (slot < 0) return;
+    const int row = S.slot_gid[slot];
+    const TpCandState st = S.st0[row];
+    for (int i = threadIdx.x; i < st.n; i += blockDim.x) S.x[(size_t)slot * S.xs + i] = S.x0[(size_t)row * S.xs + i];
+    if (threadIdx.x == 0) S.st[slot] = st;
+}
+
+static int no_session() {
+    tp_set_error("no streaming session: call topay_solver_stream_begin first");
+    return TOPAY_ERR_NOT_READY;
+}
+
+// The success gate of n store rows (a device list): verdicts into the checker's `feas`, in list order.
+static int stream_gate(topay_solver* s, const int32_t* d_rows, int n, TpLaunches& l) {
+    int rc = solver_checker(s);
+    if (rc != TOPAY_OK) return rc;
+    const TpSolverDev& D = s->dev;
+    k_solver_traj_view<<<(D.max_cand + 127) / 128, 128, 0, s->stream>>>(D.res_st, D.start_xy, D.head_pva, D.max_cand,
+                                                                        s->d_pn, s->d_start);
+    const TpTrajView V{n, D.max_pieces, s->d_pn, D.res_T, D.res_coeff, s->d_start, d_rows};
+    TpGrid G;
+    solver_grid(s, &G);
+    rc = s->checker->run(V, s->params, G, D.n_fields > 1 ? D.grids : nullptr, D.field_of);
+    s->checker->checked_n = 0;   // `feas` holds these rows' verdicts, not those of a batch solve
+    l.kernels += 4;              // traj view + the checker's three
+    return rc;
+}
+
+// After a batch: the m plans on the done ring get their winners (through the gate with use_gate) and wait for poll.
+static int stream_finish_plans(topay_solver* s, int m, TpLaunches& l) {
+    TpStream& ss = s->sess;
+    const TpSolverDev& D = s->dev;
+    std::vector<int32_t> done(m);
+    int rc = tp_download(s->stream, done.data(), s->d_done_ring, (size_t)m * sizeof(int32_t));
+    if (rc != TOPAY_OK) return rc;
+    TP_CUDA_OK(cudaMemsetAsync(D.queue + 3, 0, sizeof(int32_t), s->stream), {});   // the ring has been read
+    std::vector<int32_t> rows, off{0}, best((size_t)2 * m);
+    for (int p : done) {
+        rows.insert(rows.end(), ss.plans[p].rows.begin(), ss.plans[p].rows.end());
+        off.push_back((int32_t)rows.size());
+    }
+    TpStaging io(s->stream);
+    const int32_t* d_rows = io.in(rows.data(), rows.size());
+    const int32_t* d_off = io.in(off.data(), off.size());
+    int32_t* d_best = io.out(best.data(), best.size());
+    if (io.ok() && ss.gate) rc = stream_gate(s, d_rows, (int)rows.size(), l);
+    if (io.ok() && rc == TOPAY_OK) {
+        k_select<<<m, 128, 0, s->stream>>>(D.res_st, D.res_T, D.max_pieces, ss.gate ? s->checker->feas : nullptr, d_off,
+                                           d_rows, d_best);
+        l.kernels += 1;
+    }
+    const int frc = io.finish();
+    if (rc != TOPAY_OK) return rc;
+    if (frc != TOPAY_OK) return frc;
+    for (int i = 0; i < m; i++) {
+        TpStreamPlan& P = ss.plans[done[i]];
+        P.state = TP_PLAN_DONE;
+        P.best[0] = best[2 * i];
+        P.best[1] = best[2 * i + 1];
+        ss.live_rows -= (int)P.rows.size();
+        ss.ready.push_back(done[i]);
+    }
+    return TOPAY_OK;
+}
+
+extern "C" int topay_solver_stream_begin(topay_solver* s, int use_gate) {
+    if (!s) return TOPAY_ERR_INVALID_ARG;
+    if (s->sess.on) {
+        tp_set_error("topay_solver_stream_begin: a streaming session is already running");
+        return TOPAY_ERR_NOT_READY;
+    }
+    const topay_opt_params& op = s->params.opt;
+    if (op.s1_lbfgs.max_iterations <= 0 || op.s2_lbfgs.max_iterations <= 0) {
+        tp_set_error("topay_solver_stream_begin: a session needs bounded max_iterations in both stages");
+        return TOPAY_ERR_INVALID_ARG;
+    }
+    cudaSetDevice(s->device);
+    TpSolverDev& D = s->dev;
+    const size_t G = (size_t)D.max_cand;
+    int rc;
+    if (!s->d_qrow) {
+        TpDevBuffers& b = s->bufs;
+        b.alloc(&s->d_qrow, G);
+        b.alloc(&s->d_row_plan, G);
+        b.alloc(&s->d_plan_size, G);
+        b.alloc(&s->d_plan_done, G);
+        b.alloc(&s->d_done_ring, G);
+        if ((rc = b.status) != TOPAY_OK) return rc;
+    }
+    if (!s->rog && !s->d_grids) {
+        if ((rc = s->bufs.alloc(&s->d_grids, G)) != TOPAY_OK) return rc;
+        if ((rc = s->bufs.alloc(&s->d_field_of, G)) != TOPAY_OK) return rc;
+    }
+    topay_solver_set_plans(s, 0, nullptr, 0, 0);   // first success + grace belongs to a batch upload
+    s->n_cand = 0;                                   // and so does the store's content
+    s->max_N = 0;
+    s->n_slots_used = D.n_slots;
+    drop_graphs(s);   // the captured kernel arguments change
+    s->graph_max_N = -1;
+    TpStream& ss = s->sess;
+    ss = TpStream();
+    ss.gate = use_gate != 0;
+    ss.trace = D.trace;
+    ss.trace_len = D.trace_len;
+    D.trace = nullptr;
+    D.trace_len = nullptr;
+    for (int i = D.max_cand - 1; i >= 0; i--) {   // rows and plan ids are handed out lowest first
+        ss.free_rows.push_back(i);
+        ss.free_plans.push_back(i);
+    }
+    ss.plans.resize(G);
+    D.qrow = s->d_qrow;
+    D.row_plan = s->d_row_plan;
+    D.plan_size = s->d_plan_size;
+    D.plan_done = s->d_plan_done;
+    D.done_ring = s->d_done_ring;
+    if (!s->rog) {   // every plan reads its own field (the solver's, or the one it was submitted with)
+        D.grids = s->d_grids;
+        D.field_of = s->d_field_of;
+        D.n_fields = 2;
+        s->fields.clear();
+    }
+    TpLane &A = s->lane[0], &B = s->lane[1];
+    s->lanes = (!s->timed && s->lane_min_slots > 0 && D.n_slots >= s->lane_min_slots) ? 2 : 1;
+    ss.na = s->lanes == 2 ? (D.n_slots + 1) / 2 : D.n_slots;
+    A.live = B.live = 0;
+    cudaStream_t q = s->stream;
+    TP_CUDA_OK(cudaMemsetAsync(D.st, 0, (size_t)D.n_slots * sizeof(TpCandState), q), {});   // phase 0: idle
+    TP_CUDA_OK(cudaMemsetAsync(D.queue, 0, 4 * sizeof(int32_t), q), {});
+    TP_CUDA_OK(cudaMemsetAsync(A.count, 0, (TP_TICKS + 1) * sizeof(int32_t), q), {});
+    TP_CUDA_OK(cudaMemsetAsync(B.count, 0, (TP_TICKS + 1) * sizeof(int32_t), q), {});
+    TP_CUDA_OK(cudaMemsetAsync(D.node_count, 0, 2 * sizeof(unsigned long long), q), {});
+    memset(&s->stats, 0, sizeof(s->stats));
+    cudaEventRecord(s->ev_begin, q);
+    TP_CUDA_OK(cudaStreamSynchronize(q), {});
+    ss.on = true;
+    return TOPAY_OK;
+}
+
+extern "C" int topay_solver_stream_submit(topay_solver* s, int n_cand, const int32_t* path_len, const double* init_paths,
+                                          const double* bvel, const double* bacc, topay_field* field,
+                                          int32_t* plan_id) {
+    if (!s || !path_len || !init_paths || !bvel || !bacc || !plan_id) return TOPAY_ERR_INVALID_ARG;
+    TpStream& ss = s->sess;
+    if (!ss.on) return no_session();
+    if (field && (s->rog || tp_field_device(field) != s->device)) {
+        tp_set_error("topay_solver_stream_submit: a plan's field is a dense field on the solver's device (ROG: NULL)");
+        return TOPAY_ERR_INVALID_ARG;
+    }
+    topay_field* f = field ? field : s->field;
+    if (!(s->rog ? tp_rogfield_ready(s->rog) : tp_field_ready(f))) {
+        tp_set_error("field not built: call topay_field_rebuild first");
+        return TOPAY_ERR_NOT_READY;
+    }
+    TpSolverDev& D = s->dev;
+    if (n_cand < 1 || n_cand > D.max_cand) {
+        tp_set_error("n_cand above the solver capacity");
+        return TOPAY_ERR_TOO_LARGE;
+    }
+    const int NP = D.max_pieces, R = stream_record(D);
+    std::vector<TpCandState> st(n_cand);
+    std::vector<double> rec((size_t)n_cand * R, 0.0);
+    size_t off = 0;
+    int maxN = 0;
+    for (int c = 0; c < n_cand; c++) {
+        double* r = &rec[(size_t)c * R];
+        int32_t pn = 0, past = 0;
+        const int rc = topay_prepare_candidate(&s->params.opt, &s->params.robot, init_paths + off * 10, path_len[c],
+                                               bvel + (size_t)c * 20, bacc + (size_t)c * 20, NP, &pn, r + D.xs,
+                                               r + D.xs + 27, r + D.xs + 54, r + D.xs + 56, r + D.xs + 58, r, &past);
+        if (rc != TOPAY_OK) {
+            tp_set_error("candidate needs more pieces than max_pieces");
+            return rc;
+        }
+        init_state(s, st[c], 1, pn, past, nullptr, nullptr);
+        maxN = std::max(maxN, pn);
+        off += path_len[c];
+    }
+    if ((int)ss.free_rows.size() < n_cand) {
+        tp_set_error("topay_solver_stream_submit: not enough free store rows (take finished plans first)");
+        return TOPAY_ERR_TOO_LARGE;
+    }
+    std::vector<int32_t> rows(ss.free_rows.end() - n_cand, ss.free_rows.end());
+    std::reverse(rows.begin(), rows.end());
+    const int32_t p = ss.free_plans.back();
+    TpGrid g{};
+    if (!s->rog) tp_field_grid(f, &g);
+    cudaSetDevice(s->device);
+    TpStaging io(s->stream);
+    const TpCandState* d_st = io.in(st.data(), st.size());
+    const double* d_rec = io.in(rec.data(), rec.size());
+    const int32_t* d_rows = io.in(rows.data(), rows.size());
+    if (io.ok()) {
+        k_stream_scatter<<<n_cand, 128, 0, s->stream>>>(D, d_st, d_rec, d_rows, n_cand, p, s->d_row_plan,
+                                                        s->d_plan_size, s->rog ? nullptr : s->d_grids, s->d_field_of, g);
+        k_stream_push<<<1, 256, 0, s->stream>>>(D, d_rows, n_cand);
+    }
+    const int rc = io.finish();
+    if (rc != TOPAY_OK) return rc;
+    ss.free_rows.resize(ss.free_rows.size() - n_cand);
+    ss.free_plans.pop_back();
+    ss.plans[p].rows = rows;
+    ss.plans[p].state = TP_PLAN_LIVE;
+    ss.live_rows += n_cand;
+    ss.refill = true;
+    s->max_N = std::max(s->max_N, maxN);   // a larger plan rebuilds the graphs at the next batch
+    s->stats.kernel_launches += 2;
+    *plan_id = p;
+    return TOPAY_OK;
+}
+
+extern "C" int topay_solver_stream_advance(topay_solver* s, int max_batches, int32_t* n_live) {
+    if (!s || max_batches < 0) return TOPAY_ERR_INVALID_ARG;
+    TpStream& ss = s->sess;
+    if (!ss.on) return no_session();
+    cudaSetDevice(s->device);
+    const TpSolverDev& D = s->dev;
+    cudaStream_t q = s->stream;
+    TpLane &A = s->lane[0], &B = s->lane[1];
+    TpRunningGuard running;
+    if (ss.refill) {
+        // idle slots take the queued rows and generate their first evaluation, outside the batch graph
+        const int nx = std::max(1, std::min(D.n_slots, ss.live_rows));
+        TpLaunches l;
+        k_stream_refill<<<1, 1024, 0, q>>>(D, B.list, B.count, ss.na);
+        k_stream_load<<<nx, 128, 0, q>>>(D);
+        launch_cand(s, A, TP_MODE_GEN, 0, -1, nx, l);
+        l.kernels += 2;
+        l.add_to(s->stats);
+        cudaMemcpyAsync(A.h_live, A.count + TP_TICKS, sizeof(int32_t), cudaMemcpyDeviceToHost, q);
+        cudaMemcpyAsync(B.h_live, B.count + TP_TICKS, sizeof(int32_t), cudaMemcpyDeviceToHost, q);
+        TP_CUDA_OK(cudaStreamSynchronize(q), {});
+        TP_CUDA_OK(cudaGetLastError(), {});
+        A.live = *A.h_live;
+        B.live = s->lanes == 2 ? *B.h_live : 0;
+        ss.refill = false;
+    }
+    if (s->graph_max_N != s->max_N) {
+        drop_graphs(s);
+        s->graph_max_N = s->max_N;
+    }
+    for (int b = 0; b < max_batches && A.live + B.live > 0; b++) {
+        int rc = run_batch(s, ss.sums);
+        if (rc != TOPAY_OK) return rc;
+        if (s->h_active[6] > 0) {
+            TpLaunches l;
+            rc = stream_finish_plans(s, s->h_active[6], l);
+            l.add_to(s->stats);
+            if (rc != TOPAY_OK) return rc;
+        }
+    }
+    if (n_live) *n_live = A.live + B.live;
+    return finish_stats(s, ss.sums);
+}
+
+extern "C" int topay_solver_stream_poll(topay_solver* s, int cap, int32_t* plan_id, int32_t* best_by_duration,
+                                        int32_t* best_by_cost) {
+    if (!s || cap < 0 || (cap > 0 && !plan_id)) return TOPAY_ERR_INVALID_ARG;
+    TpStream& ss = s->sess;
+    if (!ss.on) return no_session();
+    int k = 0;
+    for (; k < cap && !ss.ready.empty(); k++) {
+        const int32_t p = ss.ready.front();
+        ss.ready.pop_front();
+        plan_id[k] = p;
+        if (best_by_duration) best_by_duration[k] = ss.plans[p].best[0];
+        if (best_by_cost) best_by_cost[k] = ss.plans[p].best[1];
+    }
+    return k;
+}
+
+extern "C" int topay_solver_stream_take(topay_solver* s, int32_t plan_id, int cand, topay_result_batch* out,
+                                        topay_feasibility* gate) {
+    if (!s || !out || !out->status || (gate && !gate->feasible)) return TOPAY_ERR_INVALID_ARG;
+    TpStream& ss = s->sess;
+    if (!ss.on) return no_session();
+    const TpSolverDev& D = s->dev;
+    if (plan_id < 0 || plan_id >= D.max_cand || ss.plans[plan_id].state != TP_PLAN_DONE) {
+        tp_set_error("topay_solver_stream_take: unknown, unfinished or already taken plan");
+        return TOPAY_ERR_INVALID_ARG;
+    }
+    TpStreamPlan& P = ss.plans[plan_id];
+    const int np = (int)P.rows.size(), NP = D.max_pieces;
+    if (cand < -1 || cand >= np) {
+        tp_set_error("topay_solver_stream_take: cand outside the plan");
+        return TOPAY_ERR_INVALID_ARG;
+    }
+    cudaSetDevice(s->device);
+    const cudaStream_t q = s->stream;
+    const std::vector<int32_t> rows = cand < 0 ? P.rows : std::vector<int32_t>{P.rows[cand]};
+    const int n = (int)rows.size();
+    std::vector<TpCandState> st(np);   // every candidate's state: the session's evaluation count
+    for (int k = 0; k < np; k++)
+        TP_CUDA_OK(cudaMemcpyAsync(&st[k], D.res_st + P.rows[k], sizeof(TpCandState), cudaMemcpyDeviceToHost, q), {});
+    std::vector<double> T((size_t)n * NP), xs(out->x ? (size_t)n * D.xs : 0);
+    for (int k = 0; k < n; k++) {
+        const size_t r = (size_t)rows[k];
+        TP_CUDA_OK(cudaMemcpyAsync(&T[(size_t)k * NP], D.res_T + r * NP, NP * 8, cudaMemcpyDeviceToHost, q), {});
+        if (out->coeff)
+            TP_CUDA_OK(cudaMemcpyAsync(out->coeff + (size_t)k * 6 * NP * 9, D.res_coeff + r * 6 * NP * 9,
+                                       (size_t)6 * NP * 9 * 8, cudaMemcpyDeviceToHost, q), {});
+        if (out->x)
+            TP_CUDA_OK(cudaMemcpyAsync(&xs[(size_t)k * D.xs], D.res_x + r * D.xs, (size_t)D.xs * 8,
+                                       cudaMemcpyDeviceToHost, q), {});
+    }
+    TP_CUDA_OK(cudaStreamSynchronize(q), {});
+    const int xstride = topay_num_vars(NP);
+    for (int k = 0; k < n; k++) {
+        const TpCandState& sk = st[cand < 0 ? k : cand];
+        fill_result(out, k, sk, &T[(size_t)k * NP]);
+        if (out->x) memcpy(out->x + (size_t)k * xstride, &xs[(size_t)k * D.xs], (size_t)sk.n * 8);
+    }
+    if (out->T) memcpy(out->T, T.data(), T.size() * 8);
+    for (int k = 0; k < n; k++) clear_tail(out, k, st[cand < 0 ? k : cand].N, NP);
+    if (gate) {
+        TpStaging io(q);
+        const int32_t* d_rows = io.in(rows.data(), rows.size());
+        TpLaunches l;
+        int rc = io.ok() ? stream_gate(s, d_rows, n, l) : TOPAY_OK;
+        const int frc = io.finish();
+        if (rc == TOPAY_OK) rc = frc;
+        if (rc == TOPAY_OK) rc = s->checker->fetch(n, gate);
+        if (rc != TOPAY_OK) return rc;
+        l.add_to(s->stats);
+    }
+    for (const TpCandState& sk : st) s->stats.evals_total += sk.evals_total;
+    // the plan's rows and its id are free again
+    ss.free_rows.insert(ss.free_rows.end(), P.rows.rbegin(), P.rows.rend());
+    ss.free_plans.push_back(plan_id);
+    P = TpStreamPlan();
+    auto it = std::find(ss.ready.begin(), ss.ready.end(), plan_id);
+    if (it != ss.ready.end()) ss.ready.erase(it);
+    return TOPAY_OK;
+}
+
+extern "C" int topay_solver_stream_end(topay_solver* s) {
+    if (!s) return TOPAY_ERR_INVALID_ARG;
+    TpStream& ss = s->sess;
+    if (!ss.on) return no_session();
+    cudaSetDevice(s->device);
+    TP_CUDA_OK(cudaStreamSynchronize(s->stream), {});
+    TpSolverDev& D = s->dev;
+    D.qrow = nullptr;
+    D.row_plan = D.plan_size = nullptr;
+    D.plan_done = D.done_ring = nullptr;
+    D.n_fields = 0;   // back to the solver's own field
+    D.trace = ss.trace;
+    D.trace_len = ss.trace_len;
+    drop_graphs(s);
+    s->graph_max_N = -1;
+    s->lanes = 1;
+    s->max_N = 0;
+    s->n_cand = 0;    // batch mode starts from an upload
+    ss = TpStream();
     return TOPAY_OK;
 }
 

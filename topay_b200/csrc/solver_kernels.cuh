@@ -110,7 +110,21 @@ struct TpSolverDev {
     int32_t* pending;         // [0] count, [1 + i] status-1 candidates waiting for the gate (plan_gate only)
     int32_t grace;            // evaluations a plan's candidates may run past its first success
     int32_t plan_gate;        // a success counts once printConstraintsSituations passed (published by the host's gate)
+    // streaming session (topay_solver_stream_begin); qrow is null in batch mode, and then nothing below is read. The
+    // queue then holds store rows: pop q hands out row qrow[q % max_cand], and queue[3] counts the entries of done_ring.
+    int32_t* qrow;            // [max_cand] ring of queued store rows
+    const int32_t* row_plan;  // [store] plan slot of the row's candidate
+    const int32_t* plan_size; // [plan slot] candidates of the plan
+    int32_t* plan_done;       // [plan slot] candidates of the plan that have finished
+    int32_t* done_ring;       // [max_cand] plans whose last candidate finished since the host last read the ring
 };
+
+// Session: a candidate of row `gid` has written its results; the last one of its plan puts the plan on the done ring.
+// The ring and the results are read between batches, after the kernel has ended.
+__device__ __forceinline__ void tp_stream_retire(const TpSolverDev& S, int gid) {
+    const int p = S.row_plan[gid];
+    if (atomicAdd(S.plan_done + p, 1) == S.plan_size[p] - 1) S.done_ring[atomicAdd(S.queue + 3, 1)] = p;
+}
 
 // plan_first[] is lowered by other CTAs and by the host's gate while the solve runs; it only ever decreases, so a value
 // read at any moment is an upper bound of the final one and a cancellation made against it stands.
@@ -1990,8 +2004,9 @@ k_cand(const __grid_constant__ TpSolverDev S, const __grid_constant__ TpParams P
                     else atomicMin(S.plan_first + S.plan_of[gid], st.evals_total);
                 }
                 atomicAdd(S.queue + 2, 1);
+                if (S.qrow) tp_stream_retire(S, gid);
                 const int q = atomicAdd(S.queue, 1);
-                s_next = q < S.queue[1] ? q : -1;
+                s_next = q < S.queue[1] ? (S.qrow ? S.qrow[q % S.max_cand] : q) : -1;
             }
             __syncthreads();
             const int nxt = s_next;

@@ -119,6 +119,7 @@ class MomaTrajOpt:
                        "topay_solver_create_pool")
         self.traj_cost = 0.0
         self._last = None
+        self._stream = {}      # streaming session: plan id -> (candidates, start poses, field kept alive)
 
     def close(self):
         if getattr(self, "h", None) and self.h.value:
@@ -278,6 +279,68 @@ class MomaTrajOpt:
             out.append(r)
         self._last = None
         return out
+
+    # ---- streaming session: plans arrive while the solve runs ------------------------
+    def stream_begin(self, use_gate=False):
+        """topay_solver_stream_begin: from here on plans are submitted while the solve runs and each plan's winners
+        come back as soon as its last candidate has finished. use_gate: winners must pass printConstraintsSituations.
+        The uploaded batch is dropped; the batch calls are refused until stream_end()."""
+        _lib.check(self._l.topay_solver_stream_begin(self.h, int(use_gate)), "topay_solver_stream_begin")
+        self._stream = {}
+
+    def stream_submit(self, paths, bvel, bacc, field=None):
+        """Queues one plan (its candidates' waypoint lists and boundary velocities / accelerations, as upload()) and
+        returns its plan id. field: the GridMap the plan is solved and gated against (None: the solver's own)."""
+        n, plen, flat, bvel, bacc = self._flatten(paths, bvel, bacc)
+        pid = C.c_int32(-1)
+        _lib.check(self._l.topay_solver_stream_submit(self.h, n, _p(plen, C.c_int32), _p(flat), _p(bvel), _p(bacc),
+                                                      field.h if field is not None else None, C.byref(pid)),
+                   "topay_solver_stream_submit")
+        self._stream[pid.value] = (n, [np.asarray(p)[0, :3].copy() for p in paths], field)
+        return pid.value
+
+    def stream_advance(self, max_batches=1):
+        """Runs up to max_batches batches of 16 ticks; returns the candidates still in the slots (0: all done)."""
+        live = C.c_int32(0)
+        _lib.check(self._l.topay_solver_stream_advance(self.h, int(max_batches), C.byref(live)),
+                   "topay_solver_stream_advance")
+        return live.value
+
+    def stream_poll(self, cap=None):
+        """Finished plans not reported before: a list of (plan_id, best_by_duration, best_by_cost), winners as
+        indices inside the plan (-1: none)."""
+        cap = self.max_cand if cap is None else int(cap)
+        pid, bd, bc = (np.full(max(cap, 1), -1, np.int32) for _ in range(3))
+        k = self._l.topay_solver_stream_poll(self.h, cap, _p(pid, C.c_int32), _p(bd, C.c_int32), _p(bc, C.c_int32))
+        if k < 0:
+            _lib.check(k, "topay_solver_stream_poll")
+        return [(int(pid[i]), int(bd[i]), int(bc[i])) for i in range(k)]
+
+    def stream_take(self, plan_id, cand=None, gate=False):
+        """Results of a finished plan, then its rows and id are free: the dict of download() over its candidates, or
+        with `cand` the dict of download_candidate() for that one. gate=True adds the gate metrics under "gate"."""
+        n = self._stream[plan_id][0] if plan_id in self._stream else 1
+        m = n if cand is None else 1
+        r, rb = self._result_arrays(m)
+        f, arrs = alloc_feasibility(m) if gate else (None, None)
+        _lib.check(self._l.topay_solver_stream_take(self.h, int(plan_id), -1 if cand is None else int(cand),
+                                                    C.byref(rb), C.byref(f) if gate else None),
+                   "topay_solver_stream_take")
+        starts = self._stream.pop(plan_id)[1]
+        if cand is not None:
+            r = {k: v[0] for k, v in r.items()}
+            r["index"] = int(cand)
+            if gate:
+                arrs = {k: v[0] for k, v in arrs.items()}
+        r["starts"] = starts if cand is None else starts[int(cand)]
+        if gate:
+            r["gate"] = arrs
+        return r
+
+    def stream_end(self):
+        """Ends the session, dropping every plan not taken; the solver is back in batch mode."""
+        _lib.check(self._l.topay_solver_stream_end(self.h), "topay_solver_stream_end")
+        self._stream = {}
 
     def optimizeTrajBatch(self, paths, boundary_vel, boundary_acc, grace_evals=None):
         """All candidates of a plan in one device solve; returns the result dict of download(). grace_evals: first
