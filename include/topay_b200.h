@@ -73,7 +73,8 @@ enum {
      * (topay_solver_run); the candidate comes back with status 0 */
     TOPAY_LBFGSERR_TICK_CAP = -2000,
     /* not a reference code: the candidate was cancelled because its plan had succeeded more than the grace period
-     * earlier (topay_solver_set_plans); it comes back with status 0 */
+     * earlier (topay_solver_set_plans, topay_solver_stream_set_grace), or its plan was stopped
+     * (topay_solver_stream_stop); it comes back with status 0 */
     TOPAY_LBFGSERR_PLAN_GRACE = -2001
 };
 
@@ -594,8 +595,8 @@ int topay_solver_download_candidate(topay_solver* s, int cand, topay_result_batc
  * streamed plan is bit-identical to the same plan solved alone through the batch API on a fresh upload (results, gate
  * metrics and winners): a candidate's result depends on its own inputs only, not on slots, lanes, timed mode or when
  * its plan arrived. One host thread per solver, as for every other call.
- *   stream_begin starts a session on an empty pool; it drops the uploaded batch and turns first success + grace off.
- *     Both stages need bounded max_iterations (else TOPAY_ERR_INVALID_ARG), so every candidate ends; TOPAY_MAX_TICKS
+ *   stream_begin starts a session on an empty pool; it drops the uploaded batch and its set_plans setting, so a
+ *     session starts with first success + grace off (stream_set_grace turns it on). Both stages need bounded max_iterations (else TOPAY_ERR_INVALID_ARG), so every candidate ends; TOPAY_MAX_TICKS
  *     does not apply. use_gate != 0: a candidate counts for its plan's winners only if printConstraintsSituations
  *     passes (as topay_solver_select with use_gate). Two lanes when n_slots reaches the batch run's threshold.
  *   stream_submit prepares every candidate on the host (a failure changes nothing), writes them into free store rows
@@ -610,9 +611,29 @@ int topay_solver_download_candidate(topay_solver* s, int cand, topay_result_batc
  *   stream_take downloads the results of candidate `cand` of a finished plan (-1: all of them, in submission order;
  *     topay_result_batch layout, entries past piece_num zero) and, if gate is not NULL, their gate metrics; then the
  *     plan's rows and its id are free. An unknown, unfinished or already taken plan: TOPAY_ERR_INVALID_ARG.
+ *   stream_set_grace applies first success + grace (topay_solver_set_plans) to every plan streamed from then on:
+ *     grace_evals >= 0 turns it on, -1 turns it off, any other value is TOPAY_ERR_INVALID_ARG. A success follows the
+ *     session's use_gate. Every plan streamed with grace G is bit-identical (results, gate metrics from stream_take,
+ *     winners) to the same plan solved alone on a fresh upload with set_plans(1, {0, n}, use_gate, G), whatever the
+ *     slots, lanes, timed mode, arrival schedule or store rows. G is part of each live plan's contract: while a
+ *     submitted plan has not finished, the call returns TOPAY_ERR_NOT_READY (finished plans not taken yet are fine).
+ *   stream_stop stops a live plan, as the reference's interrupt_all (planner.cpp:952) does for its workers: a candidate
+ *     in a slot is cancelled at its next L-BFGS step; a queued one still takes a slot for one tick, its first
+ *     evaluation, and is cancelled right after it. The plan then finishes through stream_advance and stream_poll as
+ *     usual, reported once. Its candidates that finished before the stop keep their results under the plan's grace
+ *     contract, with S_p taken over them (with grace off, all of them are kept); every other candidate comes back
+ *     cancelled (status 0, TOPAY_LBFGSERR_PLAN_GRACE, the values of topay_solver_set_plans). Which candidates finish
+ *     before a stop depends on timing, so a stopped plan's outcome is not deterministic. What holds: each of its
+ *     candidates is either bit-identical to its result without grace or cancelled; a candidate that finished before
+ *     the stop and is kept by the grace contract is kept; other plans are unaffected bit for bit. A plan's field must
+ *     still stay as it is until the plan is reported. A finished plan not taken yet: TOPAY_OK, nothing changes. An
+ *     unknown or taken plan: TOPAY_ERR_INVALID_ARG. The first stop of a session without grace has candidates read their
+ *     plan's bound for the rest of the session (until stream_set_grace(-1) with no plan live), which replaces the
+ *     captured graphs once.
  *   stream_end ends the session and drops every plan not taken; the next upload / run gives what a fresh solver gives.
  * Inside a session upload, run, solve_batch, eval, the download calls, select, check_feasible, assign_fields, set_plans,
- * set_timed, set_trace and debug_direction return TOPAY_ERR_NOT_READY, and so do stream calls outside one.
+ * set_timed, set_trace and debug_direction return TOPAY_ERR_NOT_READY, and so do stream calls (stream_set_grace and
+ * stream_stop included) outside one.
  * topay_solver_last_stats counts the session since stream_begin (evals_total: the candidates taken so far).
  * A field a live plan reads must not be rebuilt, slid or updated until that plan has finished; the library does not
  * check this. */
@@ -624,6 +645,8 @@ int topay_solver_stream_poll(topay_solver* s, int cap, int32_t* plan_id, int32_t
                              int32_t* best_by_cost);
 int topay_solver_stream_take(topay_solver* s, int32_t plan_id, int cand, topay_result_batch* out,
                              topay_feasibility* gate);
+int topay_solver_stream_set_grace(topay_solver* s, int32_t grace_evals);
+int topay_solver_stream_stop(topay_solver* s, int32_t plan_id);
 int topay_solver_stream_end(topay_solver* s);
 
 /* timed != 0: every k_penalty launch is bracketed by CUDA events (stats.ms_eval) and the ticks are

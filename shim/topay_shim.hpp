@@ -391,10 +391,14 @@ public:
     // come back as soon as that plan is done — the worker pool of planner.cpp:921-952 with plans arriving while it
     // works. The batch calls above are refused between streamBegin and streamEnd.
     struct StreamDone { int32_t plan_id, best_by_duration, best_by_cost; };
-    void streamBegin(bool use_gate = true) {
+    // grace_evals >= 0: first success + grace for every plan of the session (setGrace's rule; -1: off).
+    void streamBegin(bool use_gate = true, int grace_evals = -1) {
         topay_check(topay_solver_stream_begin(s_, use_gate ? 1 : 0), "topay_solver_stream_begin");
         stream_starts_.clear();
+        if (grace_evals >= 0) topay_check(topay_solver_stream_set_grace(s_, grace_evals), "topay_solver_stream_set_grace");
     }
+    // Cancels a live plan's remaining candidates (planner.cpp:952's interrupt_all); streamPoll reports it as usual.
+    void streamStop(int32_t plan_id) { topay_check(topay_solver_stream_stop(s_, plan_id), "topay_solver_stream_stop"); }
     // One plan (paths, bvel and bacc as in optimizeTrajBatch); `field` (nullptr: the solver's own) must stay as it is
     // until the plan is done. Returns the plan id.
     int32_t streamSubmit(const std::vector<std::vector<double>>& paths, const double* bvel, const double* bacc,

@@ -127,6 +127,8 @@ PROTOTYPES = {
     "topay_solver_stream_poll": (C.c_int, [C.c_void_p, C.c_int, _ip, _ip, _ip]),
     "topay_solver_stream_take": (C.c_int, [C.c_void_p, C.c_int32, C.c_int, C.POINTER(ResultBatch),
                                            C.POINTER(Feasibility)]),
+    "topay_solver_stream_set_grace": (C.c_int, [C.c_void_p, C.c_int32]),
+    "topay_solver_stream_stop": (C.c_int, [C.c_void_p, C.c_int32]),
     "topay_solver_stream_end": (C.c_int, [C.c_void_p]),
     "topay_solver_set_timed": (C.c_int, [C.c_void_p, C.c_int]),
     "topay_solver_last_stats": (C.c_int, [C.c_void_p, C.POINTER(SolverStats)]),

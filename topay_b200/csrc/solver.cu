@@ -71,6 +71,7 @@ struct TpStreamPlan {
     std::vector<int32_t> rows;
     int state = TP_PLAN_FREE;
     int32_t best[2] = {-1, -1};
+    bool graced = false;        // finished while candidates read their plan's bound: rows may carry the cancelled values
 };
 
 // Host side of a streaming session (topay_solver_stream_begin .. _end). Store rows and plan ids are handed out here;
@@ -903,15 +904,9 @@ __global__ void k_plan_publish(const __grid_constant__ TpSolverDev S, const TpFe
     if (threadIdx.x == 0) S.pending[0] = 0;
 }
 
-// End of a run, one CTA per candidate: every candidate of the store with more evaluations than its plan's first
-// success + grace leaves with the cancelled values, whether the device stopped it or it finished before the
-// plan's first success was known.
-__global__ void k_plan_fixup(const __grid_constant__ TpSolverDev S) {
-    const int gid = blockIdx.x;
-    const TpCandState st = S.res_st[gid];
-    const bool cancel = st.evals_total - S.grace > S.plan_first[S.plan_of[gid]];
-    __syncthreads();   // every thread has read res_st before thread 0 rewrites it
-    if (!cancel) return;
+// Store row gid leaves with the cancelled values: piece_num kept, everything else zero, an empty trace. st is the row's
+// final state, which every thread of the CTA has read before the call.
+__device__ void tp_cancel_row(const TpSolverDev& S, int gid, const TpCandState& st) {
     for (int i = threadIdx.x; i < S.max_pieces; i += blockDim.x) S.res_T[(size_t)gid * S.max_pieces + i] = 0.0;
     for (int i = threadIdx.x; i < 6 * S.max_pieces * 9; i += blockDim.x)
         S.res_coeff[(size_t)gid * 6 * S.max_pieces * 9 + i] = 0.0;
@@ -926,10 +921,23 @@ __global__ void k_plan_fixup(const __grid_constant__ TpSolverDev S) {
     }
 }
 
-// Gate verdicts of a candidate the grace rule cancelled: all zero.
-__global__ void k_plan_clear_gate(const TpCandState* __restrict__ st, TpFeasOut* feas, int n) {
+// End of a run, one CTA per candidate: every candidate of the store with more evaluations than its plan's first
+// success + grace leaves with the cancelled values, whether the device stopped it or it finished before the
+// plan's first success was known.
+__global__ void k_plan_fixup(const __grid_constant__ TpSolverDev S) {
+    const int gid = blockIdx.x;
+    const TpCandState st = S.res_st[gid];
+    const bool cancel = st.evals_total - S.grace > S.plan_first[S.plan_of[gid]];
+    __syncthreads();   // every thread has read res_st before thread 0 rewrites it
+    if (cancel) tp_cancel_row(S, gid, st);
+}
+
+// Gate verdicts of a candidate the grace rule cancelled: all zero. Entry c is store row c, or rows[c] when a row list
+// is given (a session's plan).
+__global__ void k_plan_clear_gate(const TpCandState* __restrict__ st, TpFeasOut* feas, const int32_t* __restrict__ rows,
+                                  int n) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c < n && st[c].last_code == TOPAY_LBFGSERR_PLAN_GRACE) feas[c] = TpFeasOut{};
+    if (c < n && st[rows ? rows[c] : c].last_code == TOPAY_LBFGSERR_PLAN_GRACE) feas[c] = TpFeasOut{};
 }
 
 // use_gate: the m successes waiting in S.pending go through the same checker as topay_solver_check_feasible, and
@@ -938,8 +946,9 @@ static int gate_pending(topay_solver* s, int m, TpLaunches& n) {
     int rc = solver_checker(s);
     if (rc != TOPAY_OK) return rc;
     const TpSolverDev& D = s->dev;
-    k_solver_traj_view<<<(s->n_cand + 127) / 128, 128, 0, s->stream>>>(D.res_st, D.start_xy, D.head_pva, s->n_cand,
-                                                                       s->d_pn, s->d_start);
+    const int rows = s->sess.on ? D.max_cand : s->n_cand;   // a session's successes may sit in any store row
+    k_solver_traj_view<<<(rows + 127) / 128, 128, 0, s->stream>>>(D.res_st, D.start_xy, D.head_pva, rows, s->d_pn,
+                                                                   s->d_start);
     const TpTrajView V{m, D.max_pieces, s->d_pn, D.res_T, D.res_coeff, s->d_start, D.pending + 1};
     TpGrid G;
     solver_grid(s, &G);
@@ -949,6 +958,16 @@ static int gate_pending(topay_solver* s, int m, TpLaunches& n) {
     k_plan_publish<<<1, 256, 0, s->stream>>>(D, s->checker->feas, m);
     n.kernels += 5;   // traj view, the checker's three, publish
     return TOPAY_OK;
+}
+
+// The buffers of first success + grace, allocated on first use.
+static int plan_buffers(topay_solver* s) {
+    if (s->d_plan_of) return TOPAY_OK;
+    const size_t G = (size_t)s->dev.max_cand;
+    int rc;
+    if ((rc = s->bufs.alloc(&s->d_plan_of, G)) != TOPAY_OK) return rc;
+    if ((rc = s->bufs.alloc(&s->d_plan_first, G)) != TOPAY_OK) return rc;
+    return s->bufs.alloc(&s->d_pending, G + 1);
 }
 
 extern "C" int topay_solver_set_plans(topay_solver* s, int n_plans, const int32_t* plan_offset, int use_gate,
@@ -975,12 +994,8 @@ extern "C" int topay_solver_set_plans(topay_solver* s, int n_plans, const int32_
         tp_set_error("topay_solver_set_plans: plan_offset must start at 0, never decrease and end at n_cand");
         return TOPAY_ERR_INVALID_ARG;
     }
-    int rc;
-    if (!s->d_plan_of) {
-        if ((rc = s->bufs.alloc(&s->d_plan_of, (size_t)D.max_cand)) != TOPAY_OK) return rc;
-        if ((rc = s->bufs.alloc(&s->d_plan_first, (size_t)D.max_cand)) != TOPAY_OK) return rc;
-        if ((rc = s->bufs.alloc(&s->d_pending, (size_t)D.max_cand + 1)) != TOPAY_OK) return rc;
-    }
+    const int rc = plan_buffers(s);
+    if (rc != TOPAY_OK) return rc;
     std::vector<int32_t> plan_of(n);
     for (int p = 0; p < n_plans; p++) std::fill(plan_of.begin() + plan_offset[p], plan_of.begin() + plan_offset[p + 1], p);
     TP_CUDA_OK(cudaMemcpyAsync(s->d_plan_of, plan_of.data(), (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, s->stream), {});
@@ -1184,7 +1199,7 @@ extern "C" int topay_solver_check_feasible(topay_solver* s, topay_feasibility* o
     }
     rc = s->checker->run(V, s->params, G, D.n_fields > 1 ? D.grids : nullptr, D.field_of);
     if (rc == TOPAY_OK && s->grace_ran)
-        k_plan_clear_gate<<<(n + 127) / 128, 128, 0, s->stream>>>(D.res_st, s->checker->feas, n);
+        k_plan_clear_gate<<<(n + 127) / 128, 128, 0, s->stream>>>(D.res_st, s->checker->feas, nullptr, n);
     if (rc == TOPAY_OK) rc = s->checker->fetch(n, out);
     s->checker->checked_n = rc == TOPAY_OK ? n : 0;
     out->feasible_print = keep_fp;
@@ -1510,9 +1525,42 @@ __global__ void k_stream_scatter(const __grid_constant__ TpSolverDev S, const Tp
         if (c == 0) {
             plan_size[plan] = m;
             S.plan_done[plan] = 0;
+            if (S.plan_of) S.plan_first[plan] = INT32_MAX;   // the id may have served a plan that was taken
         }
     }
 }
+
+// Session, the m finished plans (entries off[p] .. off[p+1]-1 of the row list), one CTA per plan: every row the device
+// stopped leaves with the cancelled values and, with by_success, so does every row with evals - grace > S_p, the fewest
+// evaluations among the plan's successes in its final results (gate verdicts in feas when the plans are gated). S_p is
+// taken from the results rather than plan_first, which a stop sets to INT32_MIN. A gated session runs it twice: the
+// stopped rows first, whose trajectories are whatever the step they were stopped at left and are not fit for the gate,
+// then, after the gate, by success.
+__global__ void __launch_bounds__(128)
+k_stream_plan_fixup(const __grid_constant__ TpSolverDev S, const TpFeasOut* __restrict__ feas,
+                    const int32_t* __restrict__ off, const int32_t* __restrict__ rows, int by_success) {
+    const int c0 = off[blockIdx.x], c1 = off[blockIdx.x + 1];
+    __shared__ int s_first;
+    if (threadIdx.x == 0) s_first = INT32_MAX;
+    __syncthreads();
+    int first = INT32_MAX;
+    for (int c = c0 + threadIdx.x; by_success && c < c1; c += blockDim.x) {
+        const TpCandState& st = S.res_st[rows[c]];
+        if (st.status == 1 && (!feas || feas[c].feasible_print != 0)) first = min(first, st.evals_total);
+    }
+    atomicMin(&s_first, first);
+    __syncthreads();
+    for (int c = c0; c < c1; c++) {
+        const int r = rows[c];
+        const TpCandState st = S.res_st[r];
+        const bool cancel = st.last_code == TOPAY_LBFGSERR_PLAN_GRACE || st.evals_total - S.grace > s_first;
+        __syncthreads();   // every thread has read res_st before thread 0 rewrites it
+        if (cancel) tp_cancel_row(S, r, st);
+    }
+}
+
+// A stopped plan's candidates are cancelled at their next L-BFGS step: evals - grace > INT32_MIN for every grace.
+__global__ void k_stream_stop(const __grid_constant__ TpSolverDev S, int plan) { S.plan_first[plan] = INT32_MIN; }
 
 // Appends m rows to the queue. Pops that found the queue empty left queue[0] past queue[1]; the head is brought back
 // to the tail, and both counters drop by whole rings, which keeps every q % max_cand and bounds them. One CTA.
@@ -1594,10 +1642,20 @@ static int stream_finish_plans(topay_solver* s, int m, TpLaunches& l) {
     const int32_t* d_rows = io.in(rows.data(), rows.size());
     const int32_t* d_off = io.in(off.data(), off.size());
     int32_t* d_best = io.out(best.data(), best.size());
+    if (io.ok() && D.plan_of && ss.gate) {   // the rows the device stopped, before the gate reads them
+        k_stream_plan_fixup<<<m, 128, 0, s->stream>>>(D, nullptr, d_off, d_rows, 0);
+        l.kernels += 1;
+    }
     if (io.ok() && ss.gate) rc = stream_gate(s, d_rows, (int)rows.size(), l);
     if (io.ok() && rc == TOPAY_OK) {
-        k_select<<<m, 128, 0, s->stream>>>(D.res_st, D.res_T, D.max_pieces, ss.gate ? s->checker->feas : nullptr, d_off,
-                                           d_rows, d_best);
+        TpFeasOut* feas = ss.gate ? s->checker->feas : nullptr;
+        if (D.plan_of) {   // the grace contract and stops, then the verdicts of the rows they cancelled
+            const int n = (int)rows.size();
+            k_stream_plan_fixup<<<m, 128, 0, s->stream>>>(D, feas, d_off, d_rows, 1);
+            if (feas) k_plan_clear_gate<<<(n + 127) / 128, 128, 0, s->stream>>>(D.res_st, feas, d_rows, n);
+            l.kernels += feas ? 2 : 1;
+        }
+        k_select<<<m, 128, 0, s->stream>>>(D.res_st, D.res_T, D.max_pieces, feas, d_off, d_rows, d_best);
         l.kernels += 1;
     }
     const int frc = io.finish();
@@ -1608,6 +1666,7 @@ static int stream_finish_plans(topay_solver* s, int m, TpLaunches& l) {
         P.state = TP_PLAN_DONE;
         P.best[0] = best[2 * i];
         P.best[1] = best[2 * i + 1];
+        P.graced = D.plan_of != nullptr;
         ss.live_rows -= (int)P.rows.size();
         ss.ready.push_back(done[i]);
     }
@@ -1642,8 +1701,8 @@ extern "C" int topay_solver_stream_begin(topay_solver* s, int use_gate) {
         if ((rc = s->bufs.alloc(&s->d_grids, G)) != TOPAY_OK) return rc;
         if ((rc = s->bufs.alloc(&s->d_field_of, G)) != TOPAY_OK) return rc;
     }
-    topay_solver_set_plans(s, 0, nullptr, 0, 0);   // first success + grace belongs to a batch upload
-    s->n_cand = 0;                                   // and so does the store's content
+    topay_solver_set_plans(s, 0, nullptr, 0, 0);   // the batch upload's plans (a session's: stream_set_grace)
+    s->n_cand = 0;                                   // and the batch upload's store content end here
     s->max_N = 0;
     s->n_slots_used = D.n_slots;
     drop_graphs(s);   // the captured kernel arguments change
@@ -1793,6 +1852,12 @@ extern "C" int topay_solver_stream_advance(topay_solver* s, int max_batches, int
     for (int b = 0; b < max_batches && A.live + B.live > 0; b++) {
         int rc = run_batch(s, ss.sums);
         if (rc != TOPAY_OK) return rc;
+        if (D.plan_of && D.plan_gate && s->h_active[5] > 0) {   // first, so that a plan's last successes publish
+            TpLaunches g;                                          // before the plan is closed
+            rc = gate_pending(s, s->h_active[5], g);
+            g.add_to(s->stats);
+            if (rc != TOPAY_OK) return rc;
+        }
         if (s->h_active[6] > 0) {
             TpLaunches l;
             rc = stream_finish_plans(s, s->h_active[6], l);
@@ -1868,6 +1933,10 @@ extern "C" int topay_solver_stream_take(topay_solver* s, int32_t plan_id, int ca
         const int32_t* d_rows = io.in(rows.data(), rows.size());
         TpLaunches l;
         int rc = io.ok() ? stream_gate(s, d_rows, n, l) : TOPAY_OK;
+        if (io.ok() && rc == TOPAY_OK && P.graced) {   // cancelled rows: verdicts and metrics zero
+            k_plan_clear_gate<<<(n + 127) / 128, 128, 0, q>>>(D.res_st, s->checker->feas, d_rows, n);
+            l.kernels += 1;
+        }
         const int frc = io.finish();
         if (rc == TOPAY_OK) rc = frc;
         if (rc == TOPAY_OK) rc = s->checker->fetch(n, gate);
@@ -1884,6 +1953,72 @@ extern "C" int topay_solver_stream_take(topay_solver* s, int32_t plan_id, int ca
     return TOPAY_OK;
 }
 
+// Session: from here on every candidate reads its plan's bound (dev.plan_of = the rows' plan ids, plan_first by plan
+// id, every id reset, nothing pending) with this grace; successes wait for the gate between batches with `gate`.
+static int stream_plans_on(topay_solver* s, int32_t grace, int gate) {
+    int rc = plan_buffers(s);
+    if (rc != TOPAY_OK) return rc;
+    TpSolverDev& D = s->dev;
+    if (D.plan_of != s->d_row_plan || D.grace != grace || D.plan_gate != gate) drop_graphs(s);   // captured arguments
+    D.plan_of = s->d_row_plan;
+    D.plan_first = s->d_plan_first;
+    D.pending = s->d_pending;
+    D.grace = grace;
+    D.plan_gate = gate;
+    k_plan_reset<<<1, 256, 0, s->stream>>>(D, D.max_cand);
+    s->stats.kernel_launches += 1;
+    TP_CUDA_OK(cudaStreamSynchronize(s->stream), {});
+    TP_CUDA_OK(cudaGetLastError(), {});
+    return TOPAY_OK;
+}
+
+extern "C" int topay_solver_stream_set_grace(topay_solver* s, int32_t grace_evals) {
+    if (!s) return TOPAY_ERR_INVALID_ARG;
+    TpStream& ss = s->sess;
+    if (!ss.on) return no_session();
+    if (grace_evals < -1) {
+        tp_set_error("topay_solver_stream_set_grace: grace_evals >= 0, or -1 for off");
+        return TOPAY_ERR_INVALID_ARG;
+    }
+    if (ss.live_rows > 0) {
+        tp_set_error("topay_solver_stream_set_grace: a submitted plan has not finished yet");
+        return TOPAY_ERR_NOT_READY;
+    }
+    cudaSetDevice(s->device);
+    TpSolverDev& D = s->dev;
+    if (grace_evals < 0) {
+        if (D.plan_of) drop_graphs(s);   // the captured kernel arguments change
+        D.plan_of = nullptr;
+        D.grace = D.plan_gate = 0;
+    } else {
+        const int rc = stream_plans_on(s, grace_evals, ss.gate ? 1 : 0);
+        if (rc != TOPAY_OK) return rc;
+    }
+    return TOPAY_OK;
+}
+
+extern "C" int topay_solver_stream_stop(topay_solver* s, int32_t plan_id) {
+    if (!s) return TOPAY_ERR_INVALID_ARG;
+    TpStream& ss = s->sess;
+    if (!ss.on) return no_session();
+    if (plan_id < 0 || plan_id >= s->dev.max_cand || ss.plans[plan_id].state == TP_PLAN_FREE) {
+        tp_set_error("topay_solver_stream_stop: unknown or already taken plan");
+        return TOPAY_ERR_INVALID_ARG;
+    }
+    if (ss.plans[plan_id].state == TP_PLAN_DONE) return TOPAY_OK;
+    cudaSetDevice(s->device);
+    if (!s->dev.plan_of) {
+        // first stop of a session without grace: plans' bounds are read from now on, with a grace no candidate can
+        // exceed and no gate, so that only a stop cancels anything
+        const int rc = stream_plans_on(s, INT32_MAX, 0);
+        if (rc != TOPAY_OK) return rc;
+    }
+    k_stream_stop<<<1, 1, 0, s->stream>>>(s->dev, plan_id);
+    s->stats.kernel_launches += 1;
+    TP_CUDA_OK(cudaGetLastError(), {});
+    return TOPAY_OK;
+}
+
 extern "C" int topay_solver_stream_end(topay_solver* s) {
     if (!s) return TOPAY_ERR_INVALID_ARG;
     TpStream& ss = s->sess;
@@ -1894,6 +2029,8 @@ extern "C" int topay_solver_stream_end(topay_solver* s) {
     D.qrow = nullptr;
     D.row_plan = D.plan_size = nullptr;
     D.plan_done = D.done_ring = nullptr;
+    D.plan_of = nullptr;   // no plans until the next set_plans
+    D.grace = D.plan_gate = 0;
     D.n_fields = 0;   // back to the solver's own field
     D.trace = ss.trace;
     D.trace_len = ss.trace_len;

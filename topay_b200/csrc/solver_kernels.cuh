@@ -104,7 +104,8 @@ struct TpSolverDev {
     int32_t *trace_len;   // [store]
     int32_t trace_cap;
     long long *prof;      // optional phase clocks of candidate 0 (dev profiling), [16] or null
-    // first success + grace (topay_solver_set_plans); plan_of is null when it is off, and then nothing else is read
+    // first success + grace (topay_solver_set_plans; in a session stream_set_grace or stream_stop, and then plan_of is
+    // row_plan and plan_first is indexed by plan id); plan_of is null when it is off, and then nothing else is read
     const int32_t* plan_of;   // [store] plan of the candidate
     int32_t* plan_first;      // [plan] fewest evaluations of a success of the plan published so far (INT32_MAX: none)
     int32_t* pending;         // [0] count, [1 + i] status-1 candidates waiting for the gate (plan_gate only)

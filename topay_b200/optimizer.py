@@ -281,12 +281,28 @@ class MomaTrajOpt:
         return out
 
     # ---- streaming session: plans arrive while the solve runs ------------------------
-    def stream_begin(self, use_gate=False):
+    def stream_begin(self, use_gate=False, grace_evals=None):
         """topay_solver_stream_begin: from here on plans are submitted while the solve runs and each plan's winners
         come back as soon as its last candidate has finished. use_gate: winners must pass printConstraintsSituations.
-        The uploaded batch is dropped; the batch calls are refused until stream_end()."""
+        grace_evals: first success + grace for every plan of the session (stream_set_grace; None = off). The uploaded
+        batch is dropped; the batch calls are refused until stream_end()."""
         _lib.check(self._l.topay_solver_stream_begin(self.h, int(use_gate)), "topay_solver_stream_begin")
         self._stream = {}
+        if grace_evals is not None:
+            self.stream_set_grace(grace_evals)
+
+    def stream_set_grace(self, grace_evals=None):
+        """topay_solver_stream_set_grace: first success + grace (set_plans) for every plan streamed from now on; each
+        is bit-identical to its solo batch solve with that grace. None turns it off. Refused (NOT_READY) while a
+        submitted plan has not finished."""
+        _lib.check(self._l.topay_solver_stream_set_grace(self.h, -1 if grace_evals is None else int(grace_evals)),
+                   "topay_solver_stream_set_grace")
+
+    def stream_stop(self, plan_id):
+        """topay_solver_stream_stop: cancels the live plan's remaining candidates (the reference's interrupt_all); the
+        plan is then reported by stream_poll as usual, its winners taken from the candidates that finished before the
+        stop. A finished plan is left as it is."""
+        _lib.check(self._l.topay_solver_stream_stop(self.h, int(plan_id)), "topay_solver_stream_stop")
 
     def stream_submit(self, paths, bvel, bacc, field=None):
         """Queues one plan (its candidates' waypoint lists and boundary velocities / accelerations, as upload()) and
