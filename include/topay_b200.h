@@ -393,6 +393,11 @@ typedef struct topay_feasibility {
 /* MomaTrajOpt::checkFeasible for n trajectories at once: one thread block per trajectory. */
 int topay_traj_check_feasible(topay_field* f, const topay_robot_params* robot, const topay_traj_batch* trajs,
                               topay_feasibility* out);
+/* The same check against a ROG-Map ring (GridMap's use_rog branches, as the solver-resident gate of a ROG solver reads
+ * it): is a trajectory still feasible on the map as it is now? Runs on the ring's stream, after every update queued
+ * there. A ring never updated (topay_rogfield_update_esdf): TOPAY_ERR_NOT_READY. */
+int topay_traj_check_feasible_rog(topay_rogfield* f, const topay_robot_params* robot, const topay_traj_batch* trajs,
+                                  topay_feasibility* out);
 /* MomaTraj::car_seq (moma_traj_opt.h:38-68): entries (x, y, yaw, t); len[i] entries of
  * trajectory i are written to car_seq[i*cap*4 ...] (TOPAY_ERR_TOO_LARGE if one needs more than cap). */
 int topay_traj_car_seq(int device, const topay_traj_batch* trajs, int cap, double* car_seq, int32_t* len);
@@ -630,13 +635,30 @@ int topay_solver_download_candidate(topay_solver* s, int cand, topay_result_batc
  *     unknown or taken plan: TOPAY_ERR_INVALID_ARG. The first stop of a session without grace has candidates read their
  *     plan's bound for the rest of the session (until stream_set_grace(-1) with no plan live), which replaces the
  *     captured graphs once.
+ *   stream_set_snapshots (ROG solver) pins each plan to the ring as it was at its submit, so that the map keeps
+ *     updating while plans solve. n_snapshots >= 1 allocates that many copies of the ring's distance_buffer and its
+ *     critical and flat 2-D maps (at the reference's 803 x 803 x 83 ring: 428 MB + 2 x 5.2 MB = 438 MB each); 0 frees
+ *     them, and plans read the live ring again, with the launches of a session that never had snapshots. From then on
+ *     every stream_submit solves and gates its plan against the ring as it is at the submit: the caller may slide,
+ *     update counters, run topay_rogfield_update_esdf or topay_probmap_update between any two calls on the solver
+ *     (from the solver's host thread, or serialised with its calls: a submit reads the ring's state and queues its
+ *     copy on the ring's stream, so it must not overlap a ring update), and each plan is
+ *     bit-identical (results, gate metrics from stream_take, winners) to the same plan solved alone through the batch
+ *     API by a ROG solver on the ring as it was then (with grace, set_plans(1, {0, n}, use_gate, G)). Plans submitted
+ *     while the ring has not changed share one snapshot; a submit after a change copies the ring (on the ring's
+ *     stream) into a snapshot no plan holds, and when every snapshot is held it returns TOPAY_ERR_TOO_LARGE with
+ *     nothing changed, as for store rows. A plan holds its snapshot until stream_take, which runs the gate again.
+ *     While a submitted plan has not been taken: TOPAY_ERR_NOT_READY; a dense solver or n_snapshots < 0:
+ *     TOPAY_ERR_INVALID_ARG. stream_begin starts with snapshots off; stream_end frees them.
  *   stream_end ends the session and drops every plan not taken; the next upload / run gives what a fresh solver gives.
  * Inside a session upload, run, solve_batch, eval, the download calls, select, check_feasible, assign_fields, set_plans,
- * set_timed, set_trace and debug_direction return TOPAY_ERR_NOT_READY, and so do stream calls (stream_set_grace and
- * stream_stop included) outside one.
+ * set_timed, set_trace and debug_direction return TOPAY_ERR_NOT_READY, and so do stream calls (stream_set_grace,
+ * stream_stop and stream_set_snapshots included) outside one.
  * topay_solver_last_stats counts the session since stream_begin (evals_total: the candidates taken so far).
- * A field a live plan reads must not be rebuilt, slid or updated until that plan has finished; the library does not
- * check this. */
+ * Fields and the ring: in a session of a ROG solver with snapshots on, the library guarantees each plan the ring as it
+ * was at its submit. Otherwise a field a live plan reads (the ring of a ROG solver without snapshots, a dense plan's
+ * field) must not be rebuilt, slid or updated until that plan has been taken, since stream_take gates it again; the
+ * library does not check this. */
 int topay_solver_stream_begin(topay_solver* s, int use_gate);
 int topay_solver_stream_submit(topay_solver* s, int n_cand, const int32_t* path_len, const double* init_paths,
                                const double* bvel, const double* bacc, topay_field* field, int32_t* plan_id);
@@ -647,6 +669,7 @@ int topay_solver_stream_take(topay_solver* s, int32_t plan_id, int cand, topay_r
                              topay_feasibility* gate);
 int topay_solver_stream_set_grace(topay_solver* s, int32_t grace_evals);
 int topay_solver_stream_stop(topay_solver* s, int32_t plan_id);
+int topay_solver_stream_set_snapshots(topay_solver* s, int n_snapshots);
 int topay_solver_stream_end(topay_solver* s);
 
 /* timed != 0: every k_penalty launch is bracketed by CUDA events (stats.ms_eval) and the ticks are

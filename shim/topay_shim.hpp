@@ -17,6 +17,10 @@
 
 #include "../include/topay_b200.h"
 
+namespace rog_map {
+class ESDFMap;   // below: MomaTrajOpt can be built over the ROG-Map ring
+}
+
 namespace nmoma_planner {
 
 inline void topay_check(int rc, const char* what) {
@@ -278,14 +282,27 @@ public:
         topay_opt_params_default(&opt_param);
         topay_robot_params_default(&moma_param);
     }
+    // GridMap with use_rog (grid_map.h:90): the solve and the gate read the ROG-Map ring
+    explicit MomaTrajOpt(std::shared_ptr<rog_map::ESDFMap> esdf_map, int max_cand = 1, int max_pieces = 32)
+        : esdf_map_(esdf_map), max_cand_(max_cand), max_pieces_(max_pieces) {
+        topay_opt_params_default(&opt_param);
+        topay_robot_params_default(&moma_param);
+    }
     MomaTrajOpt(const MomaTrajOpt&) = delete;       // owns the device solver
     MomaTrajOpt& operator=(const MomaTrajOpt&) = delete;
     ~MomaTrajOpt() { topay_solver_destroy(s_); }
 
     // void init(ros::NodeHandle&) reads the rosparams into opt_param (moma_traj_opt.h:845-941); here the
     // caller fills opt_param (defaults = params/optimizer.yaml) and then calls init().
-    void init() { topay_check(topay_solver_create(&opt_param, &moma_param, grid_map->handle(), max_cand_, max_pieces_, &s_),
-                              "topay_solver_create"); }
+    void init() {
+        if (esdf_map_)
+            topay_check(topay_solver_create_rog(&opt_param, &moma_param, ring(), max_cand_, max_pieces_, &s_),
+                        "topay_solver_create_rog");
+        else
+            topay_check(topay_solver_create(&opt_param, &moma_param, grid_map->handle(), max_cand_, max_pieces_, &s_),
+                        "topay_solver_create");
+    }
+    bool useRog() const { return esdf_map_ != nullptr; }
 
     // bool optimizeTraj(std::vector<Eigen::VectorXd> init_path, const Eigen::MatrixXd& boundary_vel,
     //                   const Eigen::MatrixXd& boundary_acc)          (moma_traj_opt.cpp:142)
@@ -392,15 +409,22 @@ public:
     // works. The batch calls above are refused between streamBegin and streamEnd.
     struct StreamDone { int32_t plan_id, best_by_duration, best_by_cost; };
     // grace_evals >= 0: first success + grace for every plan of the session (setGrace's rule; -1: off).
-    void streamBegin(bool use_gate = true, int grace_evals = -1) {
+    // snapshots >= 1 (ROG solver): streamSetSnapshots.
+    void streamBegin(bool use_gate = true, int grace_evals = -1, int snapshots = 0) {
         topay_check(topay_solver_stream_begin(s_, use_gate ? 1 : 0), "topay_solver_stream_begin");
         stream_starts_.clear();
         if (grace_evals >= 0) topay_check(topay_solver_stream_set_grace(s_, grace_evals), "topay_solver_stream_set_grace");
+        if (snapshots > 0) streamSetSnapshots(snapshots);
+    }
+    // ROG solver: every plan submitted from now on is solved and gated against the ring as it is at the submit, so
+    // the ProbMap may keep updating it; up to n ring states are held by untaken plans at once (0: the live ring).
+    void streamSetSnapshots(int n) {
+        topay_check(topay_solver_stream_set_snapshots(s_, n), "topay_solver_stream_set_snapshots");
     }
     // Cancels a live plan's remaining candidates (planner.cpp:952's interrupt_all); streamPoll reports it as usual.
     void streamStop(int32_t plan_id) { topay_check(topay_solver_stream_stop(s_, plan_id), "topay_solver_stream_stop"); }
     // One plan (paths, bvel and bacc as in optimizeTrajBatch); `field` (nullptr: the solver's own) must stay as it is
-    // until the plan is done. Returns the plan id.
+    // until the plan is taken (a ROG solver with snapshots: the ring may change). Returns the plan id.
     int32_t streamSubmit(const std::vector<std::vector<double>>& paths, const double* bvel, const double* bacc,
                          GridMap* field = nullptr) {
         const int n = (int)paths.size();
@@ -464,11 +488,16 @@ private:
         out.max_domega = &constraints.max_domega; out.max_d2omega = &constraints.max_d2omega;
         out.max_q = constraints.max_q; out.max_dq = constraints.max_dq; out.max_d2q = constraints.max_d2q;
         out.min_dist = &constraints.min_dist; out.min_dist_mani = constraints.min_dist_mani;
-        topay_check(topay_traj_check_feasible(grid_map->handle(), &moma_param, &b, &out), "topay_traj_check_feasible");
+        if (esdf_map_)
+            topay_check(topay_traj_check_feasible_rog(ring(), &moma_param, &b, &out), "topay_traj_check_feasible_rog");
+        else
+            topay_check(topay_traj_check_feasible(grid_map->handle(), &moma_param, &b, &out), "topay_traj_check_feasible");
         return (print_rule ? fp : f) != 0;
     }
+    topay_rogfield* ring() const;   // esdf_map_'s handle (defined after rog_map::ESDFMap)
     topay_robot_params moma_param;
     GridMap::Ptr grid_map;
+    std::shared_ptr<rog_map::ESDFMap> esdf_map_;   // set instead of grid_map: GridMap's use_rog
     topay_solver* s_ = nullptr;
     int max_cand_, max_pieces_;
     int grace_evals_ = -1;
@@ -574,3 +603,5 @@ private:
 };
 
 }  // namespace rog_map
+
+inline topay_rogfield* nmoma_planner::MomaTrajOpt::ring() const { return esdf_map_->handle(); }

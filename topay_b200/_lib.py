@@ -91,6 +91,8 @@ PROTOTYPES = {
     "topay_probmap_set_first_frame": (C.c_int, [C.c_void_p, C.c_int]),
     "topay_traj_check_feasible": (C.c_int, [C.c_void_p, C.POINTER(RobotParams), C.POINTER(TrajBatch),
                                             C.POINTER(Feasibility)]),
+    "topay_traj_check_feasible_rog": (C.c_int, [C.c_void_p, C.POINTER(RobotParams), C.POINTER(TrajBatch),
+                                                C.POINTER(Feasibility)]),
     "topay_traj_car_seq": (C.c_int, [C.c_int, C.POINTER(TrajBatch), C.c_int, _dp, _ip]),
     "topay_traj_sample": (C.c_int, [C.c_int, C.POINTER(TrajBatch), _dp, C.c_int, _dp, _dp]),
     "topay_select_shortest": (C.c_int, [_ip, _dp, C.c_int]),
@@ -129,6 +131,7 @@ PROTOTYPES = {
                                            C.POINTER(Feasibility)]),
     "topay_solver_stream_set_grace": (C.c_int, [C.c_void_p, C.c_int32]),
     "topay_solver_stream_stop": (C.c_int, [C.c_void_p, C.c_int32]),
+    "topay_solver_stream_set_snapshots": (C.c_int, [C.c_void_p, C.c_int]),
     "topay_solver_stream_end": (C.c_int, [C.c_void_p]),
     "topay_solver_set_timed": (C.c_int, [C.c_void_p, C.c_int]),
     "topay_solver_last_stats": (C.c_int, [C.c_void_p, C.POINTER(SolverStats)]),

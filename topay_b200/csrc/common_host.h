@@ -27,6 +27,13 @@ void tp_field_grid(const topay_field* f, TpGrid* out);
 int tp_rogfield_device(const topay_rogfield* f);
 bool tp_rogfield_ready(const topay_rogfield* f);
 void tp_rogfield_grid(const topay_rogfield* f, TpGrid* out);   // kind = 1
+cudaStream_t tp_rogfield_stream(const topay_rogfield* f);     // the ring's own stream: every update runs on it
+// Generation of dist3 / crit / flat: changes whenever one of them is written (topay_rogfield_update_esdf, which
+// topay_probmap_update also runs). Slides and counter updates write only the counters.
+uint64_t tp_rogfield_generation(const topay_rogfield* f);
+// Copies dist3 [n3], crit and flat [n2 each] into caller memory on the ring's stream, then records `done` there: a
+// reader on another stream waits on `done`, and later updates of the ring queue behind the copy.
+int tp_rogfield_snapshot(topay_rogfield* f, double* dist3, double* crit, double* flat, cudaEvent_t done);
 // what the probabilistic layer (probmap.cu) needs of the ESDF ring it feeds: geometry, the two counter arrays, its stream
 struct TpRogCounters {
     TpRog view;

@@ -41,6 +41,8 @@ struct topay_rogfield {
     cudaEvent_t ev0, ev1, ev2;
     float ms_total, ms_3d;
     bool updated;               // updateESDF3D ran at least once
+    uint64_t generation;        // bumped by every update_esdf, the only writer of dist3 / crit / flat; read by a solver's
+                                // submit, which the caller serialises with updates (one host thread at a time)
     TpDevBuffers bufs;
 };
 
@@ -242,6 +244,16 @@ void tp_rogfield_grid(const topay_rogfield* f, TpGrid* out) {
     out->resolution_inv = f->res_inv;
     out->ready = f->updated ? 1 : 0;
 }
+cudaStream_t tp_rogfield_stream(const topay_rogfield* f) { return f->stream; }
+uint64_t tp_rogfield_generation(const topay_rogfield* f) { return f->generation; }
+int tp_rogfield_snapshot(topay_rogfield* f, double* dist3, double* crit, double* flat, cudaEvent_t done) {
+    cudaSetDevice(f->device);
+    TP_CUDA_OK(cudaMemcpyAsync(dist3, f->dist3, f->n3 * 8, cudaMemcpyDeviceToDevice, f->stream), {});
+    TP_CUDA_OK(cudaMemcpyAsync(crit, f->crit, f->n2 * 8, cudaMemcpyDeviceToDevice, f->stream), {});
+    TP_CUDA_OK(cudaMemcpyAsync(flat, f->flat, f->n2 * 8, cudaMemcpyDeviceToDevice, f->stream), {});
+    TP_CUDA_OK(cudaEventRecord(done, f->stream), {});
+    return TOPAY_OK;
+}
 
 extern "C" int topay_rogfield_create(const topay_rog_desc* d, int device, topay_rogfield** out) {
     if (!d || !out || d->prob_resolution <= 0.0 || d->esdf_resolution < d->prob_resolution || d->unk_thresh < 0.0 ||
@@ -417,6 +429,7 @@ extern "C" int topay_rogfield_update_esdf(topay_rogfield* f, const double cur_od
         if (B.idl[i] != 0) wrapped = true;
     }
     f->ms_total = f->ms_3d = 0.f;
+    f->generation++;            // what a solver's snapshot copied before this call may no longer be the ring
     if (B.b[0] <= 0 || B.b[1] <= 0 || B.b[2] <= 0) {
         f->updated = true;
         return TOPAY_OK;

@@ -8,6 +8,7 @@
 #include <ctime>
 #include <deque>
 #include <map>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -72,6 +73,15 @@ struct TpStreamPlan {
     int state = TP_PLAN_FREE;
     int32_t best[2] = {-1, -1};
     bool graced = false;        // finished while candidates read their plan's bound: rows may carry the cancelled values
+    int snap = -1;              // the ring snapshot the plan is solved and gated against (-1: the live ring / its field)
+};
+
+// A copy of the ROG ring's dist3 / crit / flat (topay_solver_stream_set_snapshots), the ring generation it holds
+// (0: none yet) and the untaken plans that read it.
+struct TpSnapshot {
+    double *dist3 = nullptr, *crit = nullptr, *flat = nullptr;
+    uint64_t generation = 0;
+    int holders = 0;
 };
 
 // Host side of a streaming session (topay_solver_stream_begin .. _end). Store rows and plan ids are handed out here;
@@ -88,6 +98,8 @@ struct TpStream {
     TpRunSums sums;
     double* trace = nullptr;    // the batch mode's L-BFGS trace, set aside for the session
     int32_t* trace_len = nullptr;
+    std::vector<TpSnapshot> snaps;               // ROG sessions with snapshots on; empty: plans read the live ring
+    std::unique_ptr<TpDevBuffers> snap_bufs;     // their buffers, freed when snapshots go off or the session ends
 };
 
 struct topay_solver {
@@ -150,6 +162,7 @@ struct topay_solver {
     // streaming session (topay_solver_stream_begin): dev.qrow and the pointers after it point here while one runs
     TpStream sess;
     int32_t *d_qrow, *d_row_plan, *d_plan_size, *d_plan_done, *d_done_ring;   // [max_cand] each, allocated on first use
+    cudaEvent_t ev_snap;        // a ring snapshot's copy has landed (recorded on the ring's stream)
 };
 
 namespace {
@@ -428,6 +441,7 @@ static int solver_create(const topay_opt_params* opt, const topay_robot_params* 
     s->lane[1].h_live = s->h_active + 4;
     cudaEventCreateWithFlags(&s->ev_fork, cudaEventDisableTiming);
     cudaEventCreateWithFlags(&s->ev_join, cudaEventDisableTiming);
+    cudaEventCreateWithFlags(&s->ev_snap, cudaEventDisableTiming);
     s->lanes = 1;
     s->lane_min_slots = getenv("TOPAY_LANE_MIN_SLOTS") ? atoi(getenv("TOPAY_LANE_MIN_SLOTS")) : 512;
     // LU band + one right-hand-side matrix, or the two-loop's TMA ring + its two 256-entry tables + one
@@ -484,6 +498,7 @@ extern "C" void topay_solver_destroy(topay_solver* s) {
     if (s->ev_batch) cudaEventDestroy(s->ev_batch);
     if (s->ev_fork) cudaEventDestroy(s->ev_fork);
     if (s->ev_join) cudaEventDestroy(s->ev_join);
+    if (s->ev_snap) cudaEventDestroy(s->ev_snap);
     if (s->lane[1].stream) cudaStreamDestroy(s->lane[1].stream);
     if (s->stream) cudaStreamDestroy(s->stream);
     delete s;
@@ -1494,8 +1509,8 @@ extern "C" int topay_solver_download_trace(topay_solver* s, int cand, double* ou
 // stage-1 targets [max_pieces x 2].
 __host__ __device__ inline int stream_record(const TpSolverDev& D) { return D.xs + 58 + 2 * D.max_pieces; }
 
-// The m candidates staged for `plan` go to their store rows; each row gets the plan and, on a dense solver (grids
-// non-null), the grid of the plan's field.
+// The m candidates staged for `plan` go to their store rows; each row gets the plan and, when rows read their own
+// field (grids non-null: a dense solver, or a ROG solver with snapshots), the grid of the plan's field or snapshot.
 __global__ void k_stream_scatter(const __grid_constant__ TpSolverDev S, const TpCandState* __restrict__ st,
                                  const double* __restrict__ rec, const int32_t* __restrict__ rows, int m, int plan,
                                  int32_t* row_plan, int32_t* plan_size, TpGrid* grids, int32_t* field_of,
@@ -1790,23 +1805,56 @@ extern "C" int topay_solver_stream_submit(topay_solver* s, int n_cand, const int
         tp_set_error("topay_solver_stream_submit: not enough free store rows (take finished plans first)");
         return TOPAY_ERR_TOO_LARGE;
     }
+    // with snapshots: the one holding the ring as it is now, else one no plan holds, which the ring is copied into
+    const uint64_t gen = s->rog ? tp_rogfield_generation(s->rog) : 0;
+    int snap = -1;
+    bool copy = false;
+    for (int i = 0; i < (int)ss.snaps.size() && snap < 0; i++)
+        if (ss.snaps[i].generation == gen) snap = i;
+    for (int i = 0; i < (int)ss.snaps.size() && snap < 0; i++)
+        if (ss.snaps[i].holders == 0) snap = i, copy = true;
+    if (!ss.snaps.empty() && snap < 0) {
+        tp_set_error("topay_solver_stream_submit: every ring snapshot is held by an untaken plan (take plans first)");
+        return TOPAY_ERR_TOO_LARGE;
+    }
     std::vector<int32_t> rows(ss.free_rows.end() - n_cand, ss.free_rows.end());
     std::reverse(rows.begin(), rows.end());
     const int32_t p = ss.free_plans.back();
     TpGrid g{};
     if (!s->rog) tp_field_grid(f, &g);
     cudaSetDevice(s->device);
+    if (snap >= 0) {
+        TpSnapshot& S = ss.snaps[snap];
+        tp_rogfield_grid(s->rog, &g);
+        g.rog.dist3 = S.dist3;
+        g.rog.crit = S.crit;
+        g.rog.flat = S.flat;
+        if (copy) {
+            // the slot's last reader was a take, which left the solver's stream idle; the solver's stream waits for
+            // the copy, and later ring updates queue behind it on the ring's stream
+            S.generation = 0;
+            int rc = tp_rogfield_snapshot(s->rog, S.dist3, S.crit, S.flat, s->ev_snap);
+            if (rc != TOPAY_OK) return rc;
+            TP_CUDA_OK(cudaStreamWaitEvent(s->stream, s->ev_snap, 0), {});
+        }
+    }
     TpStaging io(s->stream);
     const TpCandState* d_st = io.in(st.data(), st.size());
     const double* d_rec = io.in(rec.data(), rec.size());
     const int32_t* d_rows = io.in(rows.data(), rows.size());
     if (io.ok()) {
         k_stream_scatter<<<n_cand, 128, 0, s->stream>>>(D, d_st, d_rec, d_rows, n_cand, p, s->d_row_plan,
-                                                        s->d_plan_size, s->rog ? nullptr : s->d_grids, s->d_field_of, g);
+                                                        s->d_plan_size, D.n_fields > 1 ? s->d_grids : nullptr,
+                                                        s->d_field_of, g);
         k_stream_push<<<1, 256, 0, s->stream>>>(D, d_rows, n_cand);
     }
     const int rc = io.finish();
     if (rc != TOPAY_OK) return rc;
+    if (snap >= 0) {
+        ss.snaps[snap].generation = gen;
+        ss.snaps[snap].holders++;
+        ss.plans[p].snap = snap;
+    }
     ss.free_rows.resize(ss.free_rows.size() - n_cand);
     ss.free_plans.pop_back();
     ss.plans[p].rows = rows;
@@ -1944,6 +1992,7 @@ extern "C" int topay_solver_stream_take(topay_solver* s, int32_t plan_id, int ca
         l.add_to(s->stats);
     }
     for (const TpCandState& sk : st) s->stats.evals_total += sk.evals_total;
+    if (P.snap >= 0) ss.snaps[P.snap].holders--;   // the gate above was the plan's last read of its snapshot
     // the plan's rows and its id are free again
     ss.free_rows.insert(ss.free_rows.end(), P.rows.rbegin(), P.rows.rend());
     ss.free_plans.push_back(plan_id);
@@ -2019,6 +2068,58 @@ extern "C" int topay_solver_stream_stop(topay_solver* s, int32_t plan_id) {
     return TOPAY_OK;
 }
 
+extern "C" int topay_solver_stream_set_snapshots(topay_solver* s, int n_snapshots) {
+    if (!s) return TOPAY_ERR_INVALID_ARG;
+    TpStream& ss = s->sess;
+    if (!ss.on) return no_session();
+    if (!s->rog || n_snapshots < 0) {
+        tp_set_error("topay_solver_stream_set_snapshots: a ROG solver and n_snapshots >= 0");
+        return TOPAY_ERR_INVALID_ARG;
+    }
+    if ((int)ss.free_plans.size() != s->dev.max_cand) {
+        tp_set_error("topay_solver_stream_set_snapshots: a submitted plan has not been taken yet");
+        return TOPAY_ERR_NOT_READY;
+    }
+    cudaSetDevice(s->device);
+    TpSolverDev& D = s->dev;
+    // off first (plans read the live ring, through the launches and graphs of a plain session); a failed call below
+    // leaves snapshots off
+    if (D.n_fields > 1) drop_graphs(s);   // the captured kernel arguments change
+    D.grids = nullptr;
+    D.field_of = nullptr;
+    D.n_fields = 0;
+    ss.snaps.clear();
+    ss.snap_bufs.reset();
+    if (n_snapshots == 0) return TOPAY_OK;
+    int rc;
+    if (!s->d_grids) {
+        if ((rc = s->bufs.alloc(&s->d_grids, (size_t)D.max_cand)) != TOPAY_OK) return rc;
+        if ((rc = s->bufs.alloc(&s->d_field_of, (size_t)D.max_cand)) != TOPAY_OK) return rc;
+    }
+    TpGrid g;
+    tp_rogfield_grid(s->rog, &g);
+    const size_t n2 = (size_t)g.rog.size[0] * g.rog.size[1], n3 = n2 * g.rog.size[2];
+    std::unique_ptr<TpDevBuffers> b(new TpDevBuffers());
+    b->stream = s->stream;
+    std::vector<TpSnapshot> snaps(n_snapshots);
+    for (TpSnapshot& S : snaps) {
+        b->alloc(&S.dist3, n3);
+        b->alloc(&S.crit, n2);
+        b->alloc(&S.flat, n2);
+    }
+    if ((rc = b->status) != TOPAY_OK) return rc;
+    TP_CUDA_OK(cudaStreamSynchronize(s->stream), {});
+    ss.snaps.swap(snaps);
+    ss.snap_bufs = std::move(b);
+    // every row reads the grid k_stream_scatter gives it: the ring with its snapshot's buffers. The graphs captured so
+    // far hold the single-field k_penalty and the live ring's grid, so they go.
+    drop_graphs(s);
+    D.grids = s->d_grids;
+    D.field_of = s->d_field_of;
+    D.n_fields = 2;
+    return TOPAY_OK;
+}
+
 extern "C" int topay_solver_stream_end(topay_solver* s) {
     if (!s) return TOPAY_ERR_INVALID_ARG;
     TpStream& ss = s->sess;
@@ -2032,6 +2133,10 @@ extern "C" int topay_solver_stream_end(topay_solver* s) {
     D.plan_of = nullptr;   // no plans until the next set_plans
     D.grace = D.plan_gate = 0;
     D.n_fields = 0;   // back to the solver's own field
+    if (s->rog) {   // a ROG solver's rows read their own grids (snapshots) only in a session
+        D.grids = nullptr;
+        D.field_of = nullptr;
+    }
     D.trace = ss.trace;
     D.trace_len = ss.trace_len;
     drop_graphs(s);

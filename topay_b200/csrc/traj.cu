@@ -396,6 +396,27 @@ int stage_batch(const topay_traj_batch* b, TpStaging& io, TpTrajView* V) {
     return io.ok() ? TOPAY_OK : io.finish();
 }
 
+// The checker of both entry points on stream q, against grid g (a dense field or the ROG ring).
+int check_feasible_on(int dev, cudaStream_t q, const TpGrid& g, const topay_robot_params* robot,
+                      const topay_traj_batch* trajs, topay_feasibility* out) {
+    int rc;
+    {
+        TpStaging io(q);
+        TpTrajView V{};
+        TpTrajChecker ck;
+        TpParams P;
+        memset(&P, 0, sizeof(P));
+        P.robot = *robot;
+        topay_opt_params_default(&P.opt);
+        tp_derive_params(P);
+        rc = stage_batch(trajs, io, &V);
+        if (rc == TOPAY_OK) rc = ck.init(dev, q);
+        if (rc == TOPAY_OK) rc = ck.check(V, P, g, out);
+        cudaStreamSynchronize(q);
+    }
+    return rc;
+}
+
 }  // namespace
 
 extern "C" int topay_traj_check_feasible(topay_field* f, const topay_robot_params* robot, const topay_traj_batch* trajs,
@@ -407,24 +428,26 @@ extern "C" int topay_traj_check_feasible(topay_field* f, const topay_robot_param
     cudaSetDevice(dev);
     cudaStream_t q;
     TP_CUDA_OK(cudaStreamCreateWithFlags(&q, cudaStreamNonBlocking), {});
-    {
-        TpStaging io(q);
-        TpTrajView V{};
-        TpTrajChecker ck;
-        TpParams P;
-        memset(&P, 0, sizeof(P));
-        P.robot = *robot;
-        topay_opt_params_default(&P.opt);
-        tp_derive_params(P);
-        TpGrid g;
-        tp_field_grid(f, &g);
-        rc = stage_batch(trajs, io, &V);
-        if (rc == TOPAY_OK) rc = ck.init(dev, q);
-        if (rc == TOPAY_OK) rc = ck.check(V, P, g, out);
-        cudaStreamSynchronize(q);
-    }
+    TpGrid g;
+    tp_field_grid(f, &g);
+    rc = check_feasible_on(dev, q, g, robot, trajs, out);
     cudaStreamDestroy(q);
     return rc;
+}
+
+// On the ring's stream, so that the check reads the ring after every update queued on it.
+extern "C" int topay_traj_check_feasible_rog(topay_rogfield* f, const topay_robot_params* robot,
+                                             const topay_traj_batch* trajs, topay_feasibility* out) {
+    if (!f || !robot || !out || !out->feasible) return TOPAY_ERR_INVALID_ARG;
+    if (!tp_rogfield_ready(f)) {
+        tp_set_error("ring not built: call topay_rogfield_update_esdf first");
+        return TOPAY_ERR_NOT_READY;
+    }
+    const int dev = tp_rogfield_device(f);
+    cudaSetDevice(dev);
+    TpGrid g;
+    tp_rogfield_grid(f, &g);
+    return check_feasible_on(dev, tp_rogfield_stream(f), g, robot, trajs, out);
 }
 
 extern "C" int topay_traj_car_seq(int device, const topay_traj_batch* trajs, int cap, double* car_seq, int32_t* len) {

@@ -281,15 +281,27 @@ class MomaTrajOpt:
         return out
 
     # ---- streaming session: plans arrive while the solve runs ------------------------
-    def stream_begin(self, use_gate=False, grace_evals=None):
+    def stream_begin(self, use_gate=False, grace_evals=None, snapshots=0):
         """topay_solver_stream_begin: from here on plans are submitted while the solve runs and each plan's winners
         come back as soon as its last candidate has finished. use_gate: winners must pass printConstraintsSituations.
-        grace_evals: first success + grace for every plan of the session (stream_set_grace; None = off). The uploaded
-        batch is dropped; the batch calls are refused until stream_end()."""
+        grace_evals: first success + grace for every plan of the session (stream_set_grace; None = off). snapshots:
+        ring snapshots of a ROG solver (stream_set_snapshots; 0 = off). The uploaded batch is dropped; the batch calls
+        are refused until stream_end()."""
         _lib.check(self._l.topay_solver_stream_begin(self.h, int(use_gate)), "topay_solver_stream_begin")
         self._stream = {}
         if grace_evals is not None:
             self.stream_set_grace(grace_evals)
+        if snapshots:
+            self.stream_set_snapshots(snapshots)
+
+    def stream_set_snapshots(self, n):
+        """topay_solver_stream_set_snapshots (ROG solver): n >= 1 pins every plan submitted from now on to a copy of the
+        ring as it is at the submit, so the map may slide and update while plans solve; each plan is bit-identical to
+        its solo batch solve on the ring of its submit (ring updates come from this solver's thread, or are serialised
+        with its calls). Up to n ring states are held at once by untaken plans (a
+        submit that needs one more is refused with TOO_LARGE). 0 = plans read the live ring. Refused (NOT_READY)
+        while a submitted plan has not been taken."""
+        _lib.check(self._l.topay_solver_stream_set_snapshots(self.h, int(n)), "topay_solver_stream_set_snapshots")
 
     def stream_set_grace(self, grace_evals=None):
         """topay_solver_stream_set_grace: first success + grace (set_plans) for every plan streamed from now on; each
@@ -412,12 +424,12 @@ class MomaTrajOpt:
         returns the verdict(s). The accumulated metrics of the last call are in self.constraints."""
         single = isinstance(trajs, MomaTraj)
         lst = [trajs] if single else list(trajs)
-        if self.use_rog:
-            raise NotImplementedError("on a ROG field use checkFeasibleBatch() (the solver-resident gate)")
         tb, keep = pack_trajs([t._tuple() for t in lst])
         f, arrs = alloc_feasibility(len(lst))
-        _lib.check(self._l.topay_traj_check_feasible(self.grid_map.h, C.byref(self.moma_param), C.byref(tb),
-                                                     C.byref(f)), "topay_traj_check_feasible")
+        # on a ROG solver the ring as it is now: is the trajectory being executed still feasible on the updated map?
+        check = self._l.topay_traj_check_feasible_rog if self.use_rog else self._l.topay_traj_check_feasible
+        _lib.check(check(self.grid_map.h, C.byref(self.moma_param), C.byref(tb), C.byref(f)),
+                   "topay_traj_check_feasible")
         self.constraints = arrs
         return bool(arrs["feasible"][0]) if single else arrs["feasible"].astype(bool)
 
